@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- gravity warp+unwarp frames/sec at 640x480 on N B200s, with HBM-roofline accounting.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one batch of synthetic frames held by this rank:
@@ -357,6 +357,27 @@ def config5(dev, rank, world, frames_per_gpu=16, steps=3):
     return res
 
 
+DUMP_FRAMES = 4                 # whole frames written by --dump-outputs (8 planes, 9.8 MB a frame at 640x480)
+DUMP_SAMPLE = 1 << 18           # elements of each per-pixel output sampled over the whole batch
+
+
+def dump_outputs(out_dir, outputs):
+    """Writes the outputs of one timed step as out_dir/<name>.npy in float32, about 44 MB in all at 640x480.  Per-frame
+    matrices are written in full; each per-pixel output as DUMP_FRAMES whole frames (<name>.npy) and DUMP_SAMPLE elements
+    drawn over the whole batch (<name>_sample.npy).  Inputs and choices are seeded, so two builds compare output for output."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    rs = np.random.RandomState(2024)
+    for name, t in outputs.items():
+        a = t.detach().float()
+        if a.dim() == 4:
+            frames = np.sort(np.random.RandomState(2023).choice(a.shape[0], min(DUMP_FRAMES, a.shape[0]), replace=False))
+            idx = torch.from_numpy(rs.randint(0, a.numel(), size=min(DUMP_SAMPLE, a.numel()))).to(a.device)
+            np.save(os.path.join(out_dir, f"{name}_sample.npy"), a.reshape(-1)[idx].cpu().numpy())
+            a = a[frames]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.cpu().numpy())
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -387,8 +408,8 @@ def run_ours(args):
 
     def step():                                # SURVEY.md section 8(d): params kernel + forward kernel + inverse kernel
         p = w.prepare(g, a)               # per-frame parameters, once for the batch
-        w.warp_rgbd(rgb, depth, params=p)      # fused forward (RGB, depth, mask)
-        w.unwarp_normals(normals, params=p)    # fused inverse (gather, R^T, normalise)
+        fwd = w.warp_rgbd(rgb, depth, params=p)      # fused forward (RGB, depth, mask)
+        return fwd, w.unwarp_normals(normals, params=p)    # fused inverse (gather, R^T, normalise)
 
     def barrier():
         if world > 1:
@@ -414,10 +435,13 @@ def run_ours(args):
     e_start, e_end = ev_end[0], ev_end[K]
     e_start.record()
     for k in range(K):
+        # the previous step's outputs go back to the allocator first: the blocks step() used in the warm-up are reused, no
+        # allocation from the device inside the timed region; the last step's outputs stay for --dump-outputs
+        fwd = inv = None
         p = w.prepare(g, a)
-        w.warp_rgbd(rgb, depth, params=p)
+        fwd = w.warp_rgbd(rgb, depth, params=p)
         ev_mid[k].record()
-        w.unwarp_normals(normals, params=p)
+        inv = w.unwarp_normals(normals, params=p)
         ev_end[k + 1].record()
     barrier()
     launches = lib.vidc_launch_count() - launches0
@@ -428,6 +452,9 @@ def run_ours(args):
     step_ms = [ev_end[k].elapsed_time(ev_end[k + 1]) for k in range(K)]  # SURVEY section 8(d): report median and min too
     # frames are independent: aggregate = sum(frames) / max(elapsed) over ranks, no data-path collective
     _, elapsed_ms, value = sharding.aggregate_throughput(B * K, elapsed_ms, dev)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"homography": fwd[0], "rgb_w": fwd[1], "depth_w": fwd[2], "mask": fwd[3], "normals": inv[1]})
+    del fwd, inv
 
     # ---- informational: the same step with the per-frame kernel inside each call (I_g / I_a handed to both entry points) ----
     def step_per_call_params():
@@ -641,7 +668,14 @@ def main():
     ap.add_argument("--steps", type=int, default=50)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (see dump_outputs; --impl ours only). "
+                         "dumps/ in the tree is git-ignored")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours only")
     if args.impl == "reference":
         run_reference(args)
     else:

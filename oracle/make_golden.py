@@ -5,9 +5,10 @@ container.  Run once here; the vectors are committed because /root/reference can
     python -m oracle.make_golden
 
 What is frozen
-  golden_tiny.npz   64x48 camera, 12 edge-case + 6 random frames: every intermediate and output IN FULL
-                    (H, R, Hinv, both sampler grids, warped RGB, warped depth bilinear / nearest, un-normalised
-                    and normalised un-warped normals, validity mask, nearest pyramid masks, loss statistics).
+  golden_tiny.npz   64x48 camera, 12 edge-case + 6 random frames: every intermediate and output (H, R, Hinv,
+                    both sampler grids, warped RGB, warped depth bilinear / nearest, un-normalised and normalised
+                    un-warped normals, validity mask, nearest pyramid masks, loss statistics) IN FULL, except the
+                    TINY_DIGESTS arrays, stored like the S configs below so that the file stays under 1 MB.
   golden_demo.npz   BASELINE config 1: the eight demo frames' real gravity + klt tracks through loader code and warper
   golden_tiny_bicubic.npz  64x48, interp_mode='bicubic' outputs IN FULL
   golden_tiny_special.npz  64x48, signed zeros / denormals / inf / NaN inputs: every output IN FULL
@@ -52,7 +53,11 @@ def load_normal_utils():
     return mod
 
 
-def run_reference(cam_name, I_g, I_a, seed, full):
+TINY_DIGESTS = ("grid", "inv_grid", "y_rgb", "z")     # the largest, least compressible arrays of golden_tiny.npz
+
+
+def run_reference(cam_name, I_g, I_a, seed, digest=None):
+    """digest: names of the large tensors stored as SHA-256 + samples (None: all of them); the others are stored in full."""
     Wref = load_reference_class("cpu")
     fx, fy, cx, cy = C.CAMERAS[cam_name]
     w = Wref(fx=fx, fy=fy, cx=cx, cy=cy)
@@ -84,16 +89,16 @@ def run_reference(cam_name, I_g, I_a, seed, full):
            "y_sdepth_nearest": ydn.numpy(), "z": z.numpy(), "zn": zn.numpy(), "mask": mask.numpy().astype(np.uint8)}
     for i, p in enumerate(pyr):
         big[f"pyr{i}"] = p.numpy().astype(np.uint8)
-    if full:
-        out.update(big)
-    else:
-        for k, v in big.items():
-            flat = v.reshape(-1)
-            idx = sample_idx(flat.size)
-            out[k + "_sha256"] = np.array(sha(v))
-            out[k + "_idx"] = idx.astype(np.int64)
-            out[k + "_val"] = flat[idx]
-            out[k + "_shape"] = np.array(v.shape, np.int64)
+    for k, v in big.items():
+        if digest is not None and k not in digest:
+            out[k] = v
+            continue
+        flat = v.reshape(-1)
+        idx = sample_idx(flat.size)
+        out[k + "_sha256"] = np.array(sha(v))
+        out[k + "_idx"] = idx.astype(np.int64)
+        out[k + "_val"] = flat[idx]
+        out[k + "_shape"] = np.array(v.shape, np.int64)
     return out
 
 
@@ -306,18 +311,18 @@ def main():
         np.savez_compressed(os.path.join(OUT, "golden_tiny_loss_backward.npz"), **loss_backward_golden())
         return
     np.savez_compressed(os.path.join(OUT, "golden_tiny_loss_backward.npz"), **loss_backward_golden())
-    # tiny: edge cases + random, everything in full
+    # tiny: edge cases + random, everything but TINY_DIGESTS in full
     eg, ea = C.edge_case_gravity()
     rg, ra = C.random_gravity(6, seed=4321, roll_deg=60, pitch_deg=45)
     np.savez_compressed(os.path.join(OUT, "golden_tiny.npz"),
-                        **run_reference("tiny", np.concatenate([eg, rg]), np.concatenate([ea, ra]), seed=7, full=True))
+                        **run_reference("tiny", np.concatenate([eg, rg]), np.concatenate([ea, ra]), seed=7, digest=TINY_DIGESTS))
     # full-resolution configs: digests
     for name, (B, roll, pitch, seed) in {"S1": (6, 30, 30, 1), "S2": (3, 30, 30, 2), "S3": (3, 75, 40, 3)}.items():
         I_g, I_a = C.random_gravity(B, seed=1234, roll_deg=roll, pitch_deg=pitch)
         if name == "S3":
             xg, xa = C.extreme_roll_gravity(3, seed=5)
             I_g, I_a = np.concatenate([I_g, xg]), np.concatenate([I_a, xa])
-        np.savez_compressed(os.path.join(OUT, f"golden_{name}.npz"), **run_reference(name, I_g, I_a, seed, full=False))
+        np.savez_compressed(os.path.join(OUT, f"golden_{name}.npz"), **run_reference(name, I_g, I_a, seed))
     np.savez_compressed(os.path.join(OUT, "golden_tiny_backward.npz"), **backward_golden())
     np.savez_compressed(os.path.join(OUT, "golden_rasterize.npz"), **rasterize_golden())
     np.savez_compressed(os.path.join(OUT, "golden_tiny_special.npz"), **special_values_golden())
