@@ -201,10 +201,24 @@ int vidc_unwarp_normals(const vidc_camera *cam, const vidc_image *x, const float
    through F.grid_sample, :152 / :251, and the bmm at :253).  grad_out: (B,C,cam.H,cam.W), any strides.
    inverse == 0: backward of warp_with_gravity_center_aligned  -> d_grad_in (B,C,Hin,Win) contiguous, zeroed by the call;
    inverse != 0: backward of inverse_warp_normal_image_...     -> grad w.r.t. x (B,3,H,W): scatter of R * grad_out.
-   Scatter-add with atomics (as ATen's CUDA backward): results agree with autograd to rounding, not bit-for-bit. */
+   Scatter-add with atomics (as ATen's CUDA backward): results agree with autograd to rounding, not bit-for-bit, and may differ
+   in the last bits from run to run; vidc_warp_backward_ordered below is the deterministic variant. */
 int vidc_warp_backward(const vidc_camera *cam, const vidc_image *grad_out, const float *d_Ig, const float *d_Ia,
                        int32_t B_gravity, int32_t inverse, vidc_interp mode, vidc_frame_params *d_params_ws,
                        float *d_grad_in, int32_t Hin, int32_t Win, void *stream);
+
+/* The same backward with ONE fixed summation order, so the gradient is a pure function of the inputs (bit-reproducible from
+   run to run, at any batch position, on any stream).  Same arguments, checks and result layout as vidc_warp_backward; every
+   element of d_grad_in is written (no zeroing needed).  Order contract: each element of grad_in starts at +0 and receives, in
+   output row-major order (Y, then X), the contribution of every output pixel that has it among its in-bounds taps: the
+   product w_tap * g rounded, then added with a separate rounding (no FMA).  A pixel reaches an element through at most one
+   tap (bilinear: nw, ne, sw, se; nearest: the rint tap with weight 1, contribution g itself).  Coordinates and weights are
+   the forward warps' bits; a non-finite coordinate contributes nothing; inverse != 0 first rotates g <- R g (k-ascending FMA
+   chain from +0).  This is the order of a serial scatter loop (tests/harness/backward_scatter.c).  A gather
+   kernel, one CTA per 32x32 tile of grad_in: no global atomics. */
+int vidc_warp_backward_ordered(const vidc_camera *cam, const vidc_image *grad_out, const float *d_Ig, const float *d_Ia,
+                               int32_t B_gravity, int32_t inverse, vidc_interp mode, vidc_frame_params *d_params_ws,
+                               float *d_grad_in, int32_t Hin, int32_t Win, void *stream);
 
 /* Replaces image_sampler_forward_inverse (:158-214) including the aspect guard (:178-187).
    d_Rt (B,3,3), d_grid / d_inv_grid (B,H,W,2) contiguous; any may be NULL. */

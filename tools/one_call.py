@@ -13,3 +13,15 @@ t = lambda x: torch.from_numpy(x).to(dev)
 out = w.warp_rgbd(t(rgb), t(depth), t(I_g), t(I_a))
 torch.cuda.synchronize()
 print("ok", float(out[1].sum()))
+# one backward call of each variant (atomic scatter, fixed-order gather), forward and inverse warp, bilinear and nearest
+for det in (False, True):
+    w.deterministic_backward = det
+    for mode in ("bilinear", "nearest"):
+        x = t(rgb).requires_grad_(True)
+        w.warp_with_gravity_center_aligned(x, t(I_g), t(I_a), interp_mode=mode)[1].sum().backward()
+        torch.cuda.synchronize()
+        print("backward", "ordered" if det else "atomic", mode, float(x.grad.sum()))
+    n = t(nrm).requires_grad_(True)
+    w.inverse_warp_normal_image_with_gravity_center_aligned(n, t(I_g), t(I_a))[1].sum().backward()
+    torch.cuda.synchronize()
+    print("backward", "ordered" if det else "atomic", "inverse", float(n.grad.sum()))

@@ -62,6 +62,8 @@ _SIGNATURES = {
                                            ctypes.c_void_p, c_f32p, _P(VidcImage), ctypes.c_void_p, ctypes.c_void_p]),
     "vidc_warp_backward": (ctypes.c_int, [_P(VidcCamera), _P(VidcImage), c_f32p, c_f32p, ctypes.c_int32, ctypes.c_int32, ctypes.c_int,
                                           ctypes.c_void_p, c_f32p, ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p]),
+    "vidc_warp_backward_ordered": (ctypes.c_int, [_P(VidcCamera), _P(VidcImage), c_f32p, c_f32p, ctypes.c_int32, ctypes.c_int32,
+                                                  ctypes.c_int, ctypes.c_void_p, c_f32p, ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p]),
     "vidc_sampler_forward_inverse": (ctypes.c_int, [_P(VidcCamera), c_f32p, c_f32p, ctypes.c_int32, ctypes.c_void_p, c_f32p,
                                                     c_f32p, c_f32p, ctypes.c_void_p]),
     "vidc_warp_normals_forward": (ctypes.c_int, [_P(VidcCamera), _P(VidcImage), c_f32p, c_f32p, ctypes.c_int32, ctypes.c_int,

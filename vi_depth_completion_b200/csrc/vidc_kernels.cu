@@ -13,6 +13,7 @@
 //   kernels_shear_cl.cuh                the same for channels-last three-channel images (12-byte pixels, (96, 32) staging tile)
 //   kernels_box.cuh                     inverse warp with the footprint staged in shared memory (opt-in, VIDC_INV_BOX=1)
 //   kernels_backward.cuh                scatter-add backward
+//   kernels_backward_ordered.cuh        gather backward in one fixed summation order (deterministic)
 //   kernels_sparse.cuh                  sparse depth warped analytically (row f2)
 //   tma_stage.cuh                       TMA / mbarrier PTX wrappers (bulk tensor loads and stores)
 //   kernels_tma.cuh                     opt-in TMA-staged LOAD variants (VIDC_TMA=1)
@@ -35,6 +36,7 @@
 #include "kernels_shear.cuh"
 #include "kernels_shear_cl.cuh"
 #include "kernels_backward.cuh"
+#include "kernels_backward_ordered.cuh"
 #include "kernels_sparse.cuh"
 #include "kernels_packed.cuh"
 #include "kernels_tma.cuh"
@@ -1188,9 +1190,10 @@ int vidc_warp_rgbd_packed(const vidc_camera* cam, const float* d_in, int32_t B, 
     return VIDC_OK;
 }
 
-int vidc_warp_backward(const vidc_camera* cam, const vidc_image* grad_out, const float* d_Ig, const float* d_Ia,
-                       int32_t B_gravity, int32_t inverse, vidc_interp mode, vidc_frame_params* d_params_ws,
-                       float* d_grad_in, int32_t Hin, int32_t Win, void* stream) {
+namespace {
+// argument checks shared by the scatter and the ordered backward
+int check_warp_backward(const vidc_camera* cam, const vidc_image* grad_out, int32_t B_gravity, int32_t inverse, vidc_interp mode,
+                        int32_t Hin, int32_t Win) {
     VIDC_TRY(check_cam(cam));
     VIDC_TRY(check_image(grad_out, "grad_out", 1, 1 << 30));
     if (grad_out->c > 4) return fail(VIDC_ERR_INVALID_ARGUMENT, "grad_out: at most 4 channels per call (3 for the inverse warp); split wider feature maps into groups");
@@ -1199,6 +1202,14 @@ int vidc_warp_backward(const vidc_camera* cam, const vidc_image* grad_out, const
     if (inverse && (grad_out->c != 3 || Hin != cam->H || Win != cam->W)) return fail(VIDC_ERR_INVALID_ARGUMENT, "inverse backward needs (B,3,H,W)");
     if (mode != VIDC_BILINEAR && mode != VIDC_NEAREST) return fail(VIDC_ERR_INVALID_ARGUMENT, "unknown interp mode %d", (int)mode);
     if (Hin <= 0 || Win <= 0 || (long long)Hin * Win * grad_out->c >= (1LL << 31)) return fail(VIDC_ERR_INVALID_ARGUMENT, "bad input size");
+    return VIDC_OK;
+}
+}  // namespace
+
+int vidc_warp_backward(const vidc_camera* cam, const vidc_image* grad_out, const float* d_Ig, const float* d_Ia,
+                       int32_t B_gravity, int32_t inverse, vidc_interp mode, vidc_frame_params* d_params_ws,
+                       float* d_grad_in, int32_t Hin, int32_t Win, void* stream) {
+    VIDC_TRY(check_warp_backward(cam, grad_out, B_gravity, inverse, mode, Hin, Win));
     if (grad_out->n == 0) return VIDC_OK;
     if (!d_grad_in) return fail(VIDC_ERR_INVALID_ARGUMENT, "null grad_in");
     cudaStream_t st = (cudaStream_t)stream;
@@ -1212,6 +1223,26 @@ int vidc_warp_backward(const vidc_camera* cam, const vidc_image* grad_out, const
     else
         warp_backward_kernel<false><<<grid2d(cam->W, cam->H, grad_out->n, blk), blk, 0, st>>>(d_params_ws, cam_const(cam), view_in(grad_out), C,
                                                                                           (int)mode, d_grad_in, (long long)C * Hin * Win, Hin * Win, Hin, Win);
+    VIDC_LAUNCH_CHECK();
+    return VIDC_OK;
+}
+
+int vidc_warp_backward_ordered(const vidc_camera* cam, const vidc_image* grad_out, const float* d_Ig, const float* d_Ia,
+                               int32_t B_gravity, int32_t inverse, vidc_interp mode, vidc_frame_params* d_params_ws,
+                               float* d_grad_in, int32_t Hin, int32_t Win, void* stream) {
+    VIDC_TRY(check_warp_backward(cam, grad_out, B_gravity, inverse, mode, Hin, Win));
+    if (grad_out->n == 0) return VIDC_OK;
+    if (!d_grad_in) return fail(VIDC_ERR_INVALID_ARGUMENT, "null grad_in");
+    cudaStream_t st = (cudaStream_t)stream;
+    const int C = grad_out->c;
+    VIDC_TRY(launch_params(cam, d_Ig, d_Ia, grad_out->n, d_params_ws, st));
+    const dim3 grd((Win + BWO_TILE - 1) / BWO_TILE, (Hin + BWO_TILE - 1) / BWO_TILE, grad_out->n);    // every grad_in element once
+    if (inverse)
+        warp_backward_ordered_kernel<true><<<grd, 256, 0, st>>>(d_params_ws, cam_const(cam), view_in(grad_out), C, (int)mode, d_grad_in,
+                                                                (long long)C * Hin * Win, Hin * Win, Hin, Win);
+    else
+        warp_backward_ordered_kernel<false><<<grd, 256, 0, st>>>(d_params_ws, cam_const(cam), view_in(grad_out), C, (int)mode, d_grad_in,
+                                                                 (long long)C * Hin * Win, Hin * Win, Hin, Win);
     VIDC_LAUNCH_CHECK();
     return VIDC_OK;
 }

@@ -12,7 +12,9 @@ Differences from the reference that are deliberate (see DESIGN.md):
   * nothing synchronises with the host (the reference reads dozens of device scalars per frame);
   * any canvas size works (the reference hard-codes 240*320 staging buffers, :121-122);
   * gradients: the two reference-shaped methods are differentiable w.r.t. the image (vidc_warp_backward, bilinear /
-    nearest); the fused entry points and interp_mode='bicubic' are forward-only and raise NotImplementedError in backward;
+    nearest; vidc_warp_backward_ordered, bit-reproducible, under torch.use_deterministic_algorithms(True) or with
+    deterministic_backward = True); the fused entry points and interp_mode='bicubic' are forward-only and raise
+    NotImplementedError in backward;
   * there is NO CPU / PyTorch fallback: CPU tensors raise RuntimeError.
 """
 import ctypes
@@ -66,7 +68,9 @@ def _gravity(I_g: torch.Tensor, I_a: torch.Tensor, device):
 class _WarpFn(torch.autograd.Function):
     """Connects the forward-only fused kernels to autograd: backward is the scatter kernel of vidc_warp_backward
     (gradient w.r.t. the sampled image only -- the gravity tensors come from the DataLoader and carry no gradient,
-    exactly as in the reference, where only self.cnn parameters are optimised, network_run.py:101)."""
+    exactly as in the reference, where only self.cnn parameters are optimised, network_run.py:101).  Under
+    torch.use_deterministic_algorithms(True), or with the warper's deterministic_backward set to True, it is the gather
+    kernel of vidc_warp_backward_ordered instead: one fixed summation order, the same bits in every run."""
 
     @staticmethod
     def forward(ctx, x, out, warper, g, a, inverse, mode):
@@ -81,15 +85,18 @@ class _WarpFn(torch.autograd.Function):
         w = ctx.warper
         B, C, Hin, Win = ctx.in_shape
         grad = grad.float()
+        det = w.deterministic_backward
+        entry = lib().vidc_warp_backward_ordered if (torch.are_deterministic_algorithms_enabled() if det is None else det) \
+            else lib().vidc_warp_backward
         groups = []
         for c0 in range(0, C, 4):                              # feature maps: the scatter kernel takes <= 4 planes per call
             gc = grad[:, c0:c0 + 4]
             gxc = torch.empty((B, gc.shape[1], Hin, Win), dtype=torch.float32, device=grad.device)
             gi = _image(gc)
             with torch.cuda.device(grad.device):
-                check(lib().vidc_warp_backward(ctypes.byref(w._cam), ctypes.byref(gi), g.data_ptr(), a.data_ptr(), g.shape[0],
-                                               1 if ctx.inverse else 0, ctx.mode, w._params_ws(g.shape[0], grad.device).data_ptr(),
-                                               gxc.data_ptr(), Hin, Win, _stream_ptr(grad.device)))
+                check(entry(ctypes.byref(w._cam), ctypes.byref(gi), g.data_ptr(), a.data_ptr(), g.shape[0],
+                            1 if ctx.inverse else 0, ctx.mode, w._params_ws(g.shape[0], grad.device).data_ptr(),
+                            gxc.data_ptr(), Hin, Win, _stream_ptr(grad.device)))
             groups.append(gxc)
         gx = groups[0] if len(groups) == 1 else torch.cat(groups, 1)
         return gx, None, None, None, None, None, None
@@ -168,6 +175,9 @@ class Warping2DOFAlignment:
         self._const_cache = {}
         self._ws_bytes = {}
         self._intr = (float(fx), float(fy), float(cx), float(cy))      # operator arguments of the torch C++ front end
+        # backward of the two reference-shaped methods: None follows torch.are_deterministic_algorithms_enabled(), True always
+        # takes the fixed-order gather kernel (bit-reproducible gradients), False always the atomic scatter kernel
+        self.deterministic_backward = None
 
     # ---- constant tensors the reference exposes as attributes (:15-24), built lazily ----------
     def _const(self, name):
