@@ -559,7 +559,7 @@ def test_special_values_match_oracle(cuda_device, oracle_mod, cam_name):
     _, z = w.inverse_warp_normal_image_with_gravity_center_aligned(_t(normals, cuda_device), g, a)
     _, nhat = w.unwarp_normals(_t(normals, cuda_device), g, a)
     from vi_depth_completion_b200 import normal_utils as NU
-    nhat2 = NU.Normalize(z)                                        # vidc_normalize3 (generic kernel)
+    nhat2 = NU.Normalize(z)                                        # vidc_normalize3 (contiguous, H*W % 4 == 0: vec4 kernel)
     with np.errstate(all="ignore"):
         _, oy = o.warp_with_gravity_center_aligned(rgb, I_g, I_a)
         _, oyd = o.warp_with_gravity_center_aligned(depth, I_g, I_a)

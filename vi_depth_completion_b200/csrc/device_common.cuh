@@ -28,6 +28,8 @@ struct CamConst {
 // norm.clamp_min(1e-12) of F.normalize (torch/nn/functional.py; surface_normal.py:170): unlike fmaxf(), a NaN
 // norm stays NaN, so every component of a vector holding one NaN comes out NaN, as in the reference.
 __device__ __forceinline__ float clamp_min_eps(float n) { return n < 1e-12f ? 1e-12f : n; }
+// torch's clamp_min (x < lo ? lo : x): keeps NaN, unlike fmaxf
+__device__ __forceinline__ float clamp_min_nan(float x, float lo) { return x < lo ? lo : x; }
 
 // ATen grid_sampler_2d, align_corners=False: ((g + 1) * size - 1) / 2 with the multiply-subtract
 // contracted into one fma, as both the CPU and the CUDA builds of ATen compile it.

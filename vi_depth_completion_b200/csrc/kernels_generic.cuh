@@ -325,7 +325,7 @@ normal_stats_kernel(ImgView gt, ImgView pred, ImgView mask, int normalize_predic
                fabs((double)(n2 * m) - (double)(g2 * m));
         // F.cosine_similarity(pred, gt, dim=1), eps = 1e-8 on each norm
         const float ng = sqrtf((g0 * g0 + g1 * g1) + g2 * g2);
-        s_cos = (double)(((r0 * g0 + r1 * g1) + r2 * g2) / (fmaxf(nr, 1e-8f) * fmaxf(ng, 1e-8f)));
+        s_cos = (double)(((r0 * g0 + r1 * g1) + r2 * g2) / (clamp_min_nan(nr, 1e-8f) * clamp_min_nan(ng, 1e-8f)));
     }
 #pragma unroll
     for (int off = 16; off > 0; off >>= 1) {
@@ -351,8 +351,15 @@ normal_stats_kernel(ImgView gt, ImgView pred, ImgView mask, int normalize_predic
 //   mode 1: the same with normalize_prediction=False                     (n^ = pred)
 //   mode 2: compute_normal_vectors_loss_l2                               loss = -sum(cos_sim(pred, g)) / sum(m) (:7-10, NOT masked)
 // stats[1] = sum(mask) from the forward pass (vidc_normal_stats); *grad_loss = upstream gradient of the scalar loss.
-// Chain rules are torch's: L1Loss(sum) -> sign(a - b) with sign(0) = 0; F.normalize -> x / norm.clamp_min(1e-12), the clamp
-// passing gradient only where norm >= 1e-12; cosine_similarity clamps each norm at 1e-8.  Channels >= 3 of pred get zeros.
+// Torch's chain, in torch's order (N = clamped norm, |r| = unclamped norm, q_c = (r_c / N) / N):
+//   L1Loss(sum)      -> sign(a - b), with sign(0) = sign(NaN) = 0
+//   x / N            -> dx_c = grad_c / N and dN = -sum_c grad_c q_c   (div backward: -grad * ((x / N) / N); N^2 and N^3
+//                       are never formed, so nothing overflows before the norm itself does at |r| ~ 1.8e19)
+//   F.normalize      -> N = |r|.clamp_min(1e-12): dN reaches the norm only where |r| >= 1e-12 (clamp_min backward)
+//   cosine_similarity-> N = |r|.clamp_min_(1e-8) under no_grad: the clamp is invisible to autograd, so dN always reaches
+//                       the norm, and the radial term survives for every |r| > 0 (the division uses the clamped norm)
+//   vector_norm      -> dr_c += dN * (r_c / |r|), where |r| == 0 gives 0
+// The clamps keep NaN (as torch's clamp_min does), so a NaN in pred gives a NaN gradient.  Channels >= 3 of pred get zeros.
 __global__ void __launch_bounds__(256)
 normal_loss_backward_kernel(ImgView gt, ImgView pred, ImgView mask, int mode, const double* __restrict__ stats,
                             const float* __restrict__ grad_loss, ImgViewOut gp) {
@@ -368,37 +375,29 @@ normal_loss_backward_kernel(ImgView gt, ImgView pred, ImgView mask, int mode, co
     const float r[3] = {__ldg(pp), __ldg(pp + pred.sc), __ldg(pp + 2 * pred.sc)};
     const float g[3] = {__ldg(pg), __ldg(pg + gt.sc), __ldg(pg + 2 * gt.sc)};
     const float nr = sqrtf((r[0] * r[0] + r[1] * r[1]) + r[2] * r[2]);
-    float d[3];
+    float dx[3], nc;          // gradient reaching x / N, and the clamped norm N
+    float dN = 0.0f;          // gradient reaching the unclamped norm
     if (mode == 2) {
-        const float ng = fmaxf(sqrtf((g[0] * g[0] + g[1] * g[1]) + g[2] * g[2]), 1e-8f);
-        const float nrc = fmaxf(nr, 1e-8f);
-        const float dot = (r[0] * g[0] + r[1] * g[1]) + r[2] * g[2];
-        const float k = nr >= 1e-8f ? dot / (nrc * nrc * nrc * ng) : 0.0f;     // d(1/|r|)/dr term, absent while the norm is clamped
+        const float ng = clamp_min_nan(sqrtf((g[0] * g[0] + g[1] * g[1]) + g[2] * g[2]), 1e-8f);
+        nc = clamp_min_nan(nr, 1e-8f);
 #pragma unroll
-        for (int c = 0; c < 3; ++c) d[c] = -go * (g[c] / (nrc * ng) - k * r[c]);
+        for (int c = 0; c < 3; ++c) dx[c] = -go * (g[c] / ng);
     } else {
-        float n[3] = {r[0], r[1], r[2]};
-        const float nn = clamp_min_eps(nr);
-        if (mode == 0) { n[0] = r[0] / nn; n[1] = r[1] / nn; n[2] = r[2] / nn; }
-        float dn[3];
+        nc = clamp_min_eps(nr);
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
-            const float diff = n[c] * m - g[c] * m;
+            const float n = mode == 0 ? r[c] / nc : r[c];
+            const float diff = n * m - g[c] * m;
             const float sg = diff > 0.0f ? 1.0f : (diff < 0.0f ? -1.0f : 0.0f);  // torch.sign: 0 for 0 and for NaN
-            dn[c] = go * sg * m;
-        }
-        if (mode == 0) {
-            const float dd = (dn[0] * r[0] + dn[1] * r[1]) + dn[2] * r[2];
-            const float k = nr >= 1e-12f ? dd / (nn * nn * nr) : 0.0f;
-#pragma unroll
-            for (int c = 0; c < 3; ++c) d[c] = dn[c] / nn - k * r[c];
-        } else {
-#pragma unroll
-            for (int c = 0; c < 3; ++c) d[c] = dn[c];
+            dx[c] = go * sg * m;
         }
     }
+    if (mode != 1) {
+        const float dd = (dx[0] * ((r[0] / nc) / nc) + dx[1] * ((r[1] / nc) / nc)) + dx[2] * ((r[2] / nc) / nc);
+        if (mode == 2 || nr >= 1e-12f) dN = -dd;
+    }
 #pragma unroll
-    for (int c = 0; c < 3; ++c) po[c * gp.sc] = d[c];
+    for (int c = 0; c < 3; ++c) po[c * gp.sc] = mode == 1 ? dx[c] : dx[c] / nc + dN * (nr == 0.0f ? 0.0f : r[c] / nr);
     for (int c = 3; c < gp.c; ++c) po[c * gp.sc] = 0.0f;
 }
 
