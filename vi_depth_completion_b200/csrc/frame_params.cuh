@@ -259,6 +259,37 @@ VIDC_HD bool inv_division_proven(const vidc_frame_params& p, const vidc_camera& 
     return ok && (slo > 0.0f || shi < 0.0f) && m >= 0x1p-10f * M;
 }
 
+// Canvas box of the inverse warp's L2 prefetch (kernels_shear.cuh: inv_prefetch_tile): out = {x0, y0, x1, y1} (inclusive,
+// clipped to the canvas) holds both bilinear taps of every camera pixel of [X0, X1] x [Y0, Y1].  Only for frames that pass
+// inv_division_proven: there s keeps its sign over the image, so (as in inv_rect_box) the mapped rectangle lies in the box of
+// its mapped corners; the 2 px margin holds the +1 taps and the difference between this evaluation (one approximate
+// reciprocal per corner) and the kernels' correctly rounded one.  A hint only.  false: nothing to prefetch (non-finite, or off the canvas).
+VIDC_HD bool inv_prefetch_box(const float* Hm, float px_min, float py_min, float kw, float kh, float cx, float cy, float ihw,
+                              float ihh, int W, int H, int X0, int Y0, int X1, int Y1, int out[4]) {
+    float xlo = 3.0e38f, xhi = -3.0e38f, ylo = 3.0e38f, yhi = -3.0e38f;
+#pragma unroll 1
+    for (int c = 0; c < 4; ++c) {                                     // not unrolled: few live registers in the kernels' prologue
+        const float X = (float)((c & 1) ? X1 : X0), Y = (float)((c >> 1) ? Y1 : Y0);
+        const float u = fmaf(Hm[1], Y, Hm[0] * X) + Hm[2];
+        const float v = fmaf(Hm[4], Y, Hm[3] * X) + Hm[5];
+        const float s = fmaf(Hm[7], Y, Hm[6] * X) + Hm[8];
+#ifdef __CUDA_ARCH__
+        const float r = __fdividef(1.0f, s);                          // 2 ulp, and no slow-path call in the kernels' prologue
+#else
+        const float r = 1.0f / s;
+#endif
+        const float ix = fmaf(ihw * (kw * (u * r - px_min) - cx) + 1.0f, (float)W, -1.0f) * 0.5f;
+        const float iy = fmaf(ihh * (kh * (v * r - py_min) - cy) + 1.0f, (float)H, -1.0f) * 0.5f;
+        xlo = fminf(xlo, ix); xhi = fmaxf(xhi, ix); ylo = fminf(ylo, iy); yhi = fmaxf(yhi, iy);
+    }
+    if (!(xlo > -1.0e6f && xhi < 1.0e6f && ylo > -1.0e6f && yhi < 1.0e6f)) return false;       // also rejects NaN
+    int x0 = (int)floorf(xlo) - 2, x1 = (int)floorf(xhi) + 3, y0 = (int)floorf(ylo) - 2, y1 = (int)floorf(yhi) + 3;
+    x0 = x0 < 0 ? 0 : x0; y0 = y0 < 0 ? 0 : y0;
+    x1 = x1 > W - 1 ? W - 1 : x1; y1 = y1 > H - 1 ? H - 1 : y1;
+    out[0] = x0; out[1] = y0; out[2] = x1; out[3] = y1;
+    return x0 <= x1 && y0 <= y1;
+}
+
 VIDC_HD void inv_tile_boxes(const vidc_frame_params& p, const vidc_camera& cam, int tx, int ty, bool div_proven, uint32_t out[4]) {
     const int X0 = tx * 32, Y0 = ty * 32;
     const int X1 = (X0 + 31 < cam.W - 1) ? X0 + 31 : cam.W - 1, Y1 = (Y0 + 31 < cam.H - 1) ? Y0 + 31 : cam.H - 1;

@@ -89,6 +89,18 @@ __device__ __forceinline__ void tma_store_commit_and_wait_read() {
     asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
 }
 
+// ---- tiled bulk tensor PREFETCH into L2 (SASS UTMAPF): the L2 prefetch of the sheared kernels -------------------------------
+// One instruction from one thread asks the TMA unit for a whole box; no shared memory, no barrier, nothing to wait for, a hint
+// only.  Elements of the box outside the tensor are not fetched.
+__device__ __forceinline__ void tma_prefetch_l2_4d(const CUtensorMap* map, int x, int y, int c, int n) {
+    asm volatile("cp.async.bulk.prefetch.tensor.4d.L2.global.tile [%0, {%1, %2, %3, %4}];"
+                 ::"l"((unsigned long long)map), "r"(x), "r"(y), "r"(c), "r"(n) : "memory");
+}
+__device__ __forceinline__ void tma_prefetch_l2_3d(const CUtensorMap* map, int x, int y, int n) {
+    asm volatile("cp.async.bulk.prefetch.tensor.3d.L2.global.tile [%0, {%1, %2, %3}];"
+                 ::"l"((unsigned long long)map), "r"(x), "r"(y), "r"(n) : "memory");
+}
+
 // plain arrive (no transaction bytes) and arrive from a consumer warp
 __device__ __forceinline__ void mbar_arrive(unsigned long long* bar) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");

@@ -140,6 +140,22 @@ int fwd_prefetch_pct() {
     static const int v = [] { const char* e = getenv("VIDC_FWD_PF_WAVES_X100"); return e ? atoi(e) : 8; }();
     return v;
 }
+// Bulk tensor form of the sheared kernels' L2 prefetch (kernels_shear.cuh: PrefetchMaps): on unless VIDC_PF_BULK=0, which
+// restores the per-thread forward prefetch and turns the inverse prefetch off (A/B runs of one build).
+bool pf_bulk_enabled() {
+    static const bool v = [] { const char* e = getenv("VIDC_PF_BULK"); return !(e && e[0] == '0'); }();
+    return v;
+}
+// L2 prefetch distance of the sheared inverse kernel (bulk form only), percent of a wave of resident CTAs
+// (VIDC_INV_PF_WAVES_X100, 0 = off).  16 %: with it the inverse takes 0.438 ms, without it 0.448 ms (profiles/r4_history.md).
+int inv_prefetch_pct() {
+    static const int v = [] { const char* e = getenv("VIDC_INV_PF_WAVES_X100"); return e ? atoi(e) : 16; }();
+    return v;
+}
+int sm_count() {
+    static const int n = [] { int dev = 0, k = 148; cudaGetDevice(&dev); cudaDeviceGetAttribute(&k, cudaDevAttrMultiProcessorCount, dev); return k; }();
+    return n;
+}
 int launch_params_tiles(const vidc_camera* cam, const float* d_Ig, const float* d_Ia, int B, vidc_frame_params* d_params,
                         cudaStream_t st, float* d_H_out) {
     if (B == 0) return VIDC_OK;
@@ -216,22 +232,24 @@ bool encode_image_map(CUtensorMap* map, const vidc_image* im, int box_h, int box
                CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 // Output tensor maps of the TMA write-out (kernels_shear.cuh: StoreMaps): (W, H, C, N) fp32 planes, box (32, 32, C, 1), or
-// (W, H, N) for a single plane.  false if the view cannot be described (strides not multiples of 16 bytes, ...).
-bool encode_store_map(CUtensorMap* map, float* data, int W, int H, int C, int N, int64_t sh, int64_t sc, int64_t sn, bool plane3d = false) {
+// (W, H, N) for a single plane; the input maps of the bulk L2 prefetch (PrefetchMaps) are the same views with a (bw, bh) box.
+// false if the view cannot be described (strides not multiples of 16 bytes, ...).
+bool encode_store_map(CUtensorMap* map, float* data, int W, int H, int C, int N, int64_t sh, int64_t sc, int64_t sn, bool plane3d = false,
+                      int bw = 32, int bh = 32) {
     PFN_encodeTiled enc = tma_encoder();
     if (!enc || ((uintptr_t)data & 15) || (sh & 3) || (sc & 3) || (sn & 3) || sh <= 0 || sn <= 0) return false;
     const cuuint32_t estr[4] = {1, 1, 1, 1};
     if (plane3d) {                                   // StoreMaps::dep: one plane per frame, stored with the 3-D instruction
         const cuuint64_t dims[3] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
         const cuuint64_t strides[2] = {(cuuint64_t)sh * 4, (cuuint64_t)sn * 4};
-        const cuuint32_t box[3] = {32, 32, 1};
+        const cuuint32_t box[3] = {(cuuint32_t)bw, (cuuint32_t)bh, 1};
         return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, data, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                    CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
     }
     if (sc <= 0) return false;
     const cuuint64_t dims[4] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)C, (cuuint64_t)N};
     const cuuint64_t strides[3] = {(cuuint64_t)sh * 4, (cuuint64_t)sc * 4, (cuuint64_t)sn * 4};
-    const cuuint32_t box[4] = {32, 32, (cuuint32_t)C, 1};
+    const cuuint32_t box[4] = {(cuuint32_t)bw, (cuuint32_t)bh, (cuuint32_t)C, 1};
     return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, data, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
@@ -324,36 +342,37 @@ void launch_unwarp_box(bool normalize, bool has_valid, dim3 grd, dim3 blk, cudaS
 }
 
 template <int GW, int GH>
-void launch_unwarp_shear(bool normalize, bool has_valid, bool ts, dim3 grd, dim3 blk, cudaStream_t st, const InvArgs& ia, const StoreMaps& sm) {
+void launch_unwarp_shear(bool normalize, bool has_valid, bool ts, dim3 grd, dim3 blk, cudaStream_t st, const InvArgs& ia, const StoreMaps& sm,
+                         const PrefetchMaps& pm) {
     if (ts && !has_valid) {
-        if (normalize) unwarp_normals_shear_kernel<GW, GH, true, false, true><<<grd, blk, 0, st>>>(ia, sm);
-        else unwarp_normals_shear_kernel<GW, GH, false, false, true><<<grd, blk, 0, st>>>(ia, sm);
+        if (normalize) unwarp_normals_shear_kernel<GW, GH, true, false, true><<<grd, blk, 0, st>>>(ia, sm, pm);
+        else unwarp_normals_shear_kernel<GW, GH, false, false, true><<<grd, blk, 0, st>>>(ia, sm, pm);
     } else if (normalize) {
-        if (has_valid) unwarp_normals_shear_kernel<GW, GH, true, true, false><<<grd, blk, 0, st>>>(ia, sm);
-        else unwarp_normals_shear_kernel<GW, GH, true, false, false><<<grd, blk, 0, st>>>(ia, sm);
+        if (has_valid) unwarp_normals_shear_kernel<GW, GH, true, true, false><<<grd, blk, 0, st>>>(ia, sm, pm);
+        else unwarp_normals_shear_kernel<GW, GH, true, false, false><<<grd, blk, 0, st>>>(ia, sm, pm);
     } else {
-        if (has_valid) unwarp_normals_shear_kernel<GW, GH, false, true, false><<<grd, blk, 0, st>>>(ia, sm);
-        else unwarp_normals_shear_kernel<GW, GH, false, false, false><<<grd, blk, 0, st>>>(ia, sm);
+        if (has_valid) unwarp_normals_shear_kernel<GW, GH, false, true, false><<<grd, blk, 0, st>>>(ia, sm, pm);
+        else unwarp_normals_shear_kernel<GW, GH, false, false, false><<<grd, blk, 0, st>>>(ia, sm, pm);
     }
 }
 template <int GW, int GH>
-void launch_rgbd_shear(bool has_d, bool ts, dim3 grd, dim3 blk, cudaStream_t st, const FwdArgs& fa, const StoreMaps& sm) {
+void launch_rgbd_shear(bool has_d, bool ts, dim3 grd, dim3 blk, cudaStream_t st, const FwdArgs& fa, const StoreMaps& sm, const PrefetchMaps& pm) {
     if (ts) {
-        if (has_d) warp_rgbd_shear_kernel<GW, GH, true, true><<<grd, blk, 0, st>>>(fa, sm);
-        else warp_rgbd_shear_kernel<GW, GH, false, true><<<grd, blk, 0, st>>>(fa, sm);
+        if (has_d) warp_rgbd_shear_kernel<GW, GH, true, true><<<grd, blk, 0, st>>>(fa, sm, pm);
+        else warp_rgbd_shear_kernel<GW, GH, false, true><<<grd, blk, 0, st>>>(fa, sm, pm);
     } else {
-        if (has_d) warp_rgbd_shear_kernel<GW, GH, true, false><<<grd, blk, 0, st>>>(fa, sm);
-        else warp_rgbd_shear_kernel<GW, GH, false, false><<<grd, blk, 0, st>>>(fa, sm);
+        if (has_d) warp_rgbd_shear_kernel<GW, GH, true, false><<<grd, blk, 0, st>>>(fa, sm, pm);
+        else warp_rgbd_shear_kernel<GW, GH, false, false><<<grd, blk, 0, st>>>(fa, sm, pm);
     }
 }
 template <int GW, int GH>
-void launch_planes_shear(int C, bool ts, dim3 grd, dim3 blk, cudaStream_t st, const PlanesArgs& pa, const StoreMaps& sm) {
+void launch_planes_shear(int C, bool ts, dim3 grd, dim3 blk, cudaStream_t st, const PlanesArgs& pa, const StoreMaps& sm, const PrefetchMaps& pm) {
     if (ts) {
-        if (C == 3) warp_planes_shear_kernel<GW, GH, 3, true><<<grd, blk, 0, st>>>(pa, sm);
-        else warp_planes_shear_kernel<GW, GH, 1, true><<<grd, blk, 0, st>>>(pa, sm);
+        if (C == 3) warp_planes_shear_kernel<GW, GH, 3, true><<<grd, blk, 0, st>>>(pa, sm, pm);
+        else warp_planes_shear_kernel<GW, GH, 1, true><<<grd, blk, 0, st>>>(pa, sm, pm);
     } else {
-        if (C == 3) warp_planes_shear_kernel<GW, GH, 3, false><<<grd, blk, 0, st>>>(pa, sm);
-        else warp_planes_shear_kernel<GW, GH, 1, false><<<grd, blk, 0, st>>>(pa, sm);
+        if (C == 3) warp_planes_shear_kernel<GW, GH, 3, false><<<grd, blk, 0, st>>>(pa, sm, pm);
+        else warp_planes_shear_kernel<GW, GH, 1, false><<<grd, blk, 0, st>>>(pa, sm, pm);
     }
 }
 
@@ -504,22 +523,24 @@ __attribute__((visibility("hidden"))) int forward_group(const vidc_camera* cam, 
         PlanesArgs pa;
         pa.prm = d_params_ws; pa.cam = cam_const(cam);
         pa.x = x->data; pa.x_sn = x->sn; pa.y = y->data; pa.y_sn = y->sn; pa.mode = (int)mode;
-        pa.src_boxes = nullptr; pa.pf_x = pa.pf_y = pa.pf_z = 0;
-        if (tile_skip_enabled() && fwd_prefetch_pct() > 0 && (size_t)grd.x * grd.y <= 320) {     // the tiles kernel wrote the boxes
-            static const int sms = [] { int dev = 0, n = 148; cudaGetDevice(&dev); cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev); return n; }();
-            const int wave = (int)((long long)sms * VIDC_SHEAR_BLOCKS_FWD * fwd_prefetch_pct() / 100);
-            pa.src_boxes = reinterpret_cast<const uint4*>(d_params_ws + x->n);
-            pa.pf_x = wave % (int)grd.x; pa.pf_y = (wave / (int)grd.x) % (int)grd.y; pa.pf_z = wave / (int)(grd.x * grd.y);
-        }
+        pa.src_boxes = nullptr; pa.pf_x = pa.pf_y = pa.pf_z = 0; pa.pf_bulk = 0;
         bool done = true;
         const bool geom = planes(640, 480) || planes(320, 240) || planes(640, 489) || (cam->W % 32 == 0 && planes(cam->W, cam->H));
+        PrefetchMaps pm;
+        if (tile_skip_enabled() && fwd_prefetch_pct() > 0 && (size_t)grd.x * grd.y <= 320) {     // the tiles kernel wrote the boxes
+            const int wave = (int)((long long)sm_count() * VIDC_SHEAR_BLOCKS_FWD * fwd_prefetch_pct() / 100);
+            pa.src_boxes = reinterpret_cast<const uint4*>(d_params_ws + x->n);
+            pa.pf_x = wave % (int)grd.x; pa.pf_y = (wave / (int)grd.x) % (int)grd.y; pa.pf_z = wave / (int)(grd.x * grd.y);
+            pa.pf_bulk = geom && x->c == 3 && pf_bulk_enabled() &&
+                         encode_store_map(&pm.img, x->data, cam->W, cam->H, 3, x->n, x->sh, x->sc, x->sn, false, PF_FWD_BW, PF_FWD_BH);
+        }
         StoreMaps sm;
         const bool ts = geom && tma_store_enabled() &&
                         encode_store_map(&sm.img, y->data, cam->W, cam->H, x->c, x->n, y->sh, x->c == 1 ? (int64_t)cam->W * cam->H : y->sc, y->sn);
-        if (planes(640, 480)) launch_planes_shear<640, 480>(x->c, ts, grd, blk, st, pa, sm);
-        else if (planes(320, 240)) launch_planes_shear<320, 240>(x->c, ts, grd, blk, st, pa, sm);
-        else if (planes(640, 489)) launch_planes_shear<640, 489>(x->c, ts, grd, blk, st, pa, sm);      // the real Azure Kinect canvas: ceil(2 cy) = 489
-        else if (geom) launch_planes_shear<0, 0>(x->c, ts, grd, blk, st, pa, sm);                      // any other canvas, runtime geometry
+        if (planes(640, 480)) launch_planes_shear<640, 480>(x->c, ts, grd, blk, st, pa, sm, pm);
+        else if (planes(320, 240)) launch_planes_shear<320, 240>(x->c, ts, grd, blk, st, pa, sm, pm);
+        else if (planes(640, 489)) launch_planes_shear<640, 489>(x->c, ts, grd, blk, st, pa, sm, pm);      // the real Azure Kinect canvas: ceil(2 cy) = 489
+        else if (geom) launch_planes_shear<0, 0>(x->c, ts, grd, blk, st, pa, sm, pm);                      // any other canvas, runtime geometry
         else done = false;
         if (done) {
             VIDC_LAUNCH_CHECK();
@@ -593,10 +614,9 @@ int warp_rgbd_impl(const vidc_camera* cam, const vidc_image* rgb, const vidc_ima
         fa.rgb_o = rgb_out->data; fa.rgbo_sn = rgb_out->sn; fa.rgbo_sc = (int)rgb_out->sc; fa.rgbo_sh = (int)rgb_out->sh;
         fa.dep_o = depth ? depth_out->data : nullptr; fa.depo_sn = depth ? depth_out->sn : 0; fa.depo_sh = depth ? (int)depth_out->sh : 0;
         fa.mode_d = (int)depth_mode; fa.mask = d_mask_u8; fa.coverage = d_coverage;
-        fa.src_boxes = nullptr; fa.pf_x = fa.pf_y = fa.pf_z = 0;
+        fa.src_boxes = nullptr; fa.pf_x = fa.pf_y = fa.pf_z = 0; fa.pf_bulk = 0;
         if (tile_skip_enabled() && shear_level() >= 1 && fwd_prefetch_pct() > 0 && (size_t)grd.x * grd.y <= 320) {
-            static const int sms = [] { int dev = 0, n = 148; cudaGetDevice(&dev); cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev); return n; }();
-            const int wave = (int)((long long)sms * VIDC_SHEAR_BLOCKS_FWD * fwd_prefetch_pct() / 100);
+            const int wave = (int)((long long)sm_count() * VIDC_SHEAR_BLOCKS_FWD * fwd_prefetch_pct() / 100);
             fa.src_boxes = reinterpret_cast<const uint4*>(d_params_ws + rgb->n);
             fa.pf_x = wave % (int)grd.x; fa.pf_y = (wave / (int)grd.x) % (int)grd.y; fa.pf_z = wave / (int)(grd.x * grd.y);
         }
@@ -641,6 +661,11 @@ int warp_rgbd_impl(const vidc_camera* cam, const vidc_image* rgb, const vidc_ima
                 VIDC_CUDA(cudaMemsetAsync(zero_depth_out->data, 0, sizeof(float) * (size_t)rgb->n * cam->W * cam->H, st));
             }
         }
+        PrefetchMaps pm;                                           // input maps of the bulk prefetch; else the per-thread form
+        fa.pf_bulk = shear_geom && fa.src_boxes && pf_bulk_enabled() &&
+                     encode_store_map(&pm.img, rgb->data, cam->W, cam->H, 3, rgb->n, rgb->sh, rgb->sc, rgb->sn, false, PF_FWD_BW, PF_FWD_BH) &&
+                     (!depth || encode_store_map(&pm.dep, depth->data, cam->W, cam->H, 1, rgb->n, depth->sh, (int64_t)cam->W * cam->H, depth->sn,
+                                                 true, PF_FWD_BW, PF_FWD_BH));
         StoreMaps sm;
         bool ts = shear_geom && tma_store_enabled() &&
                   encode_store_map(&sm.img, rgb_out->data, cam->W, cam->H, 3, rgb->n, rgb_out->sh, rgb_out->sc, rgb_out->sn);
@@ -649,13 +674,13 @@ int warp_rgbd_impl(const vidc_camera* cam, const vidc_image* rgb, const vidc_ima
             ts = encode_store_map(&sm.dep, zero_depth_out->data, cam->W, cam->H, 1, rgb->n, zero_depth_out->sh, (int64_t)cam->W * cam->H, zero_depth_out->sn, true);
         if (ts && d_mask_u8) ts = encode_mask_map(&sm.mask, d_mask_u8, cam->W, cam->H, rgb->n);
         if (shear && planes(640, 480)) {
-            launch_rgbd_shear<640, 480>(depth != nullptr, ts, grd, blk, st, fa, sm);
+            launch_rgbd_shear<640, 480>(depth != nullptr, ts, grd, blk, st, fa, sm, pm);
         } else if (shear && planes(320, 240)) {
-            launch_rgbd_shear<320, 240>(depth != nullptr, ts, grd, blk, st, fa, sm);
+            launch_rgbd_shear<320, 240>(depth != nullptr, ts, grd, blk, st, fa, sm, pm);
         } else if (shear && planes(640, 489)) {                            // the real Azure Kinect canvas: ceil(2 cy) = 489
-            launch_rgbd_shear<640, 489>(depth != nullptr, ts, grd, blk, st, fa, sm);
+            launch_rgbd_shear<640, 489>(depth != nullptr, ts, grd, blk, st, fa, sm, pm);
         } else if (shear && cam->W % 32 == 0 && planes(cam->W, cam->H)) {  // any other canvas, runtime geometry
-            launch_rgbd_shear<0, 0>(depth != nullptr, ts, grd, blk, st, fa, sm);
+            launch_rgbd_shear<0, 0>(depth != nullptr, ts, grd, blk, st, fa, sm, pm);
         } else if (planes(640, 480)) {
             if (depth) warp_rgbd_fast_kernel<640, 480, true><<<grd, blk, 0, st>>>(fa);
             else warp_rgbd_fast_kernel<640, 480, false><<<grd, blk, 0, st>>>(fa);
@@ -734,6 +759,7 @@ int vidc_unwarp_normals(const vidc_camera* cam, const vidc_image* x, const float
     ia.x = x->data; ia.x_sn = x->sn; ia.x_sc = (int)x->sc; ia.x_sh = (int)x->sh;
     ia.z = z->data; ia.z_sn = z->sn; ia.z_sc = (int)z->sc; ia.z_sh = (int)z->sh;
     ia.valid = d_valid_u8;
+    ia.pf_on = ia.pf_x = ia.pf_y = ia.pf_z = 0;
     auto planes = [&](int Wg, int Hg) {
         return cam->W == Wg && cam->H == Hg && x->sh == Wg && x->sc == (int64_t)Wg * Hg && z->sh == Wg && z->sc == (int64_t)Wg * Hg;
     };
@@ -790,17 +816,24 @@ int vidc_unwarp_normals(const vidc_camera* cam, const vidc_image* x, const float
         }
         const bool shear = shear_level() >= 2 && aligned16(z->data) && z->sn % 4 == 0 &&
                            (!d_valid_u8 || (reinterpret_cast<uintptr_t>(d_valid_u8) & 3) == 0);
+        PrefetchMaps pm;
+        if (shear && cam->W % 32 == 0 && planes(cam->W, cam->H) && pf_bulk_enabled() && inv_prefetch_pct() > 0 &&
+            encode_store_map(&pm.img, x->data, cam->W, cam->H, 3, x->n, x->sh, x->sc, x->sn, false, PF_INV_BW, PF_INV_BH)) {
+            const int wave = (int)((long long)sm_count() * VIDC_SHEAR_BLOCKS_INV * inv_prefetch_pct() / 100);
+            ia.pf_on = 1;
+            ia.pf_x = wave % (int)grd.x; ia.pf_y = (wave / (int)grd.x) % (int)grd.y; ia.pf_z = wave / (int)(grd.x * grd.y);
+        }
         StoreMaps sm;
         const bool ts = shear && tma_store_enabled() && !d_valid_u8 && cam->W % 32 == 0 && planes(cam->W, cam->H) &&
                         encode_store_map(&sm.img, z->data, cam->W, cam->H, 3, x->n, z->sh, z->sc, z->sn);
         if (shear && planes(640, 480)) {
-            launch_unwarp_shear<640, 480>(normalize != 0, d_valid_u8 != nullptr, ts, grd, blk, st, ia, sm);
+            launch_unwarp_shear<640, 480>(normalize != 0, d_valid_u8 != nullptr, ts, grd, blk, st, ia, sm, pm);
         } else if (shear && planes(320, 240)) {
-            launch_unwarp_shear<320, 240>(normalize != 0, d_valid_u8 != nullptr, ts, grd, blk, st, ia, sm);
+            launch_unwarp_shear<320, 240>(normalize != 0, d_valid_u8 != nullptr, ts, grd, blk, st, ia, sm, pm);
         } else if (shear && planes(640, 489)) {
-            launch_unwarp_shear<640, 489>(normalize != 0, d_valid_u8 != nullptr, ts, grd, blk, st, ia, sm);
+            launch_unwarp_shear<640, 489>(normalize != 0, d_valid_u8 != nullptr, ts, grd, blk, st, ia, sm, pm);
         } else if (shear && cam->W % 32 == 0 && planes(cam->W, cam->H)) {  // any other canvas, runtime geometry
-            launch_unwarp_shear<0, 0>(normalize != 0, d_valid_u8 != nullptr, ts, grd, blk, st, ia, sm);
+            launch_unwarp_shear<0, 0>(normalize != 0, d_valid_u8 != nullptr, ts, grd, blk, st, ia, sm, pm);
         } else if (planes(640, 480)) {
             if (normalize) unwarp_normals_fast_kernel<640, 480, true><<<grd, blk, 0, st>>>(ia);
             else unwarp_normals_fast_kernel<640, 480, false><<<grd, blk, 0, st>>>(ia);
