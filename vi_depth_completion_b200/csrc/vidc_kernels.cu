@@ -22,6 +22,8 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
+#include <initializer_list>
+#include <type_traits>
 #include <algorithm>
 #include <mutex>
 #include <vector>
@@ -129,6 +131,8 @@ int launch_params(const vidc_camera* cam, const float* d_Ig, const float* d_Ia, 
     VIDC_LAUNCH_CHECK();
     return VIDC_OK;
 }
+
+// ---- environment switches (read once per process) ------------------------------------------------------------------------
 // Parameters + exterior-tile bitmap for the sheared forward kernels (one CTA per frame); VIDC_TILE_SKIP=0 turns it off.
 bool tile_skip_enabled() {
     static const bool v = [] { const char* e = getenv("VIDC_TILE_SKIP"); return !(e && e[0] == '0'); }();
@@ -152,12 +156,63 @@ int inv_prefetch_pct() {
     static const int v = [] { const char* e = getenv("VIDC_INV_PF_WAVES_X100"); return e ? atoi(e) : 16; }();
     return v;
 }
+// L2 prefetch distance of the staged-footprint inverse kernel, percent of a wave (VIDC_BOX_PF_WAVES_X100): half a wave ahead
+// measured best (0.527 ms; none 0.544, a full wave 0.63).
+int box_prefetch_pct() {
+    static const int v = [] { const char* e = getenv("VIDC_BOX_PF_WAVES_X100"); return e ? atoi(e) : 50; }();
+    return v;
+}
+// TMA write-out of the sheared kernels (kernels_shear.cuh, StoreMaps): on unless VIDC_TMA_STORE=0 (A/B runs and the parity
+// suite's handle on the LSU write-out); calls whose outputs cannot be described by a tensor map take the LSU write-out.
+bool tma_store_enabled() {
+    static const bool v = [] { const char* e = getenv("VIDC_TMA_STORE"); return !(e && e[0] == '0'); }();
+    return v;
+}
+// The TMA-staged forward kernel is correct (parity suite) but, in its first one-tile-per-CTA form, slower than
+// the L1-gather kernel on the B200 (0.89 vs 0.63 ms: exposed copy latency and 3-6x bounding-box over-fetch,
+// profiles/r1_history.md), so it is opt-in: VIDC_TMA=1.
+bool tma_enabled() {
+    static const bool v = [] { const char* e = getenv("VIDC_TMA"); return e && e[0] == '1'; }();
+    return v;
+}
+// Sheared row segments (kernels_shear.cuh).  VIDC_SHEAR = 2 (default): sheared forward and inverse warps; 1: sheared
+// forward warp only; 0: straight rows everywhere.  Measured on the B200 the sheared kernels are at least as fast as the
+// straight-row ones at every roll angle and 18-30 % faster beyond ~25 deg (profiles/r1_history.md); the switch exists
+// for A/B measurements and as the parity suite's handle on each kernel family.
+int shear_level() {
+    static const int v = [] { const char* e = getenv("VIDC_SHEAR"); return (e && e[0] >= '0' && e[0] <= '2') ? e[0] - '0' : 2; }();
+    return v;
+}
+// Inverse warp with the footprint staged in shared memory (kernels_box.cuh), for contiguous planes with W % 4 == 0.  Measured
+// on the B200 it does not beat the sheared kernel (0.527 vs 0.499 ms, profiles/r2_history.md: the staging pass costs what the
+// cheaper taps save), so it is opt-in: VIDC_INV_BOX=1 (A/B runs, and the parity suite's handle on it).
+bool inv_box_enabled() {
+    static const bool v = [] { const char* e = getenv("VIDC_INV_BOX"); return e && e[0] == '1'; }();
+    return v;
+}
 int sm_count() {
     static const int n = [] { int dev = 0, k = 148; cudaGetDevice(&dev); cudaDeviceGetAttribute(&k, cudaDevAttrMultiProcessorCount, dev); return k; }();
     return n;
 }
-int launch_params_tiles(const vidc_camera* cam, const float* d_Ig, const float* d_Ia, int B, vidc_frame_params* d_params,
-                        cudaStream_t st, float* d_H_out) {
+inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
+// ---- kernel selection ------------------------------------------------------------------------------------------------------
+// The frame parameters of a warp call.  With `prepared_ok` and d_Ig == d_Ia == NULL the workspace was prepared by
+// vidc_frame_params_prepare: no per-frame kernel, Cg_H_C by a scatter if asked for.  With `tiles` (the sheared forward warps
+// read the tables) and VIDC_TILE_SKIP on, the tiles kernel adds the exterior-tile bitmap and the per-tile source boxes of the
+// L2 prefetch; otherwise the plain kernel runs.
+bool tiles_kernel_enabled() { return tile_skip_enabled() && shear_level() >= 1; }
+int warp_params(const vidc_camera* cam, const float* d_Ig, const float* d_Ia, int B, vidc_frame_params* d_params, float* d_H_out,
+                cudaStream_t st, bool prepared_ok, bool tiles) {
+    if (prepared_ok && !d_Ig && !d_Ia) {
+        if (!d_params) return fail(VIDC_ERR_INVALID_ARGUMENT, "null params pointer");
+        if (d_H_out) {
+            scatter_homography_kernel<<<(B * 9 + 127) / 128, 128, 0, st>>>(d_params, B, d_H_out, nullptr, nullptr, nullptr);
+            VIDC_LAUNCH_CHECK();
+        }
+        return VIDC_OK;
+    }
+    if (!tiles || !tiles_kernel_enabled()) return launch_params(cam, d_Ig, d_Ia, B, d_params, st, d_H_out);
     if (B == 0) return VIDC_OK;
     if (!d_Ig || !d_Ia || !d_params) return fail(VIDC_ERR_INVALID_ARGUMENT, "null gravity / alignment / params pointer");
     static_assert(sizeof(vidc_frame_params) == 48 * sizeof(float), "frame params layout");
@@ -168,14 +223,51 @@ int launch_params_tiles(const vidc_camera* cam, const float* d_Ig, const float* 
     return VIDC_OK;
 }
 
-// d_Ig == d_Ia == NULL: the workspace was prepared by vidc_frame_params_prepare (no per-frame kernel; Cg_H_C by a scatter if asked for)
-int prepared_params(const vidc_frame_params* d_params_ws, int B, float* d_H_out, cudaStream_t st) {
-    if (!d_params_ws) return fail(VIDC_ERR_INVALID_ARGUMENT, "null params pointer");
-    if (d_H_out) {
-        scatter_homography_kernel<<<(B * 9 + 127) / 128, 128, 0, st>>>(d_params_ws, B, d_H_out, nullptr, nullptr, nullptr);
-        VIDC_LAUNCH_CHECK();
-    }
-    return VIDC_OK;
+// L2 prefetch distance: `pct` percent of a wave of resident CTAs (SMs x CTAs per SM), as an offset in grid coordinates
+int3 prefetch_offset(int pct, int ctas_per_sm, dim3 grd) {
+    const int wave = (int)((long long)sm_count() * ctas_per_sm * pct / 100);
+    return make_int3(wave % (int)grd.x, (wave / (int)grd.x) % (int)grd.y, wave / (int)(grd.x * grd.y));
+}
+// L2 prefetch of the sheared forward kernels (FwdArgs, PlanesArgs): the source boxes the tiles kernel wrote behind the B
+// parameter blocks, when it wrote them; the bulk form (pf_bulk) is the caller's to turn on.
+template <typename Args>
+void set_fwd_prefetch(Args& a, const vidc_frame_params* prm, int B, dim3 grd) {
+    a.src_boxes = nullptr; a.pf_x = a.pf_y = a.pf_z = 0; a.pf_bulk = 0;
+    if (!(tiles_kernel_enabled() && fwd_prefetch_pct() > 0 && (size_t)grd.x * grd.y <= 320)) return;
+    const int3 pf = prefetch_offset(fwd_prefetch_pct(), VIDC_SHEAR_BLOCKS_FWD, grd);
+    a.src_boxes = reinterpret_cast<const uint4*>(prm + B);
+    a.pf_x = pf.x; a.pf_y = pf.y; a.pf_z = pf.z;
+}
+
+// Every image given is a run of contiguous W x H planes (rows of W floats, planes of W H floats), the layout of the
+// compile-time geometries and of the sheared kernels' tensor maps.  NULL entries (absent optional images) are skipped.
+bool contiguous_planes(const vidc_camera* cam, std::initializer_list<const vidc_image*> ims) {
+    for (const vidc_image* im : ims)
+        if (im && !(im->w == cam->W && im->h == cam->H && im->sh == cam->W && (im->c == 1 || im->sc == (int64_t)cam->W * cam->H)))
+            return false;
+    return true;
+}
+
+// f(std::integral_constant<bool, flag>...): each runtime flag becomes a template argument of the launch f writes once.
+template <typename F>
+void with_flags(F&& f) { f(); }
+template <typename F, typename... Flags>
+void with_flags(F&& f, bool flag, Flags... rest) {
+    if (flag) with_flags([&](auto... t) { f(std::true_type{}, t...); }, rest...);
+    else with_flags([&](auto... t) { f(std::false_type{}, t...); }, rest...);
+}
+// f(GW, GH, flags...) with the canvas as compile-time geometry: 640x480, 320x240 and, in the families compiled for it
+// (WITH_489), the real Azure Kinect canvas 640x489 (ceil(2 cy) = 489).  Any other canvas, or images that are not contiguous
+// planes of it (`compiled` false), run the runtime geometry <0, 0>.
+template <int V> using int_ = std::integral_constant<int, V>;
+template <bool WITH_489, typename F, typename... Flags>
+void with_geometry(const vidc_camera* cam, bool compiled, F&& f, Flags... flags) {
+    auto go = [&](auto gw, auto gh) { with_flags([&](auto... t) { f(gw, gh, t...); }, flags...); };
+    if (compiled && cam->W == 640 && cam->H == 480) return go(int_<640>{}, int_<480>{});
+    if (compiled && cam->W == 320 && cam->H == 240) return go(int_<320>{}, int_<240>{});
+    if constexpr (WITH_489)
+        if (compiled && cam->W == 640 && cam->H == 489) return go(int_<640>{}, int_<489>{});
+    go(int_<0>{}, int_<0>{});
 }
 
 template <int C_A, bool HAS_D, bool ROT>
@@ -189,6 +281,16 @@ int launch_forward(const vidc_camera* cam, const vidc_frame_params* prm, const v
     VIDC_LAUNCH_CHECK();
     return VIDC_OK;
 }
+// 1..4 planes of any layout through the generic forward kernel
+int launch_forward_planes(const vidc_camera* cam, const vidc_frame_params* prm, const vidc_image* x, const vidc_image* y, int mode,
+                          cudaStream_t st) {
+    switch (x->c) {
+        case 1: return launch_forward<1, false, false>(cam, prm, x, y, mode, nullptr, nullptr, 0, nullptr, nullptr, st);
+        case 2: return launch_forward<2, false, false>(cam, prm, x, y, mode, nullptr, nullptr, 0, nullptr, nullptr, st);
+        case 3: return launch_forward<3, false, false>(cam, prm, x, y, mode, nullptr, nullptr, 0, nullptr, nullptr, st);
+        default: return launch_forward<4, false, false>(cam, prm, x, y, mode, nullptr, nullptr, 0, nullptr, nullptr, st);
+    }
+}
 
 int check_out(const vidc_camera* cam, const vidc_image* x, const vidc_image* y, const char* name) {
     if (y->n != x->n || y->c != x->c || y->h != cam->H || y->w != cam->W)
@@ -201,6 +303,14 @@ int scatter_h(const vidc_frame_params* prm, int B, float* H, float* R, float* Hi
     if (B == 0 || (!H && !R && !Hi && !Rt)) return VIDC_OK;
     scatter_homography_kernel<<<(B * 9 + 127) / 128, 128, 0, st>>>(prm, B, H, R, Hi, Rt);
     VIDC_LAUNCH_CHECK();
+    return VIDC_OK;
+}
+
+// The (B,1,H,W) zero plane of the sparse-depth route where no RGB kernel writes it: a memset of a contiguous output
+int zero_depth_plane(const vidc_camera* cam, const vidc_image* z, int B, cudaStream_t st) {
+    if (z->sw != 1 || z->sh != cam->W || z->sn != (int64_t)cam->W * cam->H)
+        return fail(VIDC_ERR_INVALID_ARGUMENT, "depth_out: the sparse-depth path needs a contiguous (B,1,H,W) output");
+    VIDC_CUDA(cudaMemsetAsync(z->data, 0, sizeof(float) * (size_t)B * cam->W * cam->H, st));
     return VIDC_OK;
 }
 
@@ -218,95 +328,63 @@ PFN_encodeTiled tma_encoder() {
     }();
     return fn;
 }
+// A tiled map of `rank` dimensions (innermost first; rank - 1 byte strides), unit element strides, no interleave or swizzle,
+// no fill value (out of range reads zero).  false if the driver has no encoder or refuses the view.
+bool encode_tiled(CUtensorMap* map, CUtensorMapDataType type, cuuint32_t rank, void* data, const cuuint64_t* dims,
+                  const cuuint64_t* strides, const cuuint32_t* box, CUtensorMapL2promotion l2 = CU_TENSOR_MAP_L2_PROMOTION_NONE) {
+    static const cuuint32_t estr[4] = {1, 1, 1, 1};
+    PFN_encodeTiled enc = tma_encoder();
+    return enc && enc(map, type, rank, data, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, l2,
+                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
 // (W, H, C, N) fp32 view with a (64, box_h, C, 1) box; zero fill out of range.  false if the view cannot be described.
 bool encode_image_map(CUtensorMap* map, const vidc_image* im, int box_h, int box_w = TMA_BW) {
-    PFN_encodeTiled enc = tma_encoder();
-    if (!enc || im->sw != 1) return false;
+    if (im->sw != 1) return false;
     if (((uintptr_t)im->data & 15) || (im->sh & 3) || (im->sc & 3) || (im->sn & 3) || im->sh <= 0 || im->sc <= 0) return false;
     if (im->w < 1 || im->h < 1) return false;
     const cuuint64_t dims[4] = {(cuuint64_t)im->w, (cuuint64_t)im->h, (cuuint64_t)im->c, (cuuint64_t)im->n};
     const cuuint64_t strides[3] = {(cuuint64_t)im->sh * 4, (cuuint64_t)im->sc * 4, (cuuint64_t)(im->sn > 0 ? im->sn : im->sc * im->c) * 4};
     const cuuint32_t box[4] = {(cuuint32_t)box_w, (cuuint32_t)box_h, (cuuint32_t)im->c, 1};
-    const cuuint32_t estr[4] = {1, 1, 1, 1};
-    return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, im->data, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+    return encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, im->data, dims, strides, box, CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
 }
 // Output tensor maps of the TMA write-out (kernels_shear.cuh: StoreMaps): (W, H, C, N) fp32 planes, box (32, 32, C, 1), or
 // (W, H, N) for a single plane; the input maps of the bulk L2 prefetch (PrefetchMaps) are the same views with a (bw, bh) box.
 // false if the view cannot be described (strides not multiples of 16 bytes, ...).
 bool encode_store_map(CUtensorMap* map, float* data, int W, int H, int C, int N, int64_t sh, int64_t sc, int64_t sn, bool plane3d = false,
                       int bw = 32, int bh = 32) {
-    PFN_encodeTiled enc = tma_encoder();
-    if (!enc || ((uintptr_t)data & 15) || (sh & 3) || (sc & 3) || (sn & 3) || sh <= 0 || sn <= 0) return false;
-    const cuuint32_t estr[4] = {1, 1, 1, 1};
+    if (((uintptr_t)data & 15) || (sh & 3) || (sc & 3) || (sn & 3) || sh <= 0 || sn <= 0) return false;
     if (plane3d) {                                   // StoreMaps::dep: one plane per frame, stored with the 3-D instruction
         const cuuint64_t dims[3] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
         const cuuint64_t strides[2] = {(cuuint64_t)sh * 4, (cuuint64_t)sn * 4};
         const cuuint32_t box[3] = {(cuuint32_t)bw, (cuuint32_t)bh, 1};
-        return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, data, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+        return encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, data, dims, strides, box);
     }
     if (sc <= 0) return false;
     const cuuint64_t dims[4] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)C, (cuuint64_t)N};
     const cuuint64_t strides[3] = {(cuuint64_t)sh * 4, (cuuint64_t)sc * 4, (cuuint64_t)sn * 4};
     const cuuint32_t box[4] = {(cuuint32_t)bw, (cuuint32_t)bh, (cuuint32_t)C, 1};
-    return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, data, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+    return encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, data, dims, strides, box);
 }
 // channels-last three-channel image (kernels_shear_cl.cuh): the output seen as (3 W, H, N) fp32, box (96, 32, 1)
 bool is_channels_last3(const vidc_image* im, int W, int H) {
     return im->c == 3 && im->w == W && im->h == H && im->sc == 1 && im->sw == 3 && im->sh == 3 * (int64_t)W && im->sn == 3 * (int64_t)W * H;
 }
 bool encode_cl_map(CUtensorMap* map, float* data, int W, int H, int N) {
-    PFN_encodeTiled enc = tma_encoder();
-    if (!enc || ((uintptr_t)data & 15) || (W & 3)) return false;
+    if (((uintptr_t)data & 15) || (W & 3)) return false;
     const cuuint64_t dims[3] = {(cuuint64_t)3 * W, (cuuint64_t)H, (cuuint64_t)N};
     const cuuint64_t strides[2] = {(cuuint64_t)3 * W * 4, (cuuint64_t)3 * W * H * 4};
-    const cuuint32_t box[3] = {96, 32, 1}, estr[3] = {1, 1, 1};
-    return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, data, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+    const cuuint32_t box[3] = {96, 32, 1};
+    return encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, data, dims, strides, box);
 }
 bool encode_mask_map(CUtensorMap* map, uint8_t* data, int W, int H, int N) {            // (W, H, N) uint8, contiguous, box (32, 32, 1)
-    PFN_encodeTiled enc = tma_encoder();
-    if (!enc || ((uintptr_t)data & 15) || (W & 15)) return false;
+    if (((uintptr_t)data & 15) || (W & 15)) return false;
     const cuuint64_t dims[3] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
     const cuuint64_t strides[2] = {(cuuint64_t)W, (cuuint64_t)W * H};
-    const cuuint32_t box[3] = {32, 32, 1}, estr[3] = {1, 1, 1};
+    const cuuint32_t box[3] = {32, 32, 1};
     if (strides[1] & 15) return false;
-    return enc(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, data, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-// TMA write-out of the sheared kernels (kernels_shear.cuh, StoreMaps): on unless VIDC_TMA_STORE=0 (A/B runs and the parity
-// suite's handle on the LSU write-out); calls whose outputs cannot be described by a tensor map take the LSU write-out.
-bool tma_store_enabled() {
-    static const bool v = [] { const char* e = getenv("VIDC_TMA_STORE"); return !(e && e[0] == '0'); }();
-    return v;
-}
-// The TMA-staged forward kernel is correct (parity suite) but, in its first one-tile-per-CTA form, slower than
-// the L1-gather kernel on the B200 (0.89 vs 0.63 ms: exposed copy latency and 3-6x bounding-box over-fetch,
-// profiles/r1_history.md), so it is opt-in: VIDC_TMA=1.
-bool tma_enabled() {
-    static const bool v = [] { const char* e = getenv("VIDC_TMA"); return e && e[0] == '1'; }();
-    return v;
+    return encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, data, dims, strides, box);
 }
 
-// Sheared row segments (kernels_shear.cuh).  VIDC_SHEAR = 2 (default): sheared forward and inverse warps; 1: sheared
-// forward warp only; 0: straight rows everywhere.  Measured on the B200 the sheared kernels are at least as fast as the
-// straight-row ones at every roll angle and 18-30 % faster beyond ~25 deg (profiles/r1_history.md); the switch exists
-// for A/B measurements and as the parity suite's handle on each kernel family.
-int shear_level() {
-    static const int v = [] { const char* e = getenv("VIDC_SHEAR"); return (e && e[0] >= '0' && e[0] <= '2') ? e[0] - '0' : 2; }();
-    return v;
-}
-inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
-
-// Inverse warp with the footprint staged in shared memory (kernels_box.cuh), for contiguous planes with W % 4 == 0.  Measured
-// on the B200 it does not beat the sheared kernel (0.527 vs 0.499 ms, profiles/r2_history.md: the staging pass costs what the
-// cheaper taps save), so it is opt-in: VIDC_INV_BOX=1 (A/B runs, and the parity suite's handle on it).
-bool inv_box_enabled() {
-    static const bool v = [] { const char* e = getenv("VIDC_INV_BOX"); return e && e[0] == '1'; }();
-    return v;
-}
 template <typename K>
 void prefer_shared_carveout(K kernel) {          // per device: function attributes belong to the device's context
     static std::atomic<unsigned long long> done[2] = {{0ull}, {0ull}};
@@ -317,77 +395,7 @@ void prefer_shared_carveout(K kernel) {          // per device: function attribu
     cudaFuncSetAttribute(kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
     done[dev >> 6].fetch_or(bit, std::memory_order_relaxed);
 }
-template <int GW, int GH>
-void launch_unwarp_box(bool normalize, bool has_valid, dim3 grd, dim3 blk, cudaStream_t st, const InvArgs& ia, const uint4* boxes) {
-    const dim3 grd2(grd.x, (grd.y + 1) / 2, grd.z);               // one CTA = two vertically adjacent tiles
-    // prefetch distance: about one wave of resident CTAs (SMs x CTAs per SM), as an offset in grid coordinates
-    static const int wave = [] {
-        int dev = 0, sms = 148;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        const char* e = getenv("VIDC_BOX_PF_WAVES_X100");
-        const int pct = e ? atoi(e) : 50;             // half a wave ahead measured best (0.527 ms; none 0.544, a full wave 0.63)
-        return (int)((long long)sms * VIDC_BOX_BLOCKS * pct / 100);
-    }();
-    int3 pf;
-    pf.x = wave % (int)grd2.x; pf.y = (wave / (int)grd2.x) % (int)grd2.y; pf.z = wave / (int)(grd2.x * grd2.y);
-#define VIDC_BOX_LAUNCH(N, V)                                                          \
-    do {                                                                               \
-        prefer_shared_carveout(unwarp_normals_box_kernel<GW, GH, N, V>);               \
-        unwarp_normals_box_kernel<GW, GH, N, V><<<grd2, blk, 0, st>>>(ia, boxes, (int)grd.y, pf); \
-    } while (0)
-    if (normalize) { if (has_valid) VIDC_BOX_LAUNCH(true, true); else VIDC_BOX_LAUNCH(true, false); }
-    else { if (has_valid) VIDC_BOX_LAUNCH(false, true); else VIDC_BOX_LAUNCH(false, false); }
-#undef VIDC_BOX_LAUNCH
-}
 
-template <int GW, int GH>
-void launch_unwarp_shear(bool normalize, bool has_valid, bool ts, dim3 grd, dim3 blk, cudaStream_t st, const InvArgs& ia, const StoreMaps& sm,
-                         const PrefetchMaps& pm) {
-    if (ts && !has_valid) {
-        if (normalize) unwarp_normals_shear_kernel<GW, GH, true, false, true><<<grd, blk, 0, st>>>(ia, sm, pm);
-        else unwarp_normals_shear_kernel<GW, GH, false, false, true><<<grd, blk, 0, st>>>(ia, sm, pm);
-    } else if (normalize) {
-        if (has_valid) unwarp_normals_shear_kernel<GW, GH, true, true, false><<<grd, blk, 0, st>>>(ia, sm, pm);
-        else unwarp_normals_shear_kernel<GW, GH, true, false, false><<<grd, blk, 0, st>>>(ia, sm, pm);
-    } else {
-        if (has_valid) unwarp_normals_shear_kernel<GW, GH, false, true, false><<<grd, blk, 0, st>>>(ia, sm, pm);
-        else unwarp_normals_shear_kernel<GW, GH, false, false, false><<<grd, blk, 0, st>>>(ia, sm, pm);
-    }
-}
-template <int GW, int GH>
-void launch_rgbd_shear(bool has_d, bool ts, dim3 grd, dim3 blk, cudaStream_t st, const FwdArgs& fa, const StoreMaps& sm, const PrefetchMaps& pm) {
-    if (ts) {
-        if (has_d) warp_rgbd_shear_kernel<GW, GH, true, true><<<grd, blk, 0, st>>>(fa, sm, pm);
-        else warp_rgbd_shear_kernel<GW, GH, false, true><<<grd, blk, 0, st>>>(fa, sm, pm);
-    } else {
-        if (has_d) warp_rgbd_shear_kernel<GW, GH, true, false><<<grd, blk, 0, st>>>(fa, sm, pm);
-        else warp_rgbd_shear_kernel<GW, GH, false, false><<<grd, blk, 0, st>>>(fa, sm, pm);
-    }
-}
-template <int GW, int GH>
-void launch_planes_shear(int C, bool ts, dim3 grd, dim3 blk, cudaStream_t st, const PlanesArgs& pa, const StoreMaps& sm, const PrefetchMaps& pm) {
-    if (ts) {
-        if (C == 3) warp_planes_shear_kernel<GW, GH, 3, true><<<grd, blk, 0, st>>>(pa, sm, pm);
-        else warp_planes_shear_kernel<GW, GH, 1, true><<<grd, blk, 0, st>>>(pa, sm, pm);
-    } else {
-        if (C == 3) warp_planes_shear_kernel<GW, GH, 3, false><<<grd, blk, 0, st>>>(pa, sm, pm);
-        else warp_planes_shear_kernel<GW, GH, 1, false><<<grd, blk, 0, st>>>(pa, sm, pm);
-    }
-}
-
-template <bool HAS_D>
-void launch_rgbd_cl(const vidc_camera* cam, dim3 grd, dim3 blk, cudaStream_t st, const FwdArgs& fa, const ClStoreMaps& sm) {
-    if (cam->W == 640 && cam->H == 480) warp_rgbd_shear_cl_kernel<640, 480, HAS_D><<<grd, blk, 0, st>>>(fa, sm);
-    else if (cam->W == 320 && cam->H == 240) warp_rgbd_shear_cl_kernel<320, 240, HAS_D><<<grd, blk, 0, st>>>(fa, sm);
-    else warp_rgbd_shear_cl_kernel<0, 0, HAS_D><<<grd, blk, 0, st>>>(fa, sm);
-}
-template <bool NORMALIZE>
-void launch_unwarp_cl(const vidc_camera* cam, dim3 grd, dim3 blk, cudaStream_t st, const InvArgs& ia, const ClStoreMaps& sm) {
-    if (cam->W == 640 && cam->H == 480) unwarp_normals_shear_cl_kernel<640, 480, NORMALIZE><<<grd, blk, 0, st>>>(ia, sm);
-    else if (cam->W == 320 && cam->H == 240) unwarp_normals_shear_cl_kernel<320, 240, NORMALIZE><<<grd, blk, 0, st>>>(ia, sm);
-    else unwarp_normals_shear_cl_kernel<0, 0, NORMALIZE><<<grd, blk, 0, st>>>(ia, sm);
-}
 // channels-last RGB (+ planar depth, mask, coverage) through warp_rgbd_shear_cl_kernel; false: not applicable, take another path
 bool try_rgbd_cl(const vidc_camera* cam, const vidc_frame_params* prm, const vidc_image* rgb, const vidc_image* depth, int depth_mode,
                  const vidc_image* rgb_out, const vidc_image* depth_out, uint8_t* d_mask_u8, uint32_t* d_coverage, cudaStream_t st) {
@@ -404,8 +412,9 @@ bool try_rgbd_cl(const vidc_camera* cam, const vidc_frame_params* prm, const vid
     fa.rgb = rgb->data; fa.rgb_sn = rgb->sn; fa.dep = depth ? depth->data : nullptr; fa.dep_sn = depth ? depth->sn : 0;
     fa.Hin = cam->H; fa.Win = cam->W; fa.mode_d = depth_mode; fa.mask = d_mask_u8; fa.coverage = d_coverage;
     const dim3 blk(32, 8), grd((cam->W + TILE_W - 1) / TILE_W, (cam->H + TILE_H - 1) / TILE_H, rgb->n);
-    if (depth) launch_rgbd_cl<true>(cam, grd, blk, st, fa, sm);
-    else launch_rgbd_cl<false>(cam, grd, blk, st, fa, sm);
+    with_geometry<false>(cam, true, [&](auto gw, auto gh, auto has_d) {
+        warp_rgbd_shear_cl_kernel<gw, gh, has_d><<<grd, blk, 0, st>>>(fa, sm);
+    }, depth != nullptr);
     return true;                                                   // the caller checks the launch
 }
 
@@ -460,8 +469,7 @@ int vidc_frame_params_prepare(const vidc_camera* cam, const float* d_Ig, const f
                               vidc_frame_params* d_params_ws, float* d_H_out, void* stream) {
     VIDC_TRY(check_cam(cam));
     if (B < 0) return fail(VIDC_ERR_INVALID_ARGUMENT, "negative batch");
-    if (tile_skip_enabled() && shear_level() >= 1) return launch_params_tiles(cam, d_Ig, d_Ia, B, d_params_ws, (cudaStream_t)stream, d_H_out);
-    return launch_params(cam, d_Ig, d_Ia, B, d_params_ws, (cudaStream_t)stream, d_H_out);
+    return warp_params(cam, d_Ig, d_Ia, B, d_params_ws, d_H_out, (cudaStream_t)stream, /*prepared_ok=*/false, /*tiles=*/true);
 }
 
 int vidc_build_homography(const vidc_camera* cam, const float* d_Ig, const float* d_Ia, int32_t B,
@@ -489,8 +497,7 @@ int vidc_warp_forward(const vidc_camera* cam, const vidc_image* x, const float* 
     VIDC_TRY(check_out(cam, x, y, "y"));
     if (x->n == 0) return VIDC_OK;
     cudaStream_t st = (cudaStream_t)stream;
-    if (tile_skip_enabled() && shear_level() >= 1) VIDC_TRY(launch_params_tiles(cam, d_Ig, d_Ia, x->n, d_params_ws, st, d_H_out));
-    else VIDC_TRY(launch_params(cam, d_Ig, d_Ia, x->n, d_params_ws, st, d_H_out));
+    VIDC_TRY(warp_params(cam, d_Ig, d_Ia, x->n, d_params_ws, d_H_out, st, /*prepared_ok=*/false, /*tiles=*/true));
     // F.grid_sample takes any channel count (feature maps): more than four channels go through the kernels in groups of <= 4
     // planes that share the frame parameters computed above
     if (x->c > 4) {
@@ -512,47 +519,27 @@ __attribute__((visibility("hidden"))) int forward_group(const vidc_camera* cam, 
         VIDC_LAUNCH_CHECK();                                       // channels-last RGB (kernels_shear_cl.cuh)
         return VIDC_OK;
     }
-    // contiguous planes of a compile-time geometry: sheared segments (kernels_shear.cuh)
-    if (shear_level() >= 1 && mode != VIDC_BICUBIC && (x->c == 1 || x->c == 3) && x->sw == 1 && y->sw == 1 && aligned16(y->data) && y->sn % 4 == 0) {
-        auto planes = [&](int Wg, int Hg) {
-            const int64_t hw = (int64_t)Wg * Hg;
-            return cam->W == Wg && cam->H == Hg && x->w == Wg && x->h == Hg && x->sh == Wg && y->sh == Wg &&
-                   (x->c == 1 || (x->sc == hw && y->sc == hw));
-        };
+    // contiguous planes of the canvas: sheared segments (kernels_shear.cuh)
+    if (shear_level() >= 1 && mode != VIDC_BICUBIC && (x->c == 1 || x->c == 3) && x->sw == 1 && y->sw == 1 && aligned16(y->data) &&
+        y->sn % 4 == 0 && cam->W % 32 == 0 && contiguous_planes(cam, {x, y})) {
         const dim3 blk(32, 8), grd((cam->W + TILE_W - 1) / TILE_W, (cam->H + TILE_H - 1) / TILE_H, x->n);
         PlanesArgs pa;
         pa.prm = d_params_ws; pa.cam = cam_const(cam);
         pa.x = x->data; pa.x_sn = x->sn; pa.y = y->data; pa.y_sn = y->sn; pa.mode = (int)mode;
-        pa.src_boxes = nullptr; pa.pf_x = pa.pf_y = pa.pf_z = 0; pa.pf_bulk = 0;
-        bool done = true;
-        const bool geom = planes(640, 480) || planes(320, 240) || planes(640, 489) || (cam->W % 32 == 0 && planes(cam->W, cam->H));
+        set_fwd_prefetch(pa, d_params_ws, x->n, grd);
         PrefetchMaps pm;
-        if (tile_skip_enabled() && fwd_prefetch_pct() > 0 && (size_t)grd.x * grd.y <= 320) {     // the tiles kernel wrote the boxes
-            const int wave = (int)((long long)sm_count() * VIDC_SHEAR_BLOCKS_FWD * fwd_prefetch_pct() / 100);
-            pa.src_boxes = reinterpret_cast<const uint4*>(d_params_ws + x->n);
-            pa.pf_x = wave % (int)grd.x; pa.pf_y = (wave / (int)grd.x) % (int)grd.y; pa.pf_z = wave / (int)(grd.x * grd.y);
-            pa.pf_bulk = geom && x->c == 3 && pf_bulk_enabled() &&
-                         encode_store_map(&pm.img, x->data, cam->W, cam->H, 3, x->n, x->sh, x->sc, x->sn, false, PF_FWD_BW, PF_FWD_BH);
-        }
+        pa.pf_bulk = pa.src_boxes && x->c == 3 && pf_bulk_enabled() &&
+                     encode_store_map(&pm.img, x->data, cam->W, cam->H, 3, x->n, x->sh, x->sc, x->sn, false, PF_FWD_BW, PF_FWD_BH);
         StoreMaps sm;
-        const bool ts = geom && tma_store_enabled() &&
+        const bool ts = tma_store_enabled() &&
                         encode_store_map(&sm.img, y->data, cam->W, cam->H, x->c, x->n, y->sh, x->c == 1 ? (int64_t)cam->W * cam->H : y->sc, y->sn);
-        if (planes(640, 480)) launch_planes_shear<640, 480>(x->c, ts, grd, blk, st, pa, sm, pm);
-        else if (planes(320, 240)) launch_planes_shear<320, 240>(x->c, ts, grd, blk, st, pa, sm, pm);
-        else if (planes(640, 489)) launch_planes_shear<640, 489>(x->c, ts, grd, blk, st, pa, sm, pm);      // the real Azure Kinect canvas: ceil(2 cy) = 489
-        else if (geom) launch_planes_shear<0, 0>(x->c, ts, grd, blk, st, pa, sm, pm);                      // any other canvas, runtime geometry
-        else done = false;
-        if (done) {
-            VIDC_LAUNCH_CHECK();
-            return VIDC_OK;
-        }
+        with_geometry<true>(cam, true, [&](auto gw, auto gh, auto three, auto ts_) {
+            warp_planes_shear_kernel<gw, gh, three ? 3 : 1, ts_><<<grd, blk, 0, st>>>(pa, sm, pm);
+        }, x->c == 3, ts);
+        VIDC_LAUNCH_CHECK();
+        return VIDC_OK;
     }
-    switch (x->c) {
-        case 1: return launch_forward<1, false, false>(cam, d_params_ws, x, y, mode, nullptr, nullptr, 0, nullptr, nullptr, st);
-        case 2: return launch_forward<2, false, false>(cam, d_params_ws, x, y, mode, nullptr, nullptr, 0, nullptr, nullptr, st);
-        case 3: return launch_forward<3, false, false>(cam, d_params_ws, x, y, mode, nullptr, nullptr, 0, nullptr, nullptr, st);
-        default: return launch_forward<4, false, false>(cam, d_params_ws, x, y, mode, nullptr, nullptr, 0, nullptr, nullptr, st);
-    }
+    return launch_forward_planes(cam, d_params_ws, x, y, mode, st);
 }
 
 // zero_depth_out (sparse-depth path, depth == NULL): a (B,1,H,W) plane the call fills with zeros -- by the RGB kernel's own
@@ -594,9 +581,7 @@ int warp_rgbd_impl(const vidc_camera* cam, const vidc_image* rgb, const vidc_ima
     if (rgb->n == 0) return VIDC_OK;
     cudaStream_t st = (cudaStream_t)stream;
     if (d_coverage) VIDC_CUDA(cudaMemsetAsync(d_coverage, 0, sizeof(uint32_t) * (size_t)rgb->n, st));
-    if (!d_Ig && !d_Ia) VIDC_TRY(prepared_params(d_params_ws, rgb->n, d_H_out, st));
-    else if (tile_skip_enabled() && shear_level() >= 1) VIDC_TRY(launch_params_tiles(cam, d_Ig, d_Ia, rgb->n, d_params_ws, st, d_H_out));
-    else VIDC_TRY(launch_params(cam, d_Ig, d_Ia, rgb->n, d_params_ws, st, d_H_out));
+    VIDC_TRY(warp_params(cam, d_Ig, d_Ia, rgb->n, d_params_ws, d_H_out, st, /*prepared_ok=*/true, /*tiles=*/true));
     if (!zero_depth_out && try_rgbd_cl(cam, d_params_ws, rgb, depth, (int)depth_mode, rgb_out, depth_out, d_mask_u8, d_coverage, st)) {
         VIDC_LAUNCH_CHECK();                                       // channels-last RGB (kernels_shear_cl.cuh)
         return VIDC_OK;
@@ -604,106 +589,77 @@ int warp_rgbd_impl(const vidc_camera* cam, const vidc_image* rgb, const vidc_ima
     const bool fast = rgb->sw == 1 && rgb_out->sw == 1 &&
                       (!depth || (depth->sw == 1 && depth_out->sw == 1 && depth->h == rgb->h && depth->w == rgb->w &&
                                   depth->sh == rgb->sh));
-    if (fast) {
-        const dim3 blk(32, 8), grd((cam->W + TILE_W - 1) / TILE_W, (cam->H + TILE_H - 1) / TILE_H, rgb->n);
-        FwdArgs fa;
-        fa.prm = d_params_ws; fa.cam = cam_const(cam);
-        fa.rgb = rgb->data; fa.rgb_sn = rgb->sn; fa.rgb_sc = (int)rgb->sc;
-        fa.dep = depth ? depth->data : nullptr; fa.dep_sn = depth ? depth->sn : 0;
-        fa.Hin = rgb->h; fa.Win = rgb->w; fa.in_sh = (int)rgb->sh;
-        fa.rgb_o = rgb_out->data; fa.rgbo_sn = rgb_out->sn; fa.rgbo_sc = (int)rgb_out->sc; fa.rgbo_sh = (int)rgb_out->sh;
-        fa.dep_o = depth ? depth_out->data : nullptr; fa.depo_sn = depth ? depth_out->sn : 0; fa.depo_sh = depth ? (int)depth_out->sh : 0;
-        fa.mode_d = (int)depth_mode; fa.mask = d_mask_u8; fa.coverage = d_coverage;
-        fa.src_boxes = nullptr; fa.pf_x = fa.pf_y = fa.pf_z = 0; fa.pf_bulk = 0;
-        if (tile_skip_enabled() && shear_level() >= 1 && fwd_prefetch_pct() > 0 && (size_t)grd.x * grd.y <= 320) {
-            const int wave = (int)((long long)sm_count() * VIDC_SHEAR_BLOCKS_FWD * fwd_prefetch_pct() / 100);
-            fa.src_boxes = reinterpret_cast<const uint4*>(d_params_ws + rgb->n);
-            fa.pf_x = wave % (int)grd.x; fa.pf_y = (wave / (int)grd.x) % (int)grd.y; fa.pf_z = wave / (int)(grd.x * grd.y);
+    if (!fast) {
+        if (zero_depth_out) VIDC_TRY(zero_depth_plane(cam, zero_depth_out, rgb->n, st));
+        if (depth)
+            return launch_forward<3, true, false>(cam, d_params_ws, rgb, rgb_out, VIDC_BILINEAR, depth, depth_out, depth_mode,
+                                                  d_mask_u8, d_coverage, st);
+        return launch_forward<3, false, false>(cam, d_params_ws, rgb, rgb_out, VIDC_BILINEAR, nullptr, nullptr, 0, d_mask_u8,
+                                               d_coverage, st);
+    }
+    const dim3 blk(32, 8), grd((cam->W + TILE_W - 1) / TILE_W, (cam->H + TILE_H - 1) / TILE_H, rgb->n);
+    FwdArgs fa;
+    fa.prm = d_params_ws; fa.cam = cam_const(cam);
+    fa.rgb = rgb->data; fa.rgb_sn = rgb->sn; fa.rgb_sc = (int)rgb->sc;
+    fa.dep = depth ? depth->data : nullptr; fa.dep_sn = depth ? depth->sn : 0;
+    fa.Hin = rgb->h; fa.Win = rgb->w; fa.in_sh = (int)rgb->sh;
+    fa.rgb_o = rgb_out->data; fa.rgbo_sn = rgb_out->sn; fa.rgbo_sc = (int)rgb_out->sc; fa.rgbo_sh = (int)rgb_out->sh;
+    fa.dep_o = depth ? depth_out->data : nullptr; fa.depo_sn = depth ? depth_out->sn : 0; fa.depo_sh = depth ? (int)depth_out->sh : 0;
+    fa.mode_d = (int)depth_mode; fa.mask = d_mask_u8; fa.coverage = d_coverage;
+    set_fwd_prefetch(fa, d_params_ws, rgb->n, grd);
+    if (tma_enabled()) {                                           // TMA-staged variant: footprint boxes through shared memory
+        TmaMaps maps;
+        bool ok = true;
+        for (int c = 0; c < TMA_NH && ok; ++c) {
+            ok = encode_image_map(&maps.a[c], rgb, tma_box_h(c));
+            if (ok && depth) ok = encode_image_map(&maps.d[c], depth, tma_box_h(c));
         }
-        // compile-time geometry when input and canvas are contiguous W x H planes of a known size
-        auto planes = [&](int Wg, int Hg) {
-            return cam->W == Wg && cam->H == Hg && rgb->w == Wg && rgb->h == Hg && rgb->sh == Wg && rgb->sc == (int64_t)Wg * Hg &&
-                   rgb_out->sh == Wg && rgb_out->sc == (int64_t)Wg * Hg && (!depth || (depth->sh == Wg && depth_out->sh == Wg));
-        };
-        if (tma_enabled() && rgb->n > 0) {   // TMA-staged variant: footprint boxes through shared memory
-            TmaMaps maps;
-            bool ok = true;
-            for (int c = 0; c < TMA_NH && ok; ++c) {
-                ok = encode_image_map(&maps.a[c], rgb, tma_box_h(c));
-                if (ok && depth) ok = encode_image_map(&maps.d[c], depth, tma_box_h(c));
-            }
-            if (ok) {
-                const size_t smem = (size_t)TMA_BW * TMA_BH_MAX * 4 * (depth ? 4 : 3);
-                const dim3 tgrd((cam->W + 31) / 32, (cam->H + TMA_TILE_H - 1) / TMA_TILE_H, rgb->n);
-                // function attributes belong to the device's context: set on every launch of this opt-in path (cheap)
-                if (depth) {
-                    cudaFuncSetAttribute(warp_rgbd_tma_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TMA_BW * TMA_BH_MAX * 16);
-                    warp_rgbd_tma_kernel<true><<<tgrd, blk, smem, st>>>(fa, maps);
-                } else {
-                    cudaFuncSetAttribute(warp_rgbd_tma_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TMA_BW * TMA_BH_MAX * 12);
-                    warp_rgbd_tma_kernel<false><<<tgrd, blk, smem, st>>>(fa, maps);
-                }
-                VIDC_LAUNCH_CHECK();
-                return VIDC_OK;
-            }
+        if (ok) {
+            const size_t smem = (size_t)TMA_BW * TMA_BH_MAX * 4 * (depth ? 4 : 3);
+            const dim3 tgrd((cam->W + 31) / 32, (cam->H + TMA_TILE_H - 1) / TMA_TILE_H, rgb->n);
+            // function attributes belong to the device's context: set on every launch of this opt-in path (cheap)
+            with_flags([&](auto has_d) {
+                cudaFuncSetAttribute(warp_rgbd_tma_kernel<has_d>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+                warp_rgbd_tma_kernel<has_d><<<tgrd, blk, smem, st>>>(fa, maps);
+            }, depth != nullptr);
+            VIDC_LAUNCH_CHECK();
+            return VIDC_OK;
         }
-        const bool zero_ok = !zero_depth_out || (zero_depth_out->sw == 1 && zero_depth_out->sh == cam->W && aligned16(zero_depth_out->data) &&
-                                                  zero_depth_out->sn % 4 == 0);
-        const bool shear = shear_level() >= 1 && aligned16(rgb_out->data) && rgb_out->sn % 4 == 0 && zero_ok &&
-                           (!depth || (aligned16(depth_out->data) && depth_out->sn % 4 == 0)) &&
-                           (!d_mask_u8 || (reinterpret_cast<uintptr_t>(d_mask_u8) & 3) == 0);
-        const bool shear_geom = shear && (planes(640, 480) || planes(320, 240) || planes(640, 489) || (cam->W % 32 == 0 && planes(cam->W, cam->H)));
-        if (zero_depth_out) {
-            if (shear_geom && !tma_enabled()) { fa.dep_o = zero_depth_out->data; fa.depo_sn = zero_depth_out->sn; }     // fused into the write-out
-            else {
-                if (zero_depth_out->sw != 1 || zero_depth_out->sh != cam->W || zero_depth_out->sn != (int64_t)cam->W * cam->H)
-                    return fail(VIDC_ERR_INVALID_ARGUMENT, "depth_out: the sparse-depth path needs a contiguous (B,1,H,W) output");
-                VIDC_CUDA(cudaMemsetAsync(zero_depth_out->data, 0, sizeof(float) * (size_t)rgb->n * cam->W * cam->H, st));
-            }
-        }
-        PrefetchMaps pm;                                           // input maps of the bulk prefetch; else the per-thread form
-        fa.pf_bulk = shear_geom && fa.src_boxes && pf_bulk_enabled() &&
-                     encode_store_map(&pm.img, rgb->data, cam->W, cam->H, 3, rgb->n, rgb->sh, rgb->sc, rgb->sn, false, PF_FWD_BW, PF_FWD_BH) &&
-                     (!depth || encode_store_map(&pm.dep, depth->data, cam->W, cam->H, 1, rgb->n, depth->sh, (int64_t)cam->W * cam->H, depth->sn,
-                                                 true, PF_FWD_BW, PF_FWD_BH));
-        StoreMaps sm;
-        bool ts = shear_geom && tma_store_enabled() &&
-                  encode_store_map(&sm.img, rgb_out->data, cam->W, cam->H, 3, rgb->n, rgb_out->sh, rgb_out->sc, rgb_out->sn);
-        if (ts && depth) ts = encode_store_map(&sm.dep, depth_out->data, cam->W, cam->H, 1, rgb->n, depth_out->sh, (int64_t)cam->W * cam->H, depth_out->sn, true);
-        if (ts && zero_depth_out)                                 // sparse-depth route: the zero plane leaves through the same store
-            ts = encode_store_map(&sm.dep, zero_depth_out->data, cam->W, cam->H, 1, rgb->n, zero_depth_out->sh, (int64_t)cam->W * cam->H, zero_depth_out->sn, true);
-        if (ts && d_mask_u8) ts = encode_mask_map(&sm.mask, d_mask_u8, cam->W, cam->H, rgb->n);
-        if (shear && planes(640, 480)) {
-            launch_rgbd_shear<640, 480>(depth != nullptr, ts, grd, blk, st, fa, sm, pm);
-        } else if (shear && planes(320, 240)) {
-            launch_rgbd_shear<320, 240>(depth != nullptr, ts, grd, blk, st, fa, sm, pm);
-        } else if (shear && planes(640, 489)) {                            // the real Azure Kinect canvas: ceil(2 cy) = 489
-            launch_rgbd_shear<640, 489>(depth != nullptr, ts, grd, blk, st, fa, sm, pm);
-        } else if (shear && cam->W % 32 == 0 && planes(cam->W, cam->H)) {  // any other canvas, runtime geometry
-            launch_rgbd_shear<0, 0>(depth != nullptr, ts, grd, blk, st, fa, sm, pm);
-        } else if (planes(640, 480)) {
-            if (depth) warp_rgbd_fast_kernel<640, 480, true><<<grd, blk, 0, st>>>(fa);
-            else warp_rgbd_fast_kernel<640, 480, false><<<grd, blk, 0, st>>>(fa);
-        } else if (planes(320, 240)) {
-            if (depth) warp_rgbd_fast_kernel<320, 240, true><<<grd, blk, 0, st>>>(fa);
-            else warp_rgbd_fast_kernel<320, 240, false><<<grd, blk, 0, st>>>(fa);
-        } else {
-            if (depth) warp_rgbd_fast_kernel<0, 0, true><<<grd, blk, 0, st>>>(fa);
-            else warp_rgbd_fast_kernel<0, 0, false><<<grd, blk, 0, st>>>(fa);
-        }
+    }
+    // compile-time geometry when input and canvas are contiguous W x H planes of a known size
+    const bool compiled = contiguous_planes(cam, {rgb, rgb_out, depth, depth ? depth_out : nullptr});
+    const bool zero_ok = !zero_depth_out || (zero_depth_out->sw == 1 && zero_depth_out->sh == cam->W && aligned16(zero_depth_out->data) &&
+                                              zero_depth_out->sn % 4 == 0);
+    const bool shear = shear_level() >= 1 && aligned16(rgb_out->data) && rgb_out->sn % 4 == 0 && zero_ok &&
+                       (!depth || (aligned16(depth_out->data) && depth_out->sn % 4 == 0)) &&
+                       (!d_mask_u8 || (reinterpret_cast<uintptr_t>(d_mask_u8) & 3) == 0) && cam->W % 32 == 0 && compiled;
+    if (zero_depth_out) {
+        if (shear && !tma_enabled()) { fa.dep_o = zero_depth_out->data; fa.depo_sn = zero_depth_out->sn; }     // fused into the write-out
+        else VIDC_TRY(zero_depth_plane(cam, zero_depth_out, rgb->n, st));
+    }
+    if (!shear) {
+        with_geometry<false>(cam, compiled, [&](auto gw, auto gh, auto has_d) {
+            warp_rgbd_fast_kernel<gw, gh, has_d><<<grd, blk, 0, st>>>(fa);
+        }, depth != nullptr);
         VIDC_LAUNCH_CHECK();
         return VIDC_OK;
     }
-    if (zero_depth_out) {
-        if (zero_depth_out->sw != 1 || zero_depth_out->sh != cam->W || zero_depth_out->sn != (int64_t)cam->W * cam->H)
-            return fail(VIDC_ERR_INVALID_ARGUMENT, "depth_out: the sparse-depth path needs a contiguous (B,1,H,W) output");
-        VIDC_CUDA(cudaMemsetAsync(zero_depth_out->data, 0, sizeof(float) * (size_t)rgb->n * cam->W * cam->H, st));
-    }
-    if (depth)
-        return launch_forward<3, true, false>(cam, d_params_ws, rgb, rgb_out, VIDC_BILINEAR, depth, depth_out, depth_mode,
-                                              d_mask_u8, d_coverage, st);
-    return launch_forward<3, false, false>(cam, d_params_ws, rgb, rgb_out, VIDC_BILINEAR, nullptr, nullptr, 0, d_mask_u8,
-                                           d_coverage, st);
+    PrefetchMaps pm;                                               // input maps of the bulk prefetch; else the per-thread form
+    fa.pf_bulk = fa.src_boxes && pf_bulk_enabled() &&
+                 encode_store_map(&pm.img, rgb->data, cam->W, cam->H, 3, rgb->n, rgb->sh, rgb->sc, rgb->sn, false, PF_FWD_BW, PF_FWD_BH) &&
+                 (!depth || encode_store_map(&pm.dep, depth->data, cam->W, cam->H, 1, rgb->n, depth->sh, (int64_t)cam->W * cam->H, depth->sn,
+                                             true, PF_FWD_BW, PF_FWD_BH));
+    StoreMaps sm;
+    bool ts = tma_store_enabled() && encode_store_map(&sm.img, rgb_out->data, cam->W, cam->H, 3, rgb->n, rgb_out->sh, rgb_out->sc, rgb_out->sn);
+    if (ts && depth) ts = encode_store_map(&sm.dep, depth_out->data, cam->W, cam->H, 1, rgb->n, depth_out->sh, (int64_t)cam->W * cam->H, depth_out->sn, true);
+    if (ts && zero_depth_out)                                      // sparse-depth route: the zero plane leaves through the same store
+        ts = encode_store_map(&sm.dep, zero_depth_out->data, cam->W, cam->H, 1, rgb->n, zero_depth_out->sh, (int64_t)cam->W * cam->H, zero_depth_out->sn, true);
+    if (ts && d_mask_u8) ts = encode_mask_map(&sm.mask, d_mask_u8, cam->W, cam->H, rgb->n);
+    with_geometry<true>(cam, true, [&](auto gw, auto gh, auto has_d, auto ts_) {
+        warp_rgbd_shear_kernel<gw, gh, has_d, ts_><<<grd, blk, 0, st>>>(fa, sm, pm);
+    }, depth != nullptr, ts);
+    VIDC_LAUNCH_CHECK();
+    return VIDC_OK;
 }
 
 int vidc_warp_normals_forward(const vidc_camera* cam, const vidc_image* x, const float* d_Ig, const float* d_Ia,
@@ -733,12 +689,7 @@ int vidc_warp_with_homography(const vidc_camera* cam, const vidc_image* x, const
     cudaStream_t st = (cudaStream_t)stream;
     frame_params_from_h_kernel<<<(x->n + 63) / 64, 64, 0, st>>>(*cam, d_Hm, x->n, d_params_ws);
     VIDC_LAUNCH_CHECK();
-    switch (x->c) {
-        case 1: return launch_forward<1, false, false>(cam, d_params_ws, x, y, VIDC_BILINEAR, nullptr, nullptr, 0, nullptr, nullptr, st);
-        case 2: return launch_forward<2, false, false>(cam, d_params_ws, x, y, VIDC_BILINEAR, nullptr, nullptr, 0, nullptr, nullptr, st);
-        case 3: return launch_forward<3, false, false>(cam, d_params_ws, x, y, VIDC_BILINEAR, nullptr, nullptr, 0, nullptr, nullptr, st);
-        default: return launch_forward<4, false, false>(cam, d_params_ws, x, y, VIDC_BILINEAR, nullptr, nullptr, 0, nullptr, nullptr, st);
-    }
+    return launch_forward_planes(cam, d_params_ws, x, y, VIDC_BILINEAR, st);
 }
 
 int vidc_unwarp_normals(const vidc_camera* cam, const vidc_image* x, const float* d_Ig, const float* d_Ia,
@@ -760,100 +711,84 @@ int vidc_unwarp_normals(const vidc_camera* cam, const vidc_image* x, const float
     ia.z = z->data; ia.z_sn = z->sn; ia.z_sc = (int)z->sc; ia.z_sh = (int)z->sh;
     ia.valid = d_valid_u8;
     ia.pf_on = ia.pf_x = ia.pf_y = ia.pf_z = 0;
-    auto planes = [&](int Wg, int Hg) {
-        return cam->W == Wg && cam->H == Hg && x->sh == Wg && x->sc == (int64_t)Wg * Hg && z->sh == Wg && z->sc == (int64_t)Wg * Hg;
-    };
+    const bool compiled = contiguous_planes(cam, {x, z});
     // footprint staged in shared memory (kernels_box.cuh): contiguous planes, rows that are whole float4s
-    if (inv_box_enabled() && !tma_enabled() && d_Ig && d_Ia && x->sw == 1 && z->sw == 1 && cam->W % 4 == 0 && planes(cam->W, cam->H) &&
+    if (inv_box_enabled() && !tma_enabled() && d_Ig && d_Ia && x->sw == 1 && z->sw == 1 && cam->W % 4 == 0 && compiled &&
         aligned16(x->data) && x->sn % 4 == 0 && grd.x * grd.y <= 65535u) {     // (not with a prepared workspace: the table would go into it)
         // the per-tile box table lives behind the B parameter blocks of the caller's workspace (vidc_workspace_bytes)
         uint4* boxes = reinterpret_cast<uint4*>(d_params_ws + x->n);
         frame_params_inv_boxes_kernel<<<x->n, 320, 0, st>>>(*cam, d_Ig, d_Ia, x->n, d_params_ws, d_H_out, boxes, (int)grd.x, (int)grd.y);
-        g_launches.fetch_add(1, std::memory_order_relaxed);
-        if (planes(640, 480)) launch_unwarp_box<640, 480>(normalize != 0, d_valid_u8 != nullptr, grd, blk, st, ia, boxes);
-        else if (planes(320, 240)) launch_unwarp_box<320, 240>(normalize != 0, d_valid_u8 != nullptr, grd, blk, st, ia, boxes);
-        else launch_unwarp_box<0, 0>(normalize != 0, d_valid_u8 != nullptr, grd, blk, st, ia, boxes);
-        g_launches.fetch_add(1, std::memory_order_relaxed);
-        const cudaError_t le = cudaGetLastError();
-        if (le != cudaSuccess) return fail(VIDC_ERR_CUDA, "kernel launch failed: %s", cudaGetErrorString(le));
+        g_launches.fetch_add(1, std::memory_order_relaxed);        // checked with the second launch
+        const dim3 grd2(grd.x, (grd.y + 1) / 2, grd.z);           // one CTA = two vertically adjacent tiles
+        const int3 pf = prefetch_offset(box_prefetch_pct(), VIDC_BOX_BLOCKS, grd2);
+        with_geometry<false>(cam, true, [&](auto gw, auto gh, auto norm, auto valid) {
+            prefer_shared_carveout(unwarp_normals_box_kernel<gw, gh, norm, valid>);
+            unwarp_normals_box_kernel<gw, gh, norm, valid><<<grd2, blk, 0, st>>>(ia, boxes, (int)grd.y, pf);
+        }, normalize != 0, d_valid_u8 != nullptr);
+        VIDC_LAUNCH_CHECK();
         return VIDC_OK;
     }
-    if (!d_Ig && !d_Ia) VIDC_TRY(prepared_params(d_params_ws, x->n, d_H_out, st));
-    else VIDC_TRY(launch_params(cam, d_Ig, d_Ia, x->n, d_params_ws, st, d_H_out));
+    VIDC_TRY(warp_params(cam, d_Ig, d_Ia, x->n, d_params_ws, d_H_out, st, /*prepared_ok=*/true, /*tiles=*/false));
     if (shear_level() >= 2 && tma_store_enabled() && !d_valid_u8 && cam->W % 32 == 0 && is_channels_last3(x, cam->W, cam->H) &&
         is_channels_last3(z, cam->W, cam->H)) {                    // channels-last normals (kernels_shear_cl.cuh)
         ClStoreMaps sm;
         if (encode_cl_map(&sm.img, z->data, cam->W, cam->H, x->n)) {
-            if (normalize) launch_unwarp_cl<true>(cam, grd, blk, st, ia, sm);
-            else launch_unwarp_cl<false>(cam, grd, blk, st, ia, sm);
+            with_geometry<false>(cam, true, [&](auto gw, auto gh, auto norm) {
+                unwarp_normals_shear_cl_kernel<gw, gh, norm><<<grd, blk, 0, st>>>(ia, sm);
+            }, normalize != 0);
             VIDC_LAUNCH_CHECK();
             return VIDC_OK;
         }
     }
-    if (x->sw == 1 && z->sw == 1) {
-        if (tma_enabled() && x->n > 0) {
-            InvTmaMaps maps;
-            bool ok = true;
-            for (int c = 0; c < INV_NH && ok; ++c) ok = encode_image_map(&maps.m[c], x, inv_box_h(c), INV_BW);
-            if (ok) {
-                const int tiles_x = (cam->W + 31) / 32, tiles_y = (cam->H + 31) / 32;
-                const long long n_tiles = (long long)tiles_x * tiles_y * x->n;
-                int dev = 0, sms = 148;
-                cudaGetDevice(&dev);
-                cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-                const int ctas = (int)std::min<long long>(n_tiles, (long long)sms * 4);
-                const size_t smem = sizeof(float) * INV_STAGE_FLOATS * INV_STAGES;
-                if (normalize) {
-                    cudaFuncSetAttribute(unwarp_normals_tma_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(float) * INV_STAGE_FLOATS * INV_STAGES));
-                    unwarp_normals_tma_kernel<true><<<ctas, 288, smem, st>>>(ia, maps, tiles_x, tiles_y, (int)n_tiles);
-                } else {
-                    cudaFuncSetAttribute(unwarp_normals_tma_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(float) * INV_STAGE_FLOATS * INV_STAGES));
-                    unwarp_normals_tma_kernel<false><<<ctas, 288, smem, st>>>(ia, maps, tiles_x, tiles_y, (int)n_tiles);
-                }
-                VIDC_LAUNCH_CHECK();
-                return VIDC_OK;
-            }
-        }
-        const bool shear = shear_level() >= 2 && aligned16(z->data) && z->sn % 4 == 0 &&
-                           (!d_valid_u8 || (reinterpret_cast<uintptr_t>(d_valid_u8) & 3) == 0);
-        PrefetchMaps pm;
-        if (shear && cam->W % 32 == 0 && planes(cam->W, cam->H) && pf_bulk_enabled() && inv_prefetch_pct() > 0 &&
-            encode_store_map(&pm.img, x->data, cam->W, cam->H, 3, x->n, x->sh, x->sc, x->sn, false, PF_INV_BW, PF_INV_BH)) {
-            const int wave = (int)((long long)sm_count() * VIDC_SHEAR_BLOCKS_INV * inv_prefetch_pct() / 100);
-            ia.pf_on = 1;
-            ia.pf_x = wave % (int)grd.x; ia.pf_y = (wave / (int)grd.x) % (int)grd.y; ia.pf_z = wave / (int)(grd.x * grd.y);
-        }
-        StoreMaps sm;
-        const bool ts = shear && tma_store_enabled() && !d_valid_u8 && cam->W % 32 == 0 && planes(cam->W, cam->H) &&
-                        encode_store_map(&sm.img, z->data, cam->W, cam->H, 3, x->n, z->sh, z->sc, z->sn);
-        if (shear && planes(640, 480)) {
-            launch_unwarp_shear<640, 480>(normalize != 0, d_valid_u8 != nullptr, ts, grd, blk, st, ia, sm, pm);
-        } else if (shear && planes(320, 240)) {
-            launch_unwarp_shear<320, 240>(normalize != 0, d_valid_u8 != nullptr, ts, grd, blk, st, ia, sm, pm);
-        } else if (shear && planes(640, 489)) {
-            launch_unwarp_shear<640, 489>(normalize != 0, d_valid_u8 != nullptr, ts, grd, blk, st, ia, sm, pm);
-        } else if (shear && cam->W % 32 == 0 && planes(cam->W, cam->H)) {  // any other canvas, runtime geometry
-            launch_unwarp_shear<0, 0>(normalize != 0, d_valid_u8 != nullptr, ts, grd, blk, st, ia, sm, pm);
-        } else if (planes(640, 480)) {
-            if (normalize) unwarp_normals_fast_kernel<640, 480, true><<<grd, blk, 0, st>>>(ia);
-            else unwarp_normals_fast_kernel<640, 480, false><<<grd, blk, 0, st>>>(ia);
-        } else if (planes(320, 240)) {
-            if (normalize) unwarp_normals_fast_kernel<320, 240, true><<<grd, blk, 0, st>>>(ia);
-            else unwarp_normals_fast_kernel<320, 240, false><<<grd, blk, 0, st>>>(ia);
-        } else {
-            if (normalize) unwarp_normals_fast_kernel<0, 0, true><<<grd, blk, 0, st>>>(ia);
-            else unwarp_normals_fast_kernel<0, 0, false><<<grd, blk, 0, st>>>(ia);
-        }
+    if (x->sw != 1 || z->sw != 1) {
+        with_flags([&](auto norm) {
+            unwarp_normals_kernel<norm><<<grid2d(cam->W, cam->H, x->n, blk), blk, 0, st>>>(d_params_ws, cam_const(cam), view_in(x), view_out(z), d_valid_u8);
+        }, normalize != 0);
         VIDC_LAUNCH_CHECK();
         return VIDC_OK;
     }
-    if (normalize)
-        unwarp_normals_kernel<true><<<grid2d(cam->W, cam->H, x->n, blk), blk, 0, st>>>(d_params_ws, cam_const(cam), view_in(x), view_out(z), d_valid_u8);
-    else
-        unwarp_normals_kernel<false><<<grid2d(cam->W, cam->H, x->n, blk), blk, 0, st>>>(d_params_ws, cam_const(cam), view_in(x), view_out(z), d_valid_u8);
+    if (tma_enabled()) {
+        InvTmaMaps maps;
+        bool ok = true;
+        for (int c = 0; c < INV_NH && ok; ++c) ok = encode_image_map(&maps.m[c], x, inv_box_h(c), INV_BW);
+        if (ok) {
+            const int tiles_x = (cam->W + 31) / 32, tiles_y = (cam->H + 31) / 32;
+            const long long n_tiles = (long long)tiles_x * tiles_y * x->n;
+            const int ctas = (int)std::min<long long>(n_tiles, (long long)sm_count() * 4);
+            const size_t smem = sizeof(float) * INV_STAGE_FLOATS * INV_STAGES;
+            with_flags([&](auto norm) {
+                cudaFuncSetAttribute(unwarp_normals_tma_kernel<norm>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+                unwarp_normals_tma_kernel<norm><<<ctas, 288, smem, st>>>(ia, maps, tiles_x, tiles_y, (int)n_tiles);
+            }, normalize != 0);
+            VIDC_LAUNCH_CHECK();
+            return VIDC_OK;
+        }
+    }
+    const bool shear = shear_level() >= 2 && aligned16(z->data) && z->sn % 4 == 0 &&
+                       (!d_valid_u8 || (reinterpret_cast<uintptr_t>(d_valid_u8) & 3) == 0) && cam->W % 32 == 0 && compiled;
+    if (!shear) {
+        with_geometry<false>(cam, compiled, [&](auto gw, auto gh, auto norm) {
+            unwarp_normals_fast_kernel<gw, gh, norm><<<grd, blk, 0, st>>>(ia);
+        }, normalize != 0);
+        VIDC_LAUNCH_CHECK();
+        return VIDC_OK;
+    }
+    PrefetchMaps pm;
+    if (pf_bulk_enabled() && inv_prefetch_pct() > 0 &&
+        encode_store_map(&pm.img, x->data, cam->W, cam->H, 3, x->n, x->sh, x->sc, x->sn, false, PF_INV_BW, PF_INV_BH)) {
+        const int3 pf = prefetch_offset(inv_prefetch_pct(), VIDC_SHEAR_BLOCKS_INV, grd);
+        ia.pf_on = 1; ia.pf_x = pf.x; ia.pf_y = pf.y; ia.pf_z = pf.z;
+    }
+    StoreMaps sm;
+    const bool ts = tma_store_enabled() && !d_valid_u8 && encode_store_map(&sm.img, z->data, cam->W, cam->H, 3, x->n, z->sh, z->sc, z->sn);
+    // the TMA write-out carries no validity plane: `valid && !ts_` only keeps that impossible pair from instantiating a kernel
+    with_geometry<true>(cam, true, [&](auto gw, auto gh, auto norm, auto valid, auto ts_) {
+        unwarp_normals_shear_kernel<gw, gh, norm, valid && !ts_, ts_><<<grd, blk, 0, st>>>(ia, sm, pm);
+    }, normalize != 0, d_valid_u8 != nullptr, ts);
     VIDC_LAUNCH_CHECK();
     return VIDC_OK;
 }
+
 
 int vidc_sampler_forward_inverse(const vidc_camera* cam, const float* d_Ig, const float* d_Ia, int32_t B,
                                  vidc_frame_params* d_params_ws, float* d_Rt, float* d_grid,
@@ -1250,12 +1185,10 @@ int vidc_warp_backward(const vidc_camera* cam, const vidc_image* grad_out, const
     VIDC_CUDA(cudaMemsetAsync(d_grad_in, 0, sizeof(float) * (size_t)grad_out->n * C * Hin * Win, st));
     VIDC_TRY(launch_params(cam, d_Ig, d_Ia, grad_out->n, d_params_ws, st));
     const dim3 blk(32, 8);
-    if (inverse)
-        warp_backward_kernel<true><<<grid2d(cam->W, cam->H, grad_out->n, blk), blk, 0, st>>>(d_params_ws, cam_const(cam), view_in(grad_out), C,
-                                                                                         (int)mode, d_grad_in, (long long)C * Hin * Win, Hin * Win, Hin, Win);
-    else
-        warp_backward_kernel<false><<<grid2d(cam->W, cam->H, grad_out->n, blk), blk, 0, st>>>(d_params_ws, cam_const(cam), view_in(grad_out), C,
-                                                                                          (int)mode, d_grad_in, (long long)C * Hin * Win, Hin * Win, Hin, Win);
+    with_flags([&](auto inv) {
+        warp_backward_kernel<inv><<<grid2d(cam->W, cam->H, grad_out->n, blk), blk, 0, st>>>(d_params_ws, cam_const(cam), view_in(grad_out), C,
+                                                                                       (int)mode, d_grad_in, (long long)C * Hin * Win, Hin * Win, Hin, Win);
+    }, inverse != 0);
     VIDC_LAUNCH_CHECK();
     return VIDC_OK;
 }
@@ -1270,12 +1203,10 @@ int vidc_warp_backward_ordered(const vidc_camera* cam, const vidc_image* grad_ou
     const int C = grad_out->c;
     VIDC_TRY(launch_params(cam, d_Ig, d_Ia, grad_out->n, d_params_ws, st));
     const dim3 grd((Win + BWO_TILE - 1) / BWO_TILE, (Hin + BWO_TILE - 1) / BWO_TILE, grad_out->n);    // every grad_in element once
-    if (inverse)
-        warp_backward_ordered_kernel<true><<<grd, 256, 0, st>>>(d_params_ws, cam_const(cam), view_in(grad_out), C, (int)mode, d_grad_in,
-                                                                (long long)C * Hin * Win, Hin * Win, Hin, Win);
-    else
-        warp_backward_ordered_kernel<false><<<grd, 256, 0, st>>>(d_params_ws, cam_const(cam), view_in(grad_out), C, (int)mode, d_grad_in,
-                                                                 (long long)C * Hin * Win, Hin * Win, Hin, Win);
+    with_flags([&](auto inv) {
+        warp_backward_ordered_kernel<inv><<<grd, 256, 0, st>>>(d_params_ws, cam_const(cam), view_in(grad_out), C, (int)mode, d_grad_in,
+                                                               (long long)C * Hin * Win, Hin * Win, Hin, Win);
+    }, inverse != 0);
     VIDC_LAUNCH_CHECK();
     return VIDC_OK;
 }
