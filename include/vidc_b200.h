@@ -220,6 +220,37 @@ int vidc_warp_backward_ordered(const vidc_camera *cam, const vidc_image *grad_ou
                                int32_t B_gravity, int32_t inverse, vidc_interp mode, vidc_frame_params *d_params_ws,
                                float *d_grad_in, int32_t Hin, int32_t Win, void *stream);
 
+/* Bytes of device scratch vidc_warp_backward_params needs for a batch of B frames: one slot of fp64 partial sums per 32x32 tile
+   of the canvas and frame (176 bytes per tile).  Caller-owned, no alignment beyond 8 bytes, reusable in stream order.  Host only;
+   0 for B <= 0.  Separate from vidc_workspace_bytes, which it does not change. */
+size_t vidc_warp_backward_params_scratch_bytes(const vidc_camera *cam, int32_t B);
+
+/* Backward of the two warps w.r.t. the per-frame parameters (in the reference: torch autograd through the sampling grid of
+   F.grid_sample, :142-152 / :242-251, and through the bmm with R^T at :253).  x: the forward's input, (B,C,Hin,Win) any strides;
+   grad_out: (B,C,cam.H,cam.W) any strides; the same checks as vidc_warp_backward.
+   inverse == 0 (forward warp, any C, bilinear or nearest): d_grad_params[b] receives dL/dHinv, dL/dpx_min, dL/dpy_min, dL/dikw,
+     dL/dikh in the fields of those names;
+   inverse != 0 (inverse warp, C = 3, bilinear): dL/dH, dL/dR, dL/dpx_min, dL/dpy_min, dL/dkw, dL/dkh.
+   Every other field is 0, and 'nearest' gives 0 everywhere (ATen's grid gradient of nearest sampling is zero).  Per pixel it
+   takes ATen's grid_sampler_2d_backward grid gradient at the forward's coordinates (a non-finite coordinate contributes 0).
+   Order contract: each 32x32 output tile sums its pixels' terms in fp64 (each thread its column's rows in order, then a fixed
+   shuffle tree and the 8 warps in order) into its own slot of d_scratch (vidc_warp_backward_params_scratch_bytes); a second
+   pass adds a frame's tiles in row-major tile order and rounds once to fp32.  No global atomics: bit-reproducible from run to
+   run, at any batch position, on any stream. */
+int vidc_warp_backward_params(const vidc_camera *cam, const vidc_image *x, const vidc_image *grad_out, const float *d_Ig,
+                              const float *d_Ia, int32_t B_gravity, int32_t inverse, vidc_interp mode, vidc_frame_params *d_params_ws,
+                              void *d_scratch, vidc_frame_params *d_grad_params, void *stream);
+
+/* Backward of _build_homography (:35-58) and the per-frame bbox / scale block (:125-143): the gradients of the frame parameters
+   (d_grad_params: B entries, dL/d(field) in each field's place; fwd_col_major, inv_col_major and reserved are ignored) plus an
+   optional extra gradient of the returned Cg_H_C (d_grad_H, (B,3,3), NULL = 0) -> dL/dI_g and dL/dI_a ((B,3) each, written).
+   One thread per frame, fp64 arithmetic from I_g / I_a; the 4:3 branch and the corners that attain each min / max are those of
+   the fp32 forward, and ties split the gradient evenly (torch's backward of a full min / max).  Each frame depends on its own
+   inputs only. */
+int vidc_frame_params_backward(const vidc_camera *cam, const float *d_Ig, const float *d_Ia, int32_t B,
+                               const vidc_frame_params *d_grad_params, const float *d_grad_H, float *d_grad_Ig, float *d_grad_Ia,
+                               void *stream);
+
 /* Replaces image_sampler_forward_inverse (:158-214) including the aspect guard (:178-187).
    d_Rt (B,3,3), d_grid / d_inv_grid (B,H,W,2) contiguous; any may be NULL. */
 int vidc_sampler_forward_inverse(const vidc_camera *cam, const float *d_Ig, const float *d_Ia, int32_t B,

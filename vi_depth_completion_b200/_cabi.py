@@ -64,7 +64,13 @@ _SIGNATURES = {
                                           ctypes.c_void_p, c_f32p, ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p]),
     "vidc_warp_backward_ordered": (ctypes.c_int, [_P(VidcCamera), _P(VidcImage), c_f32p, c_f32p, ctypes.c_int32, ctypes.c_int32,
                                                   ctypes.c_int, ctypes.c_void_p, c_f32p, ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p]),
-    "vidc_sampler_forward_inverse": (ctypes.c_int, [_P(VidcCamera), c_f32p, c_f32p, ctypes.c_int32, ctypes.c_void_p, c_f32p,
+    "vidc_warp_backward_params_scratch_bytes": (ctypes.c_size_t, [_P(VidcCamera), ctypes.c_int32]),
+    "vidc_warp_backward_params": (ctypes.c_int, [_P(VidcCamera), _P(VidcImage), _P(VidcImage), c_f32p, c_f32p, ctypes.c_int32,
+                                                 ctypes.c_int32, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+                                                 ctypes.c_void_p]),
+    "vidc_frame_params_backward": (ctypes.c_int, [_P(VidcCamera), c_f32p, c_f32p, ctypes.c_int32, ctypes.c_void_p, c_f32p, c_f32p,
+                                                  c_f32p, ctypes.c_void_p]),
+    "vidc_sampler_forward_inverse":(ctypes.c_int, [_P(VidcCamera), c_f32p, c_f32p, ctypes.c_int32, ctypes.c_void_p, c_f32p,
                                                     c_f32p, c_f32p, ctypes.c_void_p]),
     "vidc_warp_normals_forward": (ctypes.c_int, [_P(VidcCamera), _P(VidcImage), c_f32p, c_f32p, ctypes.c_int32, ctypes.c_int,
                                                  ctypes.c_void_p, c_f32p, _P(VidcImage), ctypes.c_void_p]),

@@ -14,6 +14,8 @@
 //   kernels_box.cuh                     inverse warp with the footprint staged in shared memory (opt-in, VIDC_INV_BOX=1)
 //   kernels_backward.cuh                scatter-add backward
 //   kernels_backward_ordered.cuh        gather backward in one fixed summation order (deterministic)
+//   frame_params_grad.cuh               adjoint of the per-frame parameter chain (__host__ __device__, also built by the tests)
+//   kernels_grad_params.cuh             gradient w.r.t. the frame parameters and I_g / I_a, fixed reduction order
 //   kernels_sparse.cuh                  sparse depth warped analytically (row f2)
 //   tma_stage.cuh                       TMA / mbarrier PTX wrappers (bulk tensor loads and stores)
 //   kernels_tma.cuh                     opt-in TMA-staged LOAD variants (VIDC_TMA=1)
@@ -39,6 +41,7 @@
 #include "kernels_shear_cl.cuh"
 #include "kernels_backward.cuh"
 #include "kernels_backward_ordered.cuh"
+#include "kernels_grad_params.cuh"
 #include "kernels_sparse.cuh"
 #include "kernels_packed.cuh"
 #include "kernels_tma.cuh"
@@ -1207,6 +1210,59 @@ int vidc_warp_backward_ordered(const vidc_camera* cam, const vidc_image* grad_ou
         warp_backward_ordered_kernel<inv><<<grd, 256, 0, st>>>(d_params_ws, cam_const(cam), view_in(grad_out), C, (int)mode, d_grad_in,
                                                                (long long)C * Hin * Win, Hin * Win, Hin, Win);
     }, inverse != 0);
+    VIDC_LAUNCH_CHECK();
+    return VIDC_OK;
+}
+
+size_t vidc_warp_backward_params_scratch_bytes(const vidc_camera* cam, int32_t B) {
+    if (!cam || B <= 0 || cam->W <= 0 || cam->H <= 0) return 0;
+    const size_t tiles = (size_t)((cam->W + GP_TILE - 1) / GP_TILE) * ((cam->H + GP_TILE - 1) / GP_TILE);
+    return (size_t)B * tiles * GP_NV * sizeof(double);
+}
+
+int vidc_warp_backward_params(const vidc_camera* cam, const vidc_image* x, const vidc_image* grad_out, const float* d_Ig,
+                              const float* d_Ia, int32_t B_gravity, int32_t inverse, vidc_interp mode, vidc_frame_params* d_params_ws,
+                              void* d_scratch, vidc_frame_params* d_grad_params, void* stream) {
+    VIDC_TRY(check_cam(cam));
+    VIDC_TRY(check_image(x, "x", 1, 1 << 30));
+    VIDC_TRY(check_image(grad_out, "grad_out", 1, 1 << 30));
+    if (grad_out->n != B_gravity) return fail(VIDC_ERR_BATCH_MISMATCH, "grad.shape[0]=%d != I_g.shape[0]=%d", grad_out->n, B_gravity);
+    if (x->n != grad_out->n || x->c != grad_out->c) return fail(VIDC_ERR_INVALID_ARGUMENT, "x and grad_out must have the same batch and channels");
+    if (grad_out->h != cam->H || grad_out->w != cam->W) return fail(VIDC_ERR_INVALID_ARGUMENT, "grad_out must have the canvas size");
+    if (inverse && (grad_out->c != 3 || x->h != cam->H || x->w != cam->W)) return fail(VIDC_ERR_INVALID_ARGUMENT, "inverse backward needs (B,3,H,W)");
+    if (inverse && mode != VIDC_BILINEAR) return fail(VIDC_ERR_INVALID_ARGUMENT, "the inverse warp samples bilinearly only");
+    if (mode != VIDC_BILINEAR && mode != VIDC_NEAREST) return fail(VIDC_ERR_INVALID_ARGUMENT, "unknown interp mode %d", (int)mode);
+    if (x->h <= 0 || x->w <= 0) return fail(VIDC_ERR_INVALID_ARGUMENT, "bad input size");
+    const int B = grad_out->n;
+    if (B == 0) return VIDC_OK;
+    if (!d_grad_params) return fail(VIDC_ERR_INVALID_ARGUMENT, "null grad_params");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (mode == VIDC_NEAREST) {          // ATen: the grid gradient of nearest sampling is zero
+        VIDC_CUDA(cudaMemsetAsync(d_grad_params, 0, sizeof(vidc_frame_params) * (size_t)B, st));
+        return VIDC_OK;
+    }
+    if (!d_scratch) return fail(VIDC_ERR_INVALID_ARGUMENT, "null scratch (vidc_warp_backward_params_scratch_bytes)");
+    VIDC_TRY(launch_params(cam, d_Ig, d_Ia, B, d_params_ws, st));
+    const dim3 grd((cam->W + GP_TILE - 1) / GP_TILE, (cam->H + GP_TILE - 1) / GP_TILE, B);
+    double* part = static_cast<double*>(d_scratch);
+    with_flags([&](auto inv) {
+        warp_grad_params_kernel<inv><<<grd, 256, 0, st>>>(d_params_ws, cam_const(cam), view_in(x), view_in(grad_out), x->c, part);
+    }, inverse != 0);
+    VIDC_LAUNCH_CHECK();
+    grad_params_reduce_kernel<<<B, 64, 0, st>>>(part, (int)(grd.x * grd.y), inverse != 0, d_grad_params);
+    VIDC_LAUNCH_CHECK();
+    return VIDC_OK;
+}
+
+int vidc_frame_params_backward(const vidc_camera* cam, const float* d_Ig, const float* d_Ia, int32_t B,
+                               const vidc_frame_params* d_grad_params, const float* d_grad_H, float* d_grad_Ig, float* d_grad_Ia,
+                               void* stream) {
+    VIDC_TRY(check_cam(cam));
+    if (B < 0) return fail(VIDC_ERR_INVALID_ARGUMENT, "negative batch");
+    if (B == 0) return VIDC_OK;
+    if (!d_Ig || !d_Ia || !d_grad_params || !d_grad_Ig || !d_grad_Ia)
+        return fail(VIDC_ERR_INVALID_ARGUMENT, "null gravity / alignment / gradient pointer");
+    frame_params_backward_kernel<<<(B + 63) / 64, 64, 0, (cudaStream_t)stream>>>(*cam, d_Ig, d_Ia, B, d_grad_params, d_grad_H, d_grad_Ig, d_grad_Ia);
     VIDC_LAUNCH_CHECK();
     return VIDC_OK;
 }

@@ -13,8 +13,11 @@ Differences from the reference that are deliberate (see DESIGN.md):
   * any canvas size works (the reference hard-codes 240*320 staging buffers, :121-122);
   * gradients: the two reference-shaped methods are differentiable w.r.t. the image (vidc_warp_backward, bilinear /
     nearest; vidc_warp_backward_ordered, bit-reproducible, under torch.use_deterministic_algorithms(True) or with
-    deterministic_backward = True); the fused entry points and interp_mode='bicubic' are forward-only and raise
-    NotImplementedError in backward;
+    deterministic_backward = True) and, as in the reference, w.r.t. I_g and I_a, through both the warped image and the
+    returned Cg_H_C (vidc_warp_backward_params, then vidc_frame_params_backward; fixed order, bit-reproducible);
+    _build_homography is differentiable w.r.t. I_g and I_a too; the fused entry points, the params= forms, prepare(),
+    image_sampler_forward_inverse, warp_normal_image_with_gravity_center_aligned, warp_with_homography and
+    interp_mode='bicubic' are forward-only and raise NotImplementedError in backward, for the image and the gravity alike;
   * there is NO CPU / PyTorch fallback: CPU tensors raise RuntimeError.
 """
 import ctypes
@@ -65,26 +68,67 @@ def _gravity(I_g: torch.Tensor, I_a: torch.Tensor, device):
     return I_g.reshape(B, 3).contiguous(), I_a.reshape(Ba, 3).contiguous()
 
 
+def _wants_grad(*ts):
+    """True when autograd records and one of the tensors requires a gradient."""
+    return torch.is_grad_enabled() and any(isinstance(t, torch.Tensor) and t.requires_grad for t in ts)
+
+
+def _nd(t):
+    """The torch operators carry no autograd kernel: they only ever see detached tensors (torch's not-implemented fallback
+    would otherwise hand out a silent None gradient)."""
+    return t.detach() if isinstance(t, torch.Tensor) and t.requires_grad else t
+
+
+def _gravity_backward(w, g, a, gparams, gH=None):
+    """dL/dI_g, dL/dI_a from the gradients of the frame parameters (vidc_frame_params_backward)."""
+    gg, ga = torch.empty_like(g, memory_format=torch.contiguous_format), torch.empty_like(a, memory_format=torch.contiguous_format)
+    with torch.cuda.device(g.device):
+        check(lib().vidc_frame_params_backward(ctypes.byref(w._cam), g.data_ptr(), a.data_ptr(), g.shape[0], gparams.data_ptr(),
+                                               gH.data_ptr() if gH is not None else None, gg.data_ptr(), ga.data_ptr(),
+                                               _stream_ptr(g.device)))
+    return gg, ga
+
+
 class _WarpFn(torch.autograd.Function):
-    """Connects the forward-only fused kernels to autograd: backward is the scatter kernel of vidc_warp_backward
-    (gradient w.r.t. the sampled image only -- the gravity tensors come from the DataLoader and carry no gradient,
-    exactly as in the reference, where only self.cnn parameters are optimised, network_run.py:101).  Under
-    torch.use_deterministic_algorithms(True), or with the warper's deterministic_backward set to True, it is the gather
-    kernel of vidc_warp_backward_ordered instead: one fixed summation order, the same bits in every run."""
+    """Connects the forward-only fused kernels to autograd.  The image gradient is the scatter kernel of vidc_warp_backward;
+    under torch.use_deterministic_algorithms(True), or with the warper's deterministic_backward set to True, it is the gather
+    kernel of vidc_warp_backward_ordered instead: one fixed summation order, the same bits in every run.  The gradient of
+    I_g / I_a (g, a: their (B,3) views) -- the reference's autograd reaches them through the sampling grid -- is
+    vidc_warp_backward_params followed by vidc_frame_params_backward, computed only when one of them requires it; x is saved
+    for it only then."""
 
     @staticmethod
     def forward(ctx, x, out, warper, g, a, inverse, mode):
         ctx.warper, ctx.inverse, ctx.mode = warper, inverse, mode
         ctx.in_shape = tuple(x.shape)
-        ctx.save_for_backward(g, a)
+        ctx.save_for_backward(g, a, x if (ctx.needs_input_grad[3] or ctx.needs_input_grad[4]) else None)
         return out.view_as(out)
 
     @staticmethod
     def backward(ctx, grad):
-        g, a = ctx.saved_tensors
+        g, a, x = ctx.saved_tensors
+        grad = grad.float()
+        gx = _WarpFn._image_grad(ctx, g, a, grad) if ctx.needs_input_grad[0] else None
+        gg = ga = None
+        if ctx.needs_input_grad[3] or ctx.needs_input_grad[4]:
+            w = ctx.warper
+            B = g.shape[0]
+            gparams = torch.empty((B, _cabi.FRAME_PARAMS_FLOATS), dtype=torch.float32, device=grad.device)
+            scratch = torch.empty((max(int(lib().vidc_warp_backward_params_scratch_bytes(ctypes.byref(w._cam), B)), 8) // 8,),
+                                  dtype=torch.float64, device=grad.device)
+            xi, gi = _image(x), _image(grad)
+            with torch.cuda.device(grad.device):
+                check(lib().vidc_warp_backward_params(ctypes.byref(w._cam), ctypes.byref(xi), ctypes.byref(gi), g.data_ptr(),
+                                                      a.data_ptr(), B, 1 if ctx.inverse else 0, ctx.mode,
+                                                      w._params_ws(B, grad.device).data_ptr(), scratch.data_ptr(),
+                                                      gparams.data_ptr(), _stream_ptr(grad.device)))
+            gg, ga = _gravity_backward(w, g, a, gparams)
+        return gx, None, None, gg, ga, None, None
+
+    @staticmethod
+    def _image_grad(ctx, g, a, grad):
         w = ctx.warper
         B, C, Hin, Win = ctx.in_shape
-        grad = grad.float()
         det = w.deterministic_backward
         entry = lib().vidc_warp_backward_ordered if (torch.are_deterministic_algorithms_enabled() if det is None else det) \
             else lib().vidc_warp_backward
@@ -98,8 +142,56 @@ class _WarpFn(torch.autograd.Function):
                             1 if ctx.inverse else 0, ctx.mode, w._params_ws(g.shape[0], grad.device).data_ptr(),
                             gxc.data_ptr(), Hin, Win, _stream_ptr(grad.device)))
             groups.append(gxc)
-        gx = groups[0] if len(groups) == 1 else torch.cat(groups, 1)
-        return gx, None, None, None, None, None, None
+        return groups[0] if len(groups) == 1 else torch.cat(groups, 1)
+
+
+class _HomographyFn(torch.autograd.Function):
+    """Cg_H_C (one matrix) or _build_homography's (Cg_H_C, Cg_R_C, Cg_H_C_inv), differentiable w.r.t. I_g / I_a (g, a: their
+    (B,3) views) through vidc_frame_params_backward, as the reference's torch ops are."""
+
+    @staticmethod
+    def forward(ctx, g, a, warper, *mats):
+        ctx.warper, ctx.n = warper, len(mats)
+        ctx.save_for_backward(g, a)
+        return tuple(m.view_as(m) for m in mats) if len(mats) > 1 else mats[0].view_as(mats[0])
+
+    @staticmethod
+    def backward(ctx, *grads):
+        g, a = ctx.saved_tensors
+        B = g.shape[0]
+        gparams = torch.zeros((B, _cabi.FRAME_PARAMS_FLOATS), dtype=torch.float32, device=g.device)
+        gH = None
+        if ctx.n == 1:
+            gH = grads[0].float().reshape(B, 9).contiguous() if grads[0] is not None else None
+        else:
+            for k, gm in enumerate(grads):                      # fields H, R, Hinv: floats 0, 9, 18
+                if gm is not None:
+                    gparams[:, 9 * k:9 * k + 9] = gm.float().reshape(B, 9)
+        gg, ga = _gravity_backward(ctx.warper, g, a, gparams, gH)
+        return (gg, ga, None) + (None,) * ctx.n
+
+
+class _NoGravityBackward(torch.autograd.Function):
+    """Outputs of entry points whose gravity (or Cg_H_C) input requires a gradient they do not compute."""
+
+    @staticmethod
+    def forward(ctx, out, *grav):
+        return out.view_as(out)
+
+    @staticmethod
+    def backward(ctx, *grads):
+        raise NotImplementedError(
+            "vi_depth_completion_b200: this entry point is not differentiable w.r.t. I_g / I_a (or Cg_H_C); gravity gradients "
+            "are computed by warp_with_gravity_center_aligned (bilinear / nearest), "
+            "inverse_warp_normal_image_with_gravity_center_aligned and _build_homography")
+
+
+def _no_gravity_grad(outs, *grav):
+    """Wrap the floating-point outputs so that a backward into the gravity raises instead of handing out None."""
+    grav = tuple(t for t in grav if isinstance(t, torch.Tensor) and t.requires_grad)
+    if not grav or not torch.is_grad_enabled():
+        return outs
+    return tuple(_NoGravityBackward.apply(o, *grav) if isinstance(o, torch.Tensor) and o.is_floating_point() else o for o in outs)
 
 
 class _NoBackward(torch.autograd.Function):
@@ -154,10 +246,11 @@ def _check_interp_mode(interp_mode, allow_bicubic=False):
 class FrameParams:
     """Per-frame parameters of one batch, prepared once (Warping2DOFAlignment.prepare) and shared by warp_rgbd and
     unwarp_normals: the reference rebuilds them in every call (:124, :225) from the same I_g / I_a.  `H` is Cg_H_C (B,3,3)."""
-    __slots__ = ("ws", "H", "B", "device", "intr")
+    __slots__ = ("ws", "H", "B", "device", "intr", "grav")
 
-    def __init__(self, ws, H, intr):
+    def __init__(self, ws, H, intr, grav=()):
         self.ws, self.H, self.B, self.device, self.intr = ws, H, H.shape[0], H.device, intr
+        self.grav = tuple(t for t in grav if isinstance(t, torch.Tensor) and t.requires_grad)   # forward-only w.r.t. these
 
 
 class Warping2DOFAlignment:
@@ -223,8 +316,13 @@ class Warping2DOFAlignment:
     # networks/warping_2dof_alignment.py:35-58
     def _build_homography(self, I_g, I_a):
         ops = _torchops.ops()
+        grav_grad = _wants_grad(I_g, I_a)
         if ops is not None and isinstance(I_g, torch.Tensor) and isinstance(I_a, torch.Tensor):
-            return _op(ops.build_homography, I_g, I_a, *self._intr)
+            out = _op(ops.build_homography, _nd(I_g), _nd(I_a), *self._intr)
+            if not grav_grad:
+                return out
+            g, a = _gravity(I_g, I_a, I_g.device)
+            return _HomographyFn.apply(g, a, self, *out)
         _require_cuda_f32(I_g, "I_g")
         device = I_g.device
         g, a = _gravity(I_g, I_a, device)
@@ -233,6 +331,8 @@ class Warping2DOFAlignment:
         with torch.cuda.device(device):
             check(lib().vidc_build_homography(ctypes.byref(self._cam), g.data_ptr(), a.data_ptr(), B,
                                               out[0].data_ptr(), out[1].data_ptr(), out[2].data_ptr(), _stream_ptr(device)))
+        if grav_grad:
+            return _HomographyFn.apply(g, a, self, out[0], out[1], out[2])
         return out[0], out[1], out[2]
 
     def frame_params(self, I_g, I_a):
@@ -245,7 +345,7 @@ class Warping2DOFAlignment:
         with torch.cuda.device(device):
             check(lib().vidc_frame_params_compute(ctypes.byref(self._cam), g.data_ptr(), a.data_ptr(), B, out.data_ptr(),
                                                   _stream_ptr(device)))
-        return out
+        return _no_gravity_grad((out,), I_g, I_a)[0]
 
     def _empty_like_canvas(self, x):
         B, C = x.shape[0], x.shape[1]
@@ -266,11 +366,12 @@ class Warping2DOFAlignment:
         device = x.device
         ops = _torchops.ops()
         needs_graph = torch.is_grad_enabled() and x.requires_grad
+        grav_grad = _wants_grad(I_g, I_a)
         if ops is not None and isinstance(I_g, torch.Tensor) and isinstance(I_a, torch.Tensor):
             # thin torch C++ extension; the operators carry no autograd kernel -- the graph is attached below (_attach), so they
             # only ever see detached tensors (torch's not-implemented fallback would otherwise hand out silent zero gradients)
-            Cg_H_C, y = _op(ops.warp_forward, x.detach() if needs_graph else x, I_g, I_a, *self._intr, mode)
-            g, a = _gravity(I_g, I_a, device) if needs_graph else (None, None)
+            Cg_H_C, y = _op(ops.warp_forward, x.detach() if needs_graph else x, _nd(I_g), _nd(I_a), *self._intr, mode)
+            g, a = _gravity(I_g, I_a, device) if (needs_graph or grav_grad) else (None, None)
         else:
             g, a = _gravity(I_g, I_a, device)
             y = self._empty_like_canvas(x)
@@ -281,8 +382,15 @@ class Warping2DOFAlignment:
                                               mode, self._params_ws(g.shape[0], device).data_ptr(), Cg_H_C.data_ptr(),
                                               ctypes.byref(yi), _stream_ptr(device)))
         # the scatter kernel of vidc_warp_backward covers bilinear and nearest; bicubic is forward-only
-        if needs_graph:
-            y = _attach(x, y) if mode == _cabi.VIDC_BICUBIC else _attach(x, y, self, g, a, False, mode)
+        if mode == _cabi.VIDC_BICUBIC:
+            if needs_graph:
+                y = _attach(x, y)
+            Cg_H_C, y = _no_gravity_grad((Cg_H_C, y), I_g, I_a)
+        else:
+            if needs_graph or grav_grad:
+                y = _WarpFn.apply(x, y, self, g, a, False, mode)
+            if grav_grad:
+                Cg_H_C = _HomographyFn.apply(g, a, self, Cg_H_C)
         if flag_fix_return:                                     # :153-154
             return Cg_H_C, y.view(x.shape[0], y.shape[2], y.shape[3])
         return Cg_H_C, y
@@ -300,24 +408,27 @@ class Warping2DOFAlignment:
             check(lib().vidc_sampler_forward_inverse(ctypes.byref(self._cam), g.data_ptr(), a.data_ptr(), B,
                                                      self._params_ws(B, device).data_ptr(), Rt.data_ptr(), grid.data_ptr(),
                                                      inv_grid.data_ptr(), _stream_ptr(device)))
-        return Rt, grid, inv_grid
+        return _no_gravity_grad((Rt, grid, inv_grid), I_g, I_a)
 
     # networks/warping_2dof_alignment.py:216-255
     def inverse_warp_normal_image_with_gravity_center_aligned(self, x, I_g, I_a):
-        return self._unwarp(x, I_g, I_a, normalize=False)[:2]
+        return self._unwarp(x, I_g, I_a, normalize=False, gravity_grad=True)[:2]
 
-    def _unwarp(self, x, I_g, I_a, normalize, want_valid=False):
+    def _unwarp(self, x, I_g, I_a, normalize, want_valid=False, gravity_grad=False):
+        """gravity_grad: the reference-shaped method, differentiable w.r.t. I_g / I_a; the fused entry point (unwarp_normals)
+        is forward-only w.r.t. them."""
         _require_cuda_f32(x, "x")
         if x.dim() != 4:
             raise RuntimeError(f"x: expected a 4-D tensor, got {x.dim()}-D")
         device = x.device
         ops = _torchops.ops()
+        grav_grad = _wants_grad(I_g, I_a)
         if ops is not None and not want_valid and isinstance(I_g, torch.Tensor) and isinstance(I_a, torch.Tensor):
             needs_graph = torch.is_grad_enabled() and x.requires_grad
-            Cg_H_C, z = _op(ops.unwarp_normals, x.detach() if needs_graph else x, I_g, I_a, *self._intr, bool(normalize))
-            if needs_graph:
+            Cg_H_C, z = _op(ops.unwarp_normals, x.detach() if needs_graph else x, _nd(I_g), _nd(I_a), *self._intr, bool(normalize))
+            if needs_graph or grav_grad:
                 g, a = _gravity(I_g, I_a, device)
-                z = _attach(x, z, self, g, a, True, _cabi.VIDC_BILINEAR) if not normalize else _attach(x, z)
+                return self._unwarp_graph(x, z, Cg_H_C, g, a, I_g, I_a, normalize, needs_graph, grav_grad and gravity_grad) + (None,)
             return Cg_H_C, z, None
         g, a = _gravity(I_g, I_a, device)
         z = self._empty_like_canvas(x)
@@ -329,8 +440,14 @@ class Warping2DOFAlignment:
                                             1 if normalize else 0, self._params_ws(g.shape[0], device).data_ptr(),
                                             Cg_H_C.data_ptr(), ctypes.byref(zi), valid.data_ptr() if want_valid else None,
                                             _stream_ptr(device)))
+        needs_graph = torch.is_grad_enabled() and x.requires_grad
+        return self._unwarp_graph(x, z, Cg_H_C, g, a, I_g, I_a, normalize, needs_graph, grav_grad and gravity_grad) + (valid,)
+
+    def _unwarp_graph(self, x, z, Cg_H_C, g, a, I_g, I_a, normalize, needs_graph, grav_diff):
+        if grav_diff and not normalize:
+            return _HomographyFn.apply(g, a, self, Cg_H_C), _WarpFn.apply(x, z, self, g, a, True, _cabi.VIDC_BILINEAR)
         z = _attach(x, z, self, g, a, True, _cabi.VIDC_BILINEAR) if not normalize else _attach(x, z)
-        return Cg_H_C, z, valid
+        return _no_gravity_grad((Cg_H_C, z), I_g, I_a)
 
     # networks/warping_2dof_alignment.py:258-290.  The reference method cannot run (:259 unpacks three
     # return values into two); this implements its evident intent: forward warp, then z = R y.
@@ -349,7 +466,7 @@ class Warping2DOFAlignment:
                                                   g.shape[0], mode,
                                                   self._params_ws(g.shape[0], device).data_ptr(), Cg_H_C.data_ptr(),
                                                   ctypes.byref(zi), _stream_ptr(device)))
-        return Cg_H_C, _attach(x, z)
+        return _no_gravity_grad((Cg_H_C, _attach(x, z)), I_g, I_a)
 
     # networks/warping_2dof_alignment.py:292-310 (numpy single-image variant, non-uniform kw/kh)
     def warp_with_homography(self, x, Cg_H_C):
@@ -370,7 +487,7 @@ class Warping2DOFAlignment:
             check(lib().vidc_warp_with_homography(ctypes.byref(self._cam), ctypes.byref(xi), Hd.data_ptr(), Hd.shape[0],
                                                   self._params_ws(Hd.shape[0], device).data_ptr(), ctypes.byref(yi),
                                                   _stream_ptr(device)))
-        return Cg_H_C, _attach(x, y)
+        return Cg_H_C, _no_gravity_grad((_attach(x, y),), Cg_H_C)[0]
 
     # ---- additive fused entry points (SURVEY.md section 8b) ------------------------------------
     def prepare(self, I_g, I_a):
@@ -378,9 +495,10 @@ class Warping2DOFAlignment:
         computed ONCE for a batch: pass the result as `params=` to warp_rgbd and unwarp_normals, which then launch no
         per-frame kernel of their own.  Valid for this camera and these I_g / I_a values."""
         ops = _torchops.ops()
+        grav = (I_g, I_a) if _wants_grad(I_g, I_a) else ()
         if ops is not None and isinstance(I_g, torch.Tensor) and isinstance(I_a, torch.Tensor):
-            ws, H = _op(ops.frame_params, I_g, I_a, *self._intr)
-            return FrameParams(ws, H, self._intr)
+            ws, H = _op(ops.frame_params, _nd(I_g), _nd(I_a), *self._intr)
+            return FrameParams(ws, _no_gravity_grad((H,), *grav)[0], self._intr, grav)
         _require_cuda_f32(I_g, "I_g")
         device = I_g.device
         g, a = _gravity(I_g, I_a, device)
@@ -389,7 +507,7 @@ class Warping2DOFAlignment:
         with torch.cuda.device(device):
             check(lib().vidc_frame_params_prepare(ctypes.byref(self._cam), g.data_ptr(), a.data_ptr(), g.shape[0], ws.data_ptr(),
                                                   H.data_ptr(), _stream_ptr(device)))
-        return FrameParams(ws, H, self._intr)
+        return FrameParams(ws, _no_gravity_grad((H,), *grav)[0], self._intr, grav)
 
     def _prepared(self, params, x, name):
         if not isinstance(params, FrameParams):
@@ -432,18 +550,18 @@ class Warping2DOFAlignment:
                                                _stream_ptr(device)))
             if x_depth.dim() == 3:
                 depth_w = depth_w.view(depth_w.shape[0], depth_w.shape[2], depth_w.shape[3])
-            return p.H, _attach(x_rgb, rgb_w), _attach(x_depth, depth_w), mask
+            return _no_gravity_grad((p.H, _attach(x_rgb, rgb_w), _attach(x_depth, depth_w), mask), *p.grav)
         if I_g is None or I_a is None:
             raise RuntimeError("warp_rgbd: pass I_g and I_a, or params=prepare(I_g, I_a)")
         if (ops is not None and with_mask and not with_coverage and isinstance(x_depth, torch.Tensor) and x_rgb.dim() == 4
                 and isinstance(I_g, torch.Tensor) and isinstance(I_a, torch.Tensor)):
             d4 = x_depth.view(x_depth.shape[0], 1, x_depth.shape[1], x_depth.shape[2]) if x_depth.dim() == 3 else x_depth
             Cg_H_C, rgb_w, depth_w, mask = _op(ops.warp_rgbd, x_rgb.detach() if x_rgb.requires_grad else x_rgb,
-                                               d4.detach() if d4.requires_grad else d4, I_g, I_a, *self._intr,
+                                               d4.detach() if d4.requires_grad else d4, _nd(I_g), _nd(I_a), *self._intr,
                                                _cabi.VIDC_BILINEAR if depth_mode == "bilinear" else _cabi.VIDC_NEAREST)
             if x_depth.dim() == 3:
                 depth_w = depth_w.view(depth_w.shape[0], depth_w.shape[2], depth_w.shape[3])
-            return Cg_H_C, _attach(x_rgb, rgb_w), _attach(x_depth, depth_w), mask          # forward-only: backward raises
+            return _no_gravity_grad((Cg_H_C, _attach(x_rgb, rgb_w), _attach(x_depth, depth_w), mask), I_g, I_a)   # forward-only
         g, a = _gravity(I_g, I_a, device)
         B = x_rgb.shape[0]
         squeeze = False
@@ -474,6 +592,7 @@ class Warping2DOFAlignment:
         if squeeze:
             depth_w = depth_w.view(B, depth_w.shape[2], depth_w.shape[3])
         out = (Cg_H_C, _attach(x_rgb, rgb_w), depth_w if depth_w is None else _attach(x_depth, depth_w), mask)   # forward-only
+        out = _no_gravity_grad(out, I_g, I_a)
         return out + (cov,) if with_coverage else out
 
     def warp_rgb_sparse_depth(self, x_rgb, tracks, counts, fc, cc, I_g, I_a, depth_mode='bilinear', with_mask=True, with_coverage=False):
@@ -510,7 +629,7 @@ class Warping2DOFAlignment:
                                                    self._params_ws(g.shape[0], device).data_ptr(), Cg_H_C.data_ptr(), ctypes.byref(rwi),
                                                    ctypes.byref(dwi), mask.data_ptr() if with_mask else None,
                                                    cov.data_ptr() if with_coverage else None, _stream_ptr(device)))
-        out = (Cg_H_C, _attach(x_rgb, rgb_w), depth_w, mask)                       # forward-only
+        out = _no_gravity_grad((Cg_H_C, _attach(x_rgb, rgb_w), depth_w, mask), I_g, I_a)          # forward-only
         return out + (cov,) if with_coverage else out
 
     def warp_rgbd_packed(self, x_rgbd, I_g, I_a, depth_mode='bilinear', with_mask=True, with_coverage=False):
@@ -533,7 +652,7 @@ class Warping2DOFAlignment:
                                               self._params_ws(g.shape[0], device).data_ptr(), Cg_H_C.data_ptr(), y.data_ptr(),
                                               mask.data_ptr() if with_mask else None, cov.data_ptr() if with_coverage else None,
                                               _stream_ptr(device)))
-        out = (Cg_H_C, _attach(x_rgbd, y), mask)                                   # forward-only
+        out = _no_gravity_grad((Cg_H_C, _attach(x_rgbd, y), mask), I_g, I_a)       # forward-only
         return out + (cov,) if with_coverage else out
 
     def unwarp_normals(self, y, I_g=None, I_a=None, normalize=True, with_valid=False, params=None):
@@ -554,7 +673,7 @@ class Warping2DOFAlignment:
                 with torch.cuda.device(y.device):
                     check(lib().vidc_unwarp_normals(ctypes.byref(self._cam), ctypes.byref(yi), None, None, p.B, 1 if normalize else 0,
                                                     p.ws.data_ptr(), None, ctypes.byref(zi), None, _stream_ptr(y.device)))
-            return p.H, (_attach(y, z) if needs_graph else z)           # forward-only with a prepared workspace
+            return _no_gravity_grad((p.H, (_attach(y, z) if needs_graph else z)), *p.grav)   # forward-only with a prepared workspace
         if I_g is None or I_a is None:
             raise RuntimeError("unwarp_normals: pass I_g and I_a, or params=prepare(I_g, I_a)")
         H, z, valid = self._unwarp(y, I_g, I_a, normalize=normalize, want_valid=with_valid)
