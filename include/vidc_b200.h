@@ -181,6 +181,19 @@ int vidc_warp_rgbd(const vidc_camera *cam, const vidc_image *rgb, const vidc_ima
                    const vidc_image *rgb_out, const vidc_image *depth_out,
                    uint8_t *d_mask_u8, uint32_t *d_coverage, void *stream);
 
+/* vidc_warp_rgbd with the RGB frames as the loader decodes them (dataset.py:468-471): d_rgb_hwc is (B, Hin, Win, 3) uint8,
+   contiguous, at any byte alignment (the layout vidc_to_tensor_u8 takes).  Every other argument, check and status is
+   vidc_warp_rgbd's, including depth = NULL, the optional mask and coverage, and d_Ig = d_Ia = NULL with a workspace from
+   vidc_frame_params_prepare.  Outputs are bit-identical to vidc_to_tensor_u8 followed by vidc_warp_rgbd: each tap is
+   converted to x / 255 before the unchanged interpolation, so the float copy of the frames is never written (RGB + depth +
+   mask: 24 B/px of HBM traffic instead of 48 B/px for the two passes).  Frames of the canvas size with a canvas width that
+   is a multiple of 32 run the sheared kernels; everything else takes the strided kernel. */
+int vidc_warp_rgbd_u8(const vidc_camera *cam, const uint8_t *d_rgb_hwc, int32_t B, int32_t Hin, int32_t Win,
+                      const vidc_image *depth, const float *d_Ig, const float *d_Ia, int32_t B_gravity,
+                      vidc_interp depth_mode, vidc_frame_params *d_params_ws, float *d_H_out,
+                      const vidc_image *rgb_out, const vidc_image *depth_out,
+                      uint8_t *d_mask_u8, uint32_t *d_coverage, void *stream);
+
 /* Packed variant of vidc_warp_rgbd for callers that hold RGB + depth interleaved: d_in is (B, Hin, Win, 4) fp32
    (channels-last, C = 4: R, G, B, depth), d_out is (B, cam.H, cam.W, 4); both contiguous and 16-byte aligned.
    Every bilinear tap is one 128-bit load and every pixel one 128-bit store.  Same results per channel. */

@@ -55,6 +55,9 @@ _SIGNATURES = {
     "vidc_warp_rgbd": (ctypes.c_int, [_P(VidcCamera), _P(VidcImage), _P(VidcImage), c_f32p, c_f32p, ctypes.c_int32, ctypes.c_int,
                                       ctypes.c_void_p, c_f32p, _P(VidcImage), _P(VidcImage), ctypes.c_void_p, ctypes.c_void_p,
                                       ctypes.c_void_p]),
+    "vidc_warp_rgbd_u8": (ctypes.c_int, [_P(VidcCamera), ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, _P(VidcImage),
+                                         c_f32p, c_f32p, ctypes.c_int32, ctypes.c_int, ctypes.c_void_p, c_f32p, _P(VidcImage),
+                                         _P(VidcImage), ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p]),
     "vidc_warp_rgbd_packed": (ctypes.c_int, [_P(VidcCamera), c_f32p, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, c_f32p, c_f32p,
                                              ctypes.c_int32, ctypes.c_int, ctypes.c_void_p, c_f32p, c_f32p, ctypes.c_void_p,
                                              ctypes.c_void_p, ctypes.c_void_p]),

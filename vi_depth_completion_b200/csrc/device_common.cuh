@@ -8,7 +8,16 @@ namespace vidc_k {
 // ------------------------------------------------------------------------------------------
 // device-side image view (strides in elements; intra-frame offsets fit 32 bits)
 struct ImgView {
+    using elem = float;
     const float* __restrict__ p;
+    int c, h, w;
+    long long sn;
+    int sc, sh, sw;
+};
+// (B,H,W,3) uint8 frames as the loader holds them (vidc_warp_rgbd_u8): element strides (3 H W, 1, 3 W, 3)
+struct ImgViewU8 {
+    using elem = uint8_t;
+    const uint8_t* __restrict__ p;
     int c, h, w;
     long long sn;
     int sc, sh, sw;
@@ -61,11 +70,17 @@ __device__ __forceinline__ Taps bilinear_taps(float ix, float iy, int Hin, int W
     return t;
 }
 
-__device__ __forceinline__ float sample_bilinear(const float* __restrict__ plane, const Taps& t) {
-    const float v_nw = t.b_nw ? __ldg(plane + t.o_nw) : 0.0f;
-    const float v_ne = t.b_ne ? __ldg(plane + t.o_ne) : 0.0f;
-    const float v_sw = t.b_sw ? __ldg(plane + t.o_sw) : 0.0f;
-    const float v_se = t.b_se ? __ldg(plane + t.o_se) : 0.0f;
+// One tap as fp32: a float element as it is, a uint8 element as ToTensor makes it (x / 255, vidc::u8_to_unit), so a warp
+// of uint8 frames gives the bits of the same warp of to_tensor(frames).
+__device__ __forceinline__ float load_tap(const float* __restrict__ p) { return __ldg(p); }
+__device__ __forceinline__ float load_tap(const uint8_t* __restrict__ p) { return vidc::u8_to_unit(__ldg(p)); }
+
+template <typename T>
+__device__ __forceinline__ float sample_bilinear(const T* __restrict__ plane, const Taps& t) {
+    const float v_nw = t.b_nw ? load_tap(plane + t.o_nw) : 0.0f;
+    const float v_ne = t.b_ne ? load_tap(plane + t.o_ne) : 0.0f;
+    const float v_sw = t.b_sw ? load_tap(plane + t.o_sw) : 0.0f;
+    const float v_se = t.b_se ? load_tap(plane + t.o_se) : 0.0f;
     // ATen accumulates nw, ne, sw, se with fused multiply-adds; a skipped (out-of-bounds) tap
     // equals adding 0 * w exactly.
     float acc = v_nw * t.w_nw;
@@ -75,11 +90,12 @@ __device__ __forceinline__ float sample_bilinear(const float* __restrict__ plane
     return acc;
 }
 
-__device__ __forceinline__ float sample_nearest(const float* __restrict__ plane, float ix, float iy,
+template <typename T>
+__device__ __forceinline__ float sample_nearest(const T* __restrict__ plane, float ix, float iy,
                                                 int Hin, int Win, int sh, int sw) {
     const int xn = (int)rintf(ix), yn = (int)rintf(iy);      // round half to even, as nearbyint
     const bool in = (unsigned)xn < (unsigned)Win && (unsigned)yn < (unsigned)Hin;
-    return in ? __ldg(plane + yn * sh + xn * sw) : 0.0f;
+    return in ? load_tap(plane + yn * sh + xn * sw) : 0.0f;
 }
 
 // ---- bicubic (interp_mode='bicubic', A = -0.75): ATen's cubic convolution as torch 2.11 rounds it on CPU (oracle/warp_oracle.c,
@@ -113,13 +129,14 @@ __device__ __forceinline__ CubicTaps bicubic_taps(float rx, float ry, int Hin, i
     }
     return t;
 }
-__device__ __forceinline__ float sample_bicubic(const float* __restrict__ plane, const CubicTaps& t, int sh, int sw) {
+template <typename T>
+__device__ __forceinline__ float sample_bicubic(const T* __restrict__ plane, const CubicTaps& t, int sh, int sw) {
     float rows[4];
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
         float v[4];
 #pragma unroll
-        for (int j = 0; j < 4; ++j) v[j] = (t.yi[i] >= 0 && t.xi[j] >= 0) ? __ldg(plane + t.yi[i] * sh + t.xi[j] * sw) : 0.0f;
+        for (int j = 0; j < 4; ++j) v[j] = (t.yi[i] >= 0 && t.xi[j] >= 0) ? load_tap(plane + t.yi[i] * sh + t.xi[j] * sw) : 0.0f;
         float acc = fmaf(t.cx[0], v[0], t.cx[1] * v[1]);          // ((c0 v0 + c1 v1) + c2 v2) + c3 v3, first add contracted
         acc = acc + t.cx[2] * v[2];
         acc = acc + t.cx[3] * v[3];

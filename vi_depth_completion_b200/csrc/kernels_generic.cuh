@@ -8,12 +8,13 @@ namespace vidc_k {
 // ------------------------------------------------------------------------------------------
 // Forward warp.  MODE_A: interpolation of image A (C_A channels, 1..4); image D (1 channel, optional)
 // has its own mode.  ROT: rotate the 3 channels of A by R after sampling (:288, intent of :258-290).
-template <int C_A, bool HAS_D, bool ROT>
-__global__ void __launch_bounds__(256)
-warp_forward_kernel(const vidc_frame_params* __restrict__ prm, CamConst cam,
-                    ImgView a, ImgViewOut ya, int mode_a,
-                    ImgView d, ImgViewOut yd, int mode_d,
-                    unsigned char* __restrict__ mask, unsigned int* __restrict__ coverage) {
+// View: ImgView (fp32) or ImgViewU8 (uint8 frames, every tap through load_tap).
+template <int C_A, bool HAS_D, bool ROT, typename View>
+__device__ __forceinline__ void
+warp_forward_pixel(const vidc_frame_params* __restrict__ prm, CamConst cam,
+                   View a, ImgViewOut ya, int mode_a,
+                   ImgView d, ImgViewOut yd, int mode_d,
+                   unsigned char* __restrict__ mask, unsigned int* __restrict__ coverage) {
     const int b = blockIdx.z;
     const int X = blockIdx.x * blockDim.x + threadIdx.x;
     const int Y = blockIdx.y * blockDim.y + threadIdx.y;
@@ -30,7 +31,7 @@ warp_forward_kernel(const vidc_frame_params* __restrict__ prm, CamConst cam,
         {
             float ix, iy;
             forward_coords(Hi, px_min, py_min, ikw, ikh, cam, (float)X, (float)Y, (float)a.w, (float)a.h, ix, iy);
-            const float* __restrict__ base = a.p + (long long)b * a.sn;
+            const typename View::elem* __restrict__ base = a.p + (long long)b * a.sn;
             if (mode_a == VIDC_BILINEAR) {
                 const Taps t = bilinear_taps(ix, iy, a.h, a.w, a.sh, a.sw);
 #pragma unroll
@@ -85,6 +86,23 @@ warp_forward_kernel(const vidc_frame_params* __restrict__ prm, CamConst cam,
         __syncthreads();
         if (tid == 0 && cta_count) atomicAdd(coverage + b, cta_count);
     }
+}
+template <int C_A, bool HAS_D, bool ROT>
+__global__ void __launch_bounds__(256)
+warp_forward_kernel(const vidc_frame_params* __restrict__ prm, CamConst cam,
+                    ImgView a, ImgViewOut ya, int mode_a,
+                    ImgView d, ImgViewOut yd, int mode_d,
+                    unsigned char* __restrict__ mask, unsigned int* __restrict__ coverage) {
+    warp_forward_pixel<C_A, HAS_D, ROT>(prm, cam, a, ya, mode_a, d, yd, mode_d, mask, coverage);
+}
+// (B,Hin,Win,3) uint8 RGB of vidc_warp_rgbd_u8 where the sheared uint8 kernel does not apply (bilinear RGB, optional depth)
+template <bool HAS_D>
+__global__ void __launch_bounds__(256)
+warp_forward_u8_kernel(const vidc_frame_params* __restrict__ prm, CamConst cam,
+                       ImgViewU8 a, ImgViewOut ya, int mode_a,
+                       ImgView d, ImgViewOut yd, int mode_d,
+                       unsigned char* __restrict__ mask, unsigned int* __restrict__ coverage) {
+    warp_forward_pixel<3, HAS_D, false>(prm, cam, a, ya, mode_a, d, yd, mode_d, mask, coverage);
 }
 
 // Inverse warp of normals: gather + R^T rotation (+ F.normalize), ref :242-253, surface_normal.py:170

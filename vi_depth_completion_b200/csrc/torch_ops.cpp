@@ -128,6 +128,42 @@ std::tuple<at::Tensor, at::Tensor, at::Tensor, at::Tensor> warp_rgbd(const at::T
     return {Hm, rgb_w, depth_w, mask};
 }
 
+// ---- the same on (B,h,w,3) uint8 frames as the loader decodes them (vidc_warp_rgbd_u8): RGB comes out as NCHW float32 -------
+void check_u8_frames(const at::Tensor& rgb) {
+    TORCH_CHECK(rgb.is_cuda(), "x_rgb: expected a CUDA tensor (this module has no CPU fallback), got device ", rgb.device());
+    TORCH_CHECK(rgb.scalar_type() == at::kByte, "x_rgb: expected scalar type Byte but found ", rgb.scalar_type());
+    TORCH_CHECK(rgb.dim() == 4 && rgb.size(3) == 3, "x_rgb: expected (B,h,w,3) uint8 frames, got ", rgb.sizes());
+    TORCH_CHECK(rgb.is_contiguous(), "x_rgb: expected contiguous (B,h,w,3) frames");
+}
+at::Tensor rgb_canvas_u8(const at::Tensor& rgb, int64_t H, int64_t W) {
+    return at::empty({rgb.size(0), 3, H, W}, rgb.options().dtype(at::kFloat));
+}
+int warp_rgbd_u8_call(const vidc_camera& cam, const at::Tensor& rgb, const at::Tensor& depth, const float* g, const float* a, int64_t B_gravity,
+                      int64_t depth_mode, const at::Tensor& ws, float* Hm, const at::Tensor& rgb_w, const at::Tensor& depth_w, const at::Tensor& mask) {
+    const vidc_image di = image_of(depth), rwi = image_of(rgb_w), dwi = image_of(depth_w);
+    return vidc_warp_rgbd_u8(&cam, rgb.data_ptr<uint8_t>(), (int32_t)rgb.size(0), (int32_t)rgb.size(1), (int32_t)rgb.size(2), &di, g, a,
+                             (int32_t)B_gravity, (vidc_interp)depth_mode, reinterpret_cast<vidc_frame_params*>(ws.data_ptr<float>()), Hm,
+                             &rwi, &dwi, mask.data_ptr<uint8_t>(), nullptr, at::cuda::getCurrentCUDAStream().stream());
+}
+std::tuple<at::Tensor, at::Tensor, at::Tensor, at::Tensor> warp_rgbd_u8(const at::Tensor& rgb, const at::Tensor& depth, const at::Tensor& I_g,
+                                                                        const at::Tensor& I_a, double fx, double fy, double cx, double cy,
+                                                                        int64_t depth_mode) {
+    check_u8_frames(rgb);
+    check_f32_cuda(depth, "x_depth");
+    TORCH_CHECK(depth.dim() == 4, "warp_rgbd_u8: expected (B,1,h,w) depth");
+    TORCH_CHECK(depth.device() == rgb.device(), "x_depth must live on ", rgb.device(), ", got ", depth.device());
+    const vidc_camera cam = make_camera(fx, fy, cx, cy);
+    const c10::cuda::CUDAGuard guard(rgb.device());
+    auto [g, a] = gravity(I_g, I_a, rgb.device());
+    at::Tensor rgb_w = rgb_canvas_u8(rgb, cam.H, cam.W), depth_w = canvas_like(depth, cam);
+    at::Tensor mask = at::empty({rgb.size(0), 1, cam.H, cam.W}, rgb.options());
+    at::Tensor Hm = at::empty({g.size(0), 3, 3}, depth.options());
+    at::Tensor ws = workspace(cam, g.size(0), depth.options());
+    check_status(warp_rgbd_u8_call(cam, rgb, depth, g.data_ptr<float>(), a.data_ptr<float>(), g.size(0), depth_mode, ws, Hm.data_ptr<float>(),
+                                   rgb_w, depth_w, mask));
+    return {Hm, rgb_w, depth_w, mask};
+}
+
 // ---- parameters prepared once per batch and shared by both directions (vidc_frame_params_prepare) ---------------------------------
 std::tuple<at::Tensor, at::Tensor> frame_params(const at::Tensor& I_g, const at::Tensor& I_a, double fx, double fy, double cx, double cy) {
     check_f32_cuda(I_g, "I_g");
@@ -162,6 +198,20 @@ std::tuple<at::Tensor, at::Tensor, at::Tensor> warp_rgbd_prepared(const at::Tens
     check_status(vidc_warp_rgbd(&cam, &ri, &di, nullptr, nullptr, (int32_t)rgb.size(0), (vidc_interp)depth_mode,
                                 reinterpret_cast<vidc_frame_params*>(ws.data_ptr<float>()), nullptr, &rwi, &dwi,
                                 mask.data_ptr<uint8_t>(), nullptr, at::cuda::getCurrentCUDAStream().stream()));
+    return {rgb_w, depth_w, mask};
+}
+std::tuple<at::Tensor, at::Tensor, at::Tensor> warp_rgbd_u8_prepared(const at::Tensor& rgb, const at::Tensor& depth, const at::Tensor& ws,
+                                                                     double fx, double fy, double cx, double cy, int64_t depth_mode) {
+    check_u8_frames(rgb);
+    check_f32_cuda(depth, "x_depth");
+    TORCH_CHECK(depth.dim() == 4, "warp_rgbd_u8: expected (B,1,h,w) depth");
+    TORCH_CHECK(depth.device() == rgb.device(), "x_depth must live on ", rgb.device(), ", got ", depth.device());
+    const vidc_camera cam = make_camera(fx, fy, cx, cy);
+    const c10::cuda::CUDAGuard guard(rgb.device());
+    check_prepared(ws, cam, rgb.size(0), rgb.device());
+    at::Tensor rgb_w = rgb_canvas_u8(rgb, cam.H, cam.W), depth_w = canvas_like(depth, cam);
+    at::Tensor mask = at::empty({rgb.size(0), 1, cam.H, cam.W}, rgb.options());
+    check_status(warp_rgbd_u8_call(cam, rgb, depth, nullptr, nullptr, rgb.size(0), depth_mode, ws, nullptr, rgb_w, depth_w, mask));
     return {rgb_w, depth_w, mask};
 }
 at::Tensor unwarp_normals_prepared(const at::Tensor& x, const at::Tensor& ws, double fx, double fy, double cx, double cy, bool normalize) {
@@ -213,6 +263,17 @@ std::tuple<at::Tensor, at::Tensor, at::Tensor, at::Tensor> warp_rgbd_meta(const 
     return {at::empty({I_g.size(0), 3, 3}, rgb.options()), canvas_like_hw(rgb, H, W), canvas_like_hw(depth, H, W),
             at::empty({rgb.size(0), 1, H, W}, rgb.options().dtype(at::kByte))};
 }
+std::tuple<at::Tensor, at::Tensor, at::Tensor, at::Tensor> warp_rgbd_u8_meta(const at::Tensor& rgb, const at::Tensor& depth, const at::Tensor& I_g,
+                                                                             const at::Tensor&, double, double, double cx, double cy, int64_t) {
+    const int64_t H = canvas_h(cy), W = canvas_w(cx);
+    return {at::empty({I_g.size(0), 3, 3}, depth.options()), rgb_canvas_u8(rgb, H, W), canvas_like_hw(depth, H, W),
+            at::empty({rgb.size(0), 1, H, W}, rgb.options().dtype(at::kByte))};
+}
+std::tuple<at::Tensor, at::Tensor, at::Tensor> warp_rgbd_u8_prepared_meta(const at::Tensor& rgb, const at::Tensor& depth, const at::Tensor&,
+                                                                          double, double, double cx, double cy, int64_t) {
+    const int64_t H = canvas_h(cy), W = canvas_w(cx);
+    return {rgb_canvas_u8(rgb, H, W), canvas_like_hw(depth, H, W), at::empty({rgb.size(0), 1, H, W}, rgb.options().dtype(at::kByte))};
+}
 int64_t workspace_floats_meta(double cx, double cy, int64_t B) {            // as vidc_workspace_bytes: 192 B per frame + 16 B per tile
     const int64_t tiles = ((canvas_w(cx) + 31) / 32) * ((canvas_h(cy) + 31) / 32), n = std::max<int64_t>(B, 1);
     return (n * 192 + n * tiles * 16 + 3) / 4;
@@ -245,6 +306,10 @@ TORCH_LIBRARY(vidc, m) {
     m.def("warp_rgbd_prepared(Tensor rgb, Tensor depth, Tensor params, float fx, float fy, float cx, float cy, int depth_mode) -> "
           "(Tensor, Tensor, Tensor)");
     m.def("unwarp_normals_prepared(Tensor x, Tensor params, float fx, float fy, float cx, float cy, bool normalize) -> Tensor");
+    m.def("warp_rgbd_u8(Tensor rgb, Tensor depth, Tensor I_g, Tensor I_a, float fx, float fy, float cx, float cy, int depth_mode) -> "
+          "(Tensor, Tensor, Tensor, Tensor)");
+    m.def("warp_rgbd_u8_prepared(Tensor rgb, Tensor depth, Tensor params, float fx, float fy, float cx, float cy, int depth_mode) -> "
+          "(Tensor, Tensor, Tensor)");
 }
 TORCH_LIBRARY_IMPL(vidc, CUDA, m) {
     m.impl("warp_forward", &warp_forward);
@@ -254,6 +319,8 @@ TORCH_LIBRARY_IMPL(vidc, CUDA, m) {
     m.impl("frame_params", &frame_params);
     m.impl("warp_rgbd_prepared", &warp_rgbd_prepared);
     m.impl("unwarp_normals_prepared", &unwarp_normals_prepared);
+    m.impl("warp_rgbd_u8", &warp_rgbd_u8);
+    m.impl("warp_rgbd_u8_prepared", &warp_rgbd_u8_prepared);
 }
 TORCH_LIBRARY_IMPL(vidc, Meta, m) {
     m.impl("warp_forward", &warp_forward_meta);
@@ -263,4 +330,6 @@ TORCH_LIBRARY_IMPL(vidc, Meta, m) {
     m.impl("frame_params", &frame_params_meta);
     m.impl("warp_rgbd_prepared", &warp_rgbd_prepared_meta);
     m.impl("unwarp_normals_prepared", &unwarp_normals_prepared_meta);
+    m.impl("warp_rgbd_u8", &warp_rgbd_u8_meta);
+    m.impl("warp_rgbd_u8_prepared", &warp_rgbd_u8_prepared_meta);
 }

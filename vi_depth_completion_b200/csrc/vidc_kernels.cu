@@ -421,6 +421,64 @@ bool try_rgbd_cl(const vidc_camera* cam, const vidc_frame_params* prm, const vid
     return true;                                                   // the caller checks the launch
 }
 
+// (B,H,W,3) uint8 frames seen as (3 W, H, B) bytes with a (3 PF_FWD_BW, PF_FWD_BH, 1) box: the bulk L2 prefetch of
+// warp_rgbd_shear_u8_kernel.  false if the view cannot be described (frames not 16-byte aligned, ...).
+bool encode_u8_frames_map(CUtensorMap* map, const uint8_t* data, int W, int H, int N) {
+    if (((uintptr_t)data & 15) || (3 * W) % 16) return false;
+    const cuuint64_t dims[3] = {(cuuint64_t)3 * W, (cuuint64_t)H, (cuuint64_t)N};
+    const cuuint64_t strides[2] = {(cuuint64_t)3 * W, (cuuint64_t)3 * W * H};
+    const cuuint32_t box[3] = {3 * PF_FWD_BW, PF_FWD_BH, 1};
+    return encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<uint8_t*>(data), dims, strides, box);
+}
+
+// RGB as (B,Hin,Win,3) uint8 (vidc_warp_rgbd_u8; `rgb` describes the bytes with element strides (3 Hin Win, 1, 3 Win, 3)).
+// Frames of the canvas size whose outputs the sheared route accepts take warp_rgbd_shear_u8_kernel, at any byte alignment
+// (the kernel loads bytes); everything else, and VIDC_TMA=1, the generic kernel through the same tap conversion.
+int launch_rgbd_u8(const vidc_camera* cam, const vidc_frame_params* prm, const vidc_image* rgb, const vidc_image* depth, int depth_mode,
+                   const vidc_image* rgb_out, const vidc_image* depth_out, uint8_t* d_mask_u8, uint32_t* d_coverage, cudaStream_t st) {
+    const uint8_t* rgb8 = reinterpret_cast<const uint8_t*>(rgb->data);
+    const bool shear = shear_level() >= 1 && !tma_enabled() && cam->W % 32 == 0 && rgb->h == cam->H && rgb->w == cam->W &&
+                       rgb_out->sw == 1 && aligned16(rgb_out->data) && rgb_out->sn % 4 == 0 &&
+                       (!depth || (depth->sw == 1 && depth_out->sw == 1 && aligned16(depth_out->data) && depth_out->sn % 4 == 0)) &&
+                       (!d_mask_u8 || (reinterpret_cast<uintptr_t>(d_mask_u8) & 3) == 0) &&
+                       contiguous_planes(cam, {rgb_out, depth, depth ? depth_out : nullptr});
+    const dim3 blk(32, 8);
+    if (!shear) {
+        const ImgViewU8 av{rgb8, 3, rgb->h, rgb->w, rgb->sn, (int)rgb->sc, (int)rgb->sh, (int)rgb->sw};
+        ImgView dv{}; ImgViewOut ydv{};
+        if (depth) { dv = view_in(depth); ydv = view_out(depth_out); }
+        with_flags([&](auto has_d) {
+            warp_forward_u8_kernel<has_d><<<grid2d(cam->W, cam->H, rgb->n, blk), blk, 0, st>>>(
+                prm, cam_const(cam), av, view_out(rgb_out), VIDC_BILINEAR, dv, ydv, depth_mode, d_mask_u8, d_coverage);
+        }, depth != nullptr);
+        VIDC_LAUNCH_CHECK();
+        return VIDC_OK;
+    }
+    const dim3 grd((cam->W + TILE_W - 1) / TILE_W, (cam->H + TILE_H - 1) / TILE_H, rgb->n);
+    FwdArgs fa{};
+    fa.prm = prm; fa.cam = cam_const(cam);
+    fa.rgb = rgb->data; fa.rgb_sn = rgb->sn; fa.rgb_sc = 1;                                  // byte address, bytes per frame
+    fa.dep = depth ? depth->data : nullptr; fa.dep_sn = depth ? depth->sn : 0;
+    fa.Hin = rgb->h; fa.Win = rgb->w; fa.in_sh = cam->W;
+    fa.rgb_o = rgb_out->data; fa.rgbo_sn = rgb_out->sn; fa.rgbo_sc = (int)rgb_out->sc; fa.rgbo_sh = (int)rgb_out->sh;
+    fa.dep_o = depth ? depth_out->data : nullptr; fa.depo_sn = depth ? depth_out->sn : 0; fa.depo_sh = depth ? (int)depth_out->sh : 0;
+    fa.mode_d = depth_mode; fa.mask = d_mask_u8; fa.coverage = d_coverage;
+    set_fwd_prefetch(fa, prm, rgb->n, grd);
+    PrefetchMaps pm;
+    fa.pf_bulk = fa.src_boxes && pf_bulk_enabled() && encode_u8_frames_map(&pm.img, rgb8, cam->W, cam->H, rgb->n) &&
+                 (!depth || encode_store_map(&pm.dep, depth->data, cam->W, cam->H, 1, rgb->n, depth->sh, (int64_t)cam->W * cam->H, depth->sn,
+                                             true, PF_FWD_BW, PF_FWD_BH));
+    StoreMaps sm;
+    bool ts = tma_store_enabled() && encode_store_map(&sm.img, rgb_out->data, cam->W, cam->H, 3, rgb->n, rgb_out->sh, rgb_out->sc, rgb_out->sn);
+    if (ts && depth) ts = encode_store_map(&sm.dep, depth_out->data, cam->W, cam->H, 1, rgb->n, depth_out->sh, (int64_t)cam->W * cam->H, depth_out->sn, true);
+    if (ts && d_mask_u8) ts = encode_mask_map(&sm.mask, d_mask_u8, cam->W, cam->H, rgb->n);
+    with_geometry<true>(cam, true, [&](auto gw, auto gh, auto has_d, auto ts_) {
+        warp_rgbd_shear_u8_kernel<gw, gh, has_d, ts_><<<grd, blk, 0, st>>>(fa, sm, pm);
+    }, depth != nullptr, ts);
+    VIDC_LAUNCH_CHECK();
+    return VIDC_OK;
+}
+
 #define VIDC_TRY(expr) do { int rc_ = (expr); if (rc_ != VIDC_OK) return rc_; } while (0)
 
 }  // namespace vidc_k
@@ -546,12 +604,13 @@ __attribute__((visibility("hidden"))) int forward_group(const vidc_camera* cam, 
 }
 
 // zero_depth_out (sparse-depth path, depth == NULL): a (B,1,H,W) plane the call fills with zeros -- by the RGB kernel's own
-// write-out where the sheared kernels run, by a memset otherwise
+// write-out where the sheared kernels run, by a memset otherwise.  rgb_u8: `rgb` describes (B,Hin,Win,3) uint8 frames
+// (vidc_warp_rgbd_u8), which launch_rgbd_u8 warps.
 __attribute__((visibility("hidden"))) int warp_rgbd_impl(const vidc_camera* cam, const vidc_image* rgb, const vidc_image* depth,
                    const float* d_Ig, const float* d_Ia, int32_t B_gravity, vidc_interp depth_mode,
                    vidc_frame_params* d_params_ws, float* d_H_out,
                    const vidc_image* rgb_out, const vidc_image* depth_out,
-                   uint8_t* d_mask_u8, uint32_t* d_coverage, const vidc_image* zero_depth_out, void* stream);
+                   uint8_t* d_mask_u8, uint32_t* d_coverage, const vidc_image* zero_depth_out, void* stream, int rgb_u8);
 
 int vidc_warp_rgbd(const vidc_camera* cam, const vidc_image* rgb, const vidc_image* depth,
                    const float* d_Ig, const float* d_Ia, int32_t B_gravity, vidc_interp depth_mode,
@@ -559,14 +618,28 @@ int vidc_warp_rgbd(const vidc_camera* cam, const vidc_image* rgb, const vidc_ima
                    const vidc_image* rgb_out, const vidc_image* depth_out,
                    uint8_t* d_mask_u8, uint32_t* d_coverage, void* stream) {
     return warp_rgbd_impl(cam, rgb, depth, d_Ig, d_Ia, B_gravity, depth_mode, d_params_ws, d_H_out, rgb_out, depth_out, d_mask_u8,
-                          d_coverage, nullptr, stream);
+                          d_coverage, nullptr, stream, 0);
+}
+
+int vidc_warp_rgbd_u8(const vidc_camera* cam, const uint8_t* d_rgb_hwc, int32_t B, int32_t Hin, int32_t Win,
+                      const vidc_image* depth, const float* d_Ig, const float* d_Ia, int32_t B_gravity,
+                      vidc_interp depth_mode, vidc_frame_params* d_params_ws, float* d_H_out,
+                      const vidc_image* rgb_out, const vidc_image* depth_out,
+                      uint8_t* d_mask_u8, uint32_t* d_coverage, void* stream) {
+    if (B < 0 || Hin < 0 || Win < 0) return fail(VIDC_ERR_INVALID_ARGUMENT, "rgb: bad shape (%d,%d,%d,3)", B, Hin, Win);
+    vidc_image rgb;                                                // the frames' bytes, element strides (3 Hin Win, 1, 3 Win, 3)
+    rgb.data = reinterpret_cast<float*>(const_cast<uint8_t*>(d_rgb_hwc));
+    rgb.n = B; rgb.c = 3; rgb.h = Hin; rgb.w = Win;
+    rgb.sn = 3LL * Hin * Win; rgb.sc = 1; rgb.sh = 3LL * Win; rgb.sw = 3;
+    return warp_rgbd_impl(cam, &rgb, depth, d_Ig, d_Ia, B_gravity, depth_mode, d_params_ws, d_H_out, rgb_out, depth_out, d_mask_u8,
+                          d_coverage, nullptr, stream, 1);
 }
 
 int warp_rgbd_impl(const vidc_camera* cam, const vidc_image* rgb, const vidc_image* depth,
                    const float* d_Ig, const float* d_Ia, int32_t B_gravity, vidc_interp depth_mode,
                    vidc_frame_params* d_params_ws, float* d_H_out,
                    const vidc_image* rgb_out, const vidc_image* depth_out,
-                   uint8_t* d_mask_u8, uint32_t* d_coverage, const vidc_image* zero_depth_out, void* stream) {
+                   uint8_t* d_mask_u8, uint32_t* d_coverage, const vidc_image* zero_depth_out, void* stream, int rgb_u8) {
     VIDC_TRY(check_cam(cam));
     VIDC_TRY(check_image(rgb, "rgb", 3, 3));
     VIDC_TRY(check_image(rgb_out, "rgb_out", 3, 3));
@@ -585,6 +658,7 @@ int warp_rgbd_impl(const vidc_camera* cam, const vidc_image* rgb, const vidc_ima
     cudaStream_t st = (cudaStream_t)stream;
     if (d_coverage) VIDC_CUDA(cudaMemsetAsync(d_coverage, 0, sizeof(uint32_t) * (size_t)rgb->n, st));
     VIDC_TRY(warp_params(cam, d_Ig, d_Ia, rgb->n, d_params_ws, d_H_out, st, /*prepared_ok=*/true, /*tiles=*/true));
+    if (rgb_u8) return launch_rgbd_u8(cam, d_params_ws, rgb, depth, (int)depth_mode, rgb_out, depth_out, d_mask_u8, d_coverage, st);
     if (!zero_depth_out && try_rgbd_cl(cam, d_params_ws, rgb, depth, (int)depth_mode, rgb_out, depth_out, d_mask_u8, d_coverage, st)) {
         VIDC_LAUNCH_CHECK();                                       // channels-last RGB (kernels_shear_cl.cuh)
         return VIDC_OK;
@@ -1301,7 +1375,7 @@ int vidc_warp_rgb_sparse_depth(const vidc_camera* cam, const vidc_image* rgb, co
         return fail(VIDC_ERR_INVALID_ARGUMENT, "depth_out must be (%d,1,%d,%d) with contiguous rows", rgb->n, cam->H, cam->W);
     if (N > 0 && !d_tracks) return fail(VIDC_ERR_INVALID_ARGUMENT, "null tracks pointer");
     VIDC_TRY(warp_rgbd_impl(cam, rgb, nullptr, d_Ig, d_Ia, B_gravity, VIDC_BILINEAR, d_params_ws, d_H_out, rgb_out, nullptr, d_mask_u8,
-                            d_coverage, depth_out, stream));
+                            d_coverage, depth_out, stream, 0));
     if (rgb->n == 0 || N == 0) return VIDC_OK;
     SparseArgs sa;
     sa.prm = d_params_ws; sa.cam = cam_const(cam); sa.tracks = d_tracks; sa.counts = d_counts; sa.N = N; sa.cols = cols;

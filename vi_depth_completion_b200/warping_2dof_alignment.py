@@ -595,6 +595,73 @@ class Warping2DOFAlignment:
         out = _no_gravity_grad(out, I_g, I_a)
         return out + (cov,) if with_coverage else out
 
+    def warp_rgbd_u8(self, rgb_u8, x_depth, I_g=None, I_a=None, depth_mode='bilinear', with_mask=True, with_coverage=False, params=None):
+        """warp_rgbd on the frames as the loader decodes them: rgb_u8 is (B,h,w,3) uint8 on the device (dataset.py:468-471,
+        before ToTensor).  Same arguments, return tuple and bits as warp_rgbd(to_tensor_u8(rgb_u8), ...); RGB comes out as
+        contiguous (B,3,H,W) float32.  The kernel converts each tap itself, so the float copy of the frames is never made."""
+        _check_interp_mode(depth_mode)
+        if not isinstance(rgb_u8, torch.Tensor) or not rgb_u8.is_cuda or rgb_u8.dtype != torch.uint8 or rgb_u8.dim() != 4:
+            raise RuntimeError("rgb_u8: expected a (B,H,W,3) uint8 CUDA tensor")
+        if rgb_u8.shape[3] != 3:
+            raise RuntimeError(f"rgb_u8: 3 channels, got {rgb_u8.shape[3]}")
+        x = rgb_u8.contiguous()
+        device = x.device
+        mode = _cabi.VIDC_BILINEAR if depth_mode == "bilinear" else _cabi.VIDC_NEAREST
+        ops = _torchops.ops()
+        d4 = None
+        if x_depth is not None:
+            _require_cuda_f32(x_depth, "x_depth")
+            d4 = x_depth.view(x_depth.shape[0], 1, x_depth.shape[1], x_depth.shape[2]) if x_depth.dim() == 3 else x_depth
+        if params is not None:
+            if d4 is None or not with_mask or with_coverage:
+                raise RuntimeError("warp_rgbd_u8(params=...): depth, mask on, no coverage")
+            p = self._prepared(params, x, "rgb_u8")
+            g = a = None
+            grav = p.grav
+        else:
+            if I_g is None or I_a is None:
+                raise RuntimeError("warp_rgbd_u8: pass I_g and I_a, or params=prepare(I_g, I_a)")
+            grav = (I_g, I_a)
+        torch_op = ops is not None and d4 is not None and with_mask and not with_coverage and (
+            params is not None or (isinstance(I_g, torch.Tensor) and isinstance(I_a, torch.Tensor)))
+        cov = None
+        if torch_op:
+            if params is not None:
+                rgb_w, depth_w, mask = _op(ops.warp_rgbd_u8_prepared, x, _nd(d4), p.ws, *self._intr, mode)
+                Cg_H_C = p.H
+            else:
+                Cg_H_C, rgb_w, depth_w, mask = _op(ops.warp_rgbd_u8, x, _nd(d4), _nd(I_g), _nd(I_a), *self._intr, mode)
+        else:
+            if params is None:
+                g, a = _gravity(I_g, I_a, device)
+                ws, B_g, Cg_H_C = self._params_ws(g.shape[0], device), g.shape[0], torch.empty((g.shape[0], 3, 3), dtype=torch.float32, device=device)
+            else:
+                ws, B_g, Cg_H_C = p.ws, p.B, p.H
+            B = x.shape[0]
+            di = dwi = depth_w = None
+            if d4 is not None:
+                if d4.device != device:
+                    raise RuntimeError(f"x_depth must live on {device}, got {d4.device}")
+                depth_w = self._empty_like_canvas(d4)
+                di, dwi = _image(d4), _image(depth_w)
+            rgb_w = torch.empty((B, 3, int(self.H), int(self.W)), dtype=torch.float32, device=device)
+            mask = torch.empty((B, 1, int(self.H), int(self.W)), dtype=torch.uint8, device=device) if with_mask else None
+            cov = torch.empty((B,), dtype=torch.int32, device=device) if with_coverage else None
+            rwi = _image(rgb_w)
+            with torch.cuda.device(device):
+                check(lib().vidc_warp_rgbd_u8(ctypes.byref(self._cam), x.data_ptr(), B, x.shape[1], x.shape[2],
+                                              ctypes.byref(di) if di is not None else None, g.data_ptr() if g is not None else None,
+                                              a.data_ptr() if a is not None else None, B_g, mode, ws.data_ptr(),
+                                              Cg_H_C.data_ptr() if params is None else None, ctypes.byref(rwi),
+                                              ctypes.byref(dwi) if dwi is not None else None, mask.data_ptr() if with_mask else None,
+                                              cov.data_ptr() if with_coverage else None, _stream_ptr(device)))
+        if depth_w is not None:
+            if x_depth.dim() == 3:
+                depth_w = depth_w.view(depth_w.shape[0], depth_w.shape[2], depth_w.shape[3])
+            depth_w = _attach(x_depth, depth_w)                                                  # forward-only
+        out = _no_gravity_grad((Cg_H_C, rgb_w, depth_w, mask), *grav)
+        return out + (cov,) if with_coverage else out
+
     def warp_rgb_sparse_depth(self, x_rgb, tracks, counts, fc, cc, I_g, I_a, depth_mode='bilinear', with_mask=True, with_coverage=False):
         """SURVEY row f2: warp RGB (B,3,H,W) and the SPARSE depth given as KLT tracks (B,N,>=4) float64 [id, x, y, z, ...] (valid
         rows per frame in `counts`, loader intrinsics fc, cc: dataset.py:496-510) without building the depth image: the points
