@@ -61,35 +61,13 @@ __device__ __forceinline__ void unwarp_normals_cl_segments(const InvArgs& a, con
     const int W = GW ? GW : a.cam.W, H = GW ? GH : a.cam.H;
     const int b = blockIdx.z, lane = threadIdx.x, warp = threadIdx.y;
     const int tileX0 = blockIdx.x * TILE_W, tileY0 = blockIdx.y * TILE_H;
-    const float* Hm = pr;
     const float* R = pr + 9;
-    const float px_min = pr[27], py_min = pr[28], kw = pr[29], kh = pr[30];
-    const float Wf = (float)W, Hf = (float)H;
     const float* __restrict__ in = a.x + (long long)b * a.x_sn;
-    const float c_fix = ALONG_Y ? (float)(tileY0 + lane) : (float)(tileX0 + lane);
-    const float u0 = Hm[0] * c_fix, v0 = Hm[3] * c_fix, s0 = Hm[6] * c_fix;        // used when the fixed one is X
+    const InvShearChain<ALONG_Y> chain(pr, W, H, tileX0, tileY0, lane);
 #pragma unroll
     for (int j = 0; j < ROWS_PER_THREAD; ++j) {
         const int S = (VIDC_SEG(warp, j) + sh_l) & 31;
-        float u, v, s;
-        if (ALONG_Y) {
-            const float Xf = (float)(tileX0 + S);
-            s = fmaf(Hm[7], c_fix, Hm[6] * Xf) + Hm[8];
-            u = fmaf(Hm[1], c_fix, Hm[0] * Xf) + Hm[2];
-            v = fmaf(Hm[4], c_fix, Hm[3] * Xf) + Hm[5];
-        } else {
-            const float Yf = (float)(tileY0 + S);
-            s = fmaf(Hm[7], Yf, s0) + Hm[8];
-            u = fmaf(Hm[1], Yf, u0) + Hm[2];
-            v = fmaf(Hm[4], Yf, v0) + Hm[5];
-        }
-        float tx, ty;
-        div2_sel(u, v, s, proven, tx, ty);                         // :245
-        const float cxp = kw * (tx - px_min);
-        const float cyp = kh * (ty - py_min);
-        const float gx = a.cam.inv_half_w * (cxp - a.cam.cx);
-        const float gy = a.cam.inv_half_h * (cyp - a.cam.cy);
-        const Pos t = make_pos(unnormalize(gx, Wf), unnormalize(gy, Hf), H, W);
+        const Pos t = chain.at(S, proven, a.cam);
         const Px3 y = cl_sample(in, 3 * W, H, W, t);
         float z0 = fmaf(R[6], y.c, fmaf(R[3], y.b, fmaf(R[0], y.a, 0.0f)));    // :253
         float z1 = fmaf(R[7], y.c, fmaf(R[4], y.b, fmaf(R[1], y.a, 0.0f)));
@@ -111,13 +89,7 @@ unwarp_normals_shear_cl_kernel(const __grid_constant__ InvArgs a, const __grid_c
     float pr[32];
     load_params(a.prm + b, pr, 0, 8);
     int sh_l;
-    bool along_y;
-    {
-        const float* Hm = pr;
-        const float xc = (float)(tileX0 + TILE_W / 2), yc = (float)(tileY0 + TILE_H / 2);
-        const float vc = fmaf(Hm[4], yc, Hm[3] * xc) + Hm[5], sc = fmaf(Hm[7], yc, Hm[6] * xc) + Hm[8];
-        along_y = shear_of_tile(Hm[3] * sc - vc * Hm[6], Hm[4] * sc - vc * Hm[7], lane, sh_l);
-    }
+    const bool along_y = inv_shear_of_tile(pr, tileX0, tileY0, lane, sh_l);
     const bool proven = __ldg(&a.prm[b].reserved[10]) != 0.0f;     // CTA-uniform (vidc::inv_division_proven)
     if (along_y) unwarp_normals_cl_segments<GW, GH, NORMALIZE, true>(a, pr, tile, sh_l, proven);
     else unwarp_normals_cl_segments<GW, GH, NORMALIZE, false>(a, pr, tile, sh_l, proven);
@@ -136,35 +108,15 @@ __device__ __forceinline__ unsigned int warp_rgbd_cl_segments(const FwdArgs& a, 
     const int W = GW ? GW : a.cam.W, H = GW ? GH : a.cam.H;
     const int b = blockIdx.z, lane = threadIdx.x, warp = threadIdx.y;
     const int tileX0 = blockIdx.x * TILE_W, tileY0 = blockIdx.y * TILE_H;
-    const float* Hi = pr + 2;
-    const float px_min = pr[11], py_min = pr[12], ikw = pr[15], ikh = pr[16];
-    const float Wf = (float)W, Hf = (float)H;
     const float* __restrict__ in_rgb = a.rgb + (long long)b * a.rgb_sn;
     const float* __restrict__ in_dep = HAS_D ? a.dep + (long long)b * a.dep_sn : nullptr;
-    const float p_fix = ALONG_Y ? ikh * (float)(tileY0 + lane) + py_min : ikw * (float)(tileX0 + lane) + px_min;
-    const float u0 = Hi[0] * p_fix, v0 = Hi[3] * p_fix, s0 = Hi[6] * p_fix;        // used when the fixed one is X
+    const FwdShearChain<ALONG_Y> chain(pr, W, H, tileX0, tileY0, lane);
     unsigned int cnt = 0;
 #pragma unroll
     for (int j = 0; j < ROWS_PER_THREAD; ++j) {
         const int S = (VIDC_SEG(warp, j) + sh_l) & 31;
-        float u, v, s;
-        if (ALONG_Y) {
-            const float px = ikw * (float)(tileX0 + S) + px_min;
-            u = fmaf(Hi[1], p_fix, Hi[0] * px) + Hi[2];
-            v = fmaf(Hi[4], p_fix, Hi[3] * px) + Hi[5];
-            s = fmaf(Hi[7], p_fix, Hi[6] * px) + Hi[8];
-        } else {
-            const float py = ikh * (float)(tileY0 + S) + py_min;
-            u = fmaf(Hi[1], py, u0) + Hi[2];
-            v = fmaf(Hi[4], py, v0) + Hi[5];
-            s = fmaf(Hi[7], py, s0) + Hi[8];
-        }
-        float sx, sy;
-        div2_rn(u, v, s, sx, sy);                                  // :146-147
-        const float gx = a.cam.inv_half_w * (sx - a.cam.cx);
-        const float gy = a.cam.inv_half_h * (sy - a.cam.cy);
-        const float ix = unnormalize(gx, Wf), iy = unnormalize(gy, Hf);
-        Pos t = make_pos(ix, iy, H, W);
+        float ix, iy;
+        const Pos t = chain.at(S, a.cam, ix, iy);
         Px3 o = {0.0f, 0.0f, 0.0f};
         float od = 0.0f;
         if (__any_sync(0xffffffffu, t.touch)) {                    // exterior segments: zeros
@@ -201,14 +153,7 @@ warp_rgbd_shear_cl_kernel(const __grid_constant__ FwdArgs a, const __grid_consta
     float pr[20];
     load_params(a.prm + b, pr, 4, 5);
     int sh_l;
-    bool along_y;
-    {
-        const float* Hi = pr + 2;
-        const float ikw = pr[15], ikh = pr[16];
-        const float pxc = ikw * (float)(tileX0 + TILE_W / 2) + pr[11], pyc = ikh * (float)(tileY0 + TILE_H / 2) + pr[12];
-        const float vc = fmaf(Hi[4], pyc, Hi[3] * pxc) + Hi[5], sc = fmaf(Hi[7], pyc, Hi[6] * pxc) + Hi[8];
-        along_y = shear_of_tile(ikw * (Hi[3] * sc - vc * Hi[6]), ikh * (Hi[4] * sc - vc * Hi[7]), lane, sh_l);
-    }
+    const bool along_y = fwd_shear_of_tile(pr, tileX0, tileY0, lane, sh_l);
     // (the exterior-tile bitmap is not consulted here: exterior segments already cost one vote and three zero deposits)
     unsigned int cnt = along_y ? warp_rgbd_cl_segments<GW, GH, HAS_D, true>(a, pr, tile, dtile, mtile, sh_l)
                                : warp_rgbd_cl_segments<GW, GH, HAS_D, false>(a, pr, tile, dtile, mtile, sh_l);

@@ -387,6 +387,44 @@ bool encode_mask_map(CUtensorMap* map, uint8_t* data, int W, int H, int N) {    
     if (strides[1] & 15) return false;
     return encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, data, dims, strides, box);
 }
+// (B,H,W,3) uint8 frames seen as (3 W, H, B) bytes with a (3 PF_FWD_BW, PF_FWD_BH, 1) box: the bulk L2 prefetch of
+// warp_rgbd_shear_u8_kernel.  false if the view cannot be described (frames not 16-byte aligned, ...).
+bool encode_u8_frames_map(CUtensorMap* map, const uint8_t* data, int W, int H, int N) {
+    if (((uintptr_t)data & 15) || (3 * W) % 16) return false;
+    const cuuint64_t dims[3] = {(cuuint64_t)3 * W, (cuuint64_t)H, (cuuint64_t)N};
+    const cuuint64_t strides[2] = {(cuuint64_t)3 * W, (cuuint64_t)3 * W * H};
+    const cuuint32_t box[3] = {3 * PF_FWD_BW, PF_FWD_BH, 1};
+    return encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<uint8_t*>(data), dims, strides, box);
+}
+// Input maps of the forward bulk L2 prefetch (PrefetchMaps): RGB planes (u8: uint8 frames), depth; false: per-thread prefetch
+bool encode_fwd_prefetch(PrefetchMaps* pm, const vidc_camera* cam, const vidc_image* rgb, const vidc_image* depth, bool u8) {
+    const bool img = u8 ? encode_u8_frames_map(&pm->img, reinterpret_cast<const uint8_t*>(rgb->data), cam->W, cam->H, rgb->n)
+                        : encode_store_map(&pm->img, rgb->data, cam->W, cam->H, 3, rgb->n, rgb->sh, rgb->sc, rgb->sn, false, PF_FWD_BW, PF_FWD_BH);
+    return img && (!depth || encode_store_map(&pm->dep, depth->data, cam->W, cam->H, 1, rgb->n, depth->sh, (int64_t)cam->W * cam->H,
+                                              depth->sn, true, PF_FWD_BW, PF_FWD_BH));
+}
+// Output maps of the forward TMA write-out (StoreMaps): RGB, `dep_out` (depth, or the sparse-depth route's zero plane) and mask
+// when given.  true (TMA write-out) when VIDC_TMA_STORE is on and a map describes every output; false: the LSU write-out.
+bool encode_fwd_store(StoreMaps* sm, const vidc_camera* cam, int N, const vidc_image* rgb_out, const vidc_image* dep_out, uint8_t* mask) {
+    bool ts = tma_store_enabled() && encode_store_map(&sm->img, rgb_out->data, cam->W, cam->H, 3, N, rgb_out->sh, rgb_out->sc, rgb_out->sn);
+    if (ts && dep_out) ts = encode_store_map(&sm->dep, dep_out->data, cam->W, cam->H, 1, N, dep_out->sh, (int64_t)cam->W * cam->H, dep_out->sn, true);
+    if (ts && mask) ts = encode_mask_map(&sm->mask, mask, cam->W, cam->H, N);
+    return ts;
+}
+
+// Forward RGB-D kernel arguments without the L2 prefetch (set_fwd_prefetch).  uint8 frames: the rgb fields count bytes.
+FwdArgs fwd_args(const vidc_camera* cam, const vidc_frame_params* prm, const vidc_image* rgb, const vidc_image* depth,
+                 const vidc_image* rgb_out, const vidc_image* depth_out, uint8_t* mask, uint32_t* coverage, int mode_d) {
+    FwdArgs fa{};
+    fa.prm = prm; fa.cam = cam_const(cam);
+    fa.rgb = rgb->data; fa.rgb_sn = rgb->sn; fa.rgb_sc = (int)rgb->sc;
+    fa.dep = depth ? depth->data : nullptr; fa.dep_sn = depth ? depth->sn : 0;
+    fa.Hin = rgb->h; fa.Win = rgb->w; fa.in_sh = (int)rgb->sh;
+    fa.rgb_o = rgb_out->data; fa.rgbo_sn = rgb_out->sn; fa.rgbo_sc = (int)rgb_out->sc; fa.rgbo_sh = (int)rgb_out->sh;
+    fa.dep_o = depth ? depth_out->data : nullptr; fa.depo_sn = depth ? depth_out->sn : 0; fa.depo_sh = depth ? (int)depth_out->sh : 0;
+    fa.mode_d = mode_d; fa.mask = mask; fa.coverage = coverage;
+    return fa;
+}
 
 template <typename K>
 void prefer_shared_carveout(K kernel) {          // per device: function attributes belong to the device's context
@@ -410,25 +448,12 @@ bool try_rgbd_cl(const vidc_camera* cam, const vidc_frame_params* prm, const vid
     if (!encode_cl_map(&sm.img, rgb_out->data, cam->W, cam->H, rgb->n)) return false;
     if (depth && !encode_store_map(&sm.dep, depth_out->data, cam->W, cam->H, 1, rgb->n, depth_out->sh, (int64_t)cam->W * cam->H, depth_out->sn, true)) return false;
     if (d_mask_u8 && !encode_mask_map(&sm.mask, d_mask_u8, cam->W, cam->H, rgb->n)) return false;
-    FwdArgs fa{};
-    fa.prm = prm; fa.cam = cam_const(cam);
-    fa.rgb = rgb->data; fa.rgb_sn = rgb->sn; fa.dep = depth ? depth->data : nullptr; fa.dep_sn = depth ? depth->sn : 0;
-    fa.Hin = cam->H; fa.Win = cam->W; fa.mode_d = depth_mode; fa.mask = d_mask_u8; fa.coverage = d_coverage;
+    const FwdArgs fa = fwd_args(cam, prm, rgb, depth, rgb_out, depth_out, d_mask_u8, d_coverage, depth_mode);
     const dim3 blk(32, 8), grd((cam->W + TILE_W - 1) / TILE_W, (cam->H + TILE_H - 1) / TILE_H, rgb->n);
     with_geometry<false>(cam, true, [&](auto gw, auto gh, auto has_d) {
         warp_rgbd_shear_cl_kernel<gw, gh, has_d><<<grd, blk, 0, st>>>(fa, sm);
     }, depth != nullptr);
     return true;                                                   // the caller checks the launch
-}
-
-// (B,H,W,3) uint8 frames seen as (3 W, H, B) bytes with a (3 PF_FWD_BW, PF_FWD_BH, 1) box: the bulk L2 prefetch of
-// warp_rgbd_shear_u8_kernel.  false if the view cannot be described (frames not 16-byte aligned, ...).
-bool encode_u8_frames_map(CUtensorMap* map, const uint8_t* data, int W, int H, int N) {
-    if (((uintptr_t)data & 15) || (3 * W) % 16) return false;
-    const cuuint64_t dims[3] = {(cuuint64_t)3 * W, (cuuint64_t)H, (cuuint64_t)N};
-    const cuuint64_t strides[2] = {(cuuint64_t)3 * W, (cuuint64_t)3 * W * H};
-    const cuuint32_t box[3] = {3 * PF_FWD_BW, PF_FWD_BH, 1};
-    return encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<uint8_t*>(data), dims, strides, box);
 }
 
 // RGB as (B,Hin,Win,3) uint8 (vidc_warp_rgbd_u8; `rgb` describes the bytes with element strides (3 Hin Win, 1, 3 Win, 3)).
@@ -455,23 +480,12 @@ int launch_rgbd_u8(const vidc_camera* cam, const vidc_frame_params* prm, const v
         return VIDC_OK;
     }
     const dim3 grd((cam->W + TILE_W - 1) / TILE_W, (cam->H + TILE_H - 1) / TILE_H, rgb->n);
-    FwdArgs fa{};
-    fa.prm = prm; fa.cam = cam_const(cam);
-    fa.rgb = rgb->data; fa.rgb_sn = rgb->sn; fa.rgb_sc = 1;                                  // byte address, bytes per frame
-    fa.dep = depth ? depth->data : nullptr; fa.dep_sn = depth ? depth->sn : 0;
-    fa.Hin = rgb->h; fa.Win = rgb->w; fa.in_sh = cam->W;
-    fa.rgb_o = rgb_out->data; fa.rgbo_sn = rgb_out->sn; fa.rgbo_sc = (int)rgb_out->sc; fa.rgbo_sh = (int)rgb_out->sh;
-    fa.dep_o = depth ? depth_out->data : nullptr; fa.depo_sn = depth ? depth_out->sn : 0; fa.depo_sh = depth ? (int)depth_out->sh : 0;
-    fa.mode_d = depth_mode; fa.mask = d_mask_u8; fa.coverage = d_coverage;
+    FwdArgs fa = fwd_args(cam, prm, rgb, depth, rgb_out, depth_out, d_mask_u8, d_coverage, depth_mode);
     set_fwd_prefetch(fa, prm, rgb->n, grd);
     PrefetchMaps pm;
-    fa.pf_bulk = fa.src_boxes && pf_bulk_enabled() && encode_u8_frames_map(&pm.img, rgb8, cam->W, cam->H, rgb->n) &&
-                 (!depth || encode_store_map(&pm.dep, depth->data, cam->W, cam->H, 1, rgb->n, depth->sh, (int64_t)cam->W * cam->H, depth->sn,
-                                             true, PF_FWD_BW, PF_FWD_BH));
+    fa.pf_bulk = fa.src_boxes && pf_bulk_enabled() && encode_fwd_prefetch(&pm, cam, rgb, depth, true);
     StoreMaps sm;
-    bool ts = tma_store_enabled() && encode_store_map(&sm.img, rgb_out->data, cam->W, cam->H, 3, rgb->n, rgb_out->sh, rgb_out->sc, rgb_out->sn);
-    if (ts && depth) ts = encode_store_map(&sm.dep, depth_out->data, cam->W, cam->H, 1, rgb->n, depth_out->sh, (int64_t)cam->W * cam->H, depth_out->sn, true);
-    if (ts && d_mask_u8) ts = encode_mask_map(&sm.mask, d_mask_u8, cam->W, cam->H, rgb->n);
+    const bool ts = encode_fwd_store(&sm, cam, rgb->n, rgb_out, depth ? depth_out : nullptr, d_mask_u8);
     with_geometry<true>(cam, true, [&](auto gw, auto gh, auto has_d, auto ts_) {
         warp_rgbd_shear_u8_kernel<gw, gh, has_d, ts_><<<grd, blk, 0, st>>>(fa, sm, pm);
     }, depth != nullptr, ts);
@@ -589,8 +603,7 @@ __attribute__((visibility("hidden"))) int forward_group(const vidc_camera* cam, 
         pa.x = x->data; pa.x_sn = x->sn; pa.y = y->data; pa.y_sn = y->sn; pa.mode = (int)mode;
         set_fwd_prefetch(pa, d_params_ws, x->n, grd);
         PrefetchMaps pm;
-        pa.pf_bulk = pa.src_boxes && x->c == 3 && pf_bulk_enabled() &&
-                     encode_store_map(&pm.img, x->data, cam->W, cam->H, 3, x->n, x->sh, x->sc, x->sn, false, PF_FWD_BW, PF_FWD_BH);
+        pa.pf_bulk = pa.src_boxes && x->c == 3 && pf_bulk_enabled() && encode_fwd_prefetch(&pm, cam, x, nullptr, false);
         StoreMaps sm;
         const bool ts = tma_store_enabled() &&
                         encode_store_map(&sm.img, y->data, cam->W, cam->H, x->c, x->n, y->sh, x->c == 1 ? (int64_t)cam->W * cam->H : y->sc, y->sn);
@@ -675,14 +688,7 @@ int warp_rgbd_impl(const vidc_camera* cam, const vidc_image* rgb, const vidc_ima
                                                d_coverage, st);
     }
     const dim3 blk(32, 8), grd((cam->W + TILE_W - 1) / TILE_W, (cam->H + TILE_H - 1) / TILE_H, rgb->n);
-    FwdArgs fa;
-    fa.prm = d_params_ws; fa.cam = cam_const(cam);
-    fa.rgb = rgb->data; fa.rgb_sn = rgb->sn; fa.rgb_sc = (int)rgb->sc;
-    fa.dep = depth ? depth->data : nullptr; fa.dep_sn = depth ? depth->sn : 0;
-    fa.Hin = rgb->h; fa.Win = rgb->w; fa.in_sh = (int)rgb->sh;
-    fa.rgb_o = rgb_out->data; fa.rgbo_sn = rgb_out->sn; fa.rgbo_sc = (int)rgb_out->sc; fa.rgbo_sh = (int)rgb_out->sh;
-    fa.dep_o = depth ? depth_out->data : nullptr; fa.depo_sn = depth ? depth_out->sn : 0; fa.depo_sh = depth ? (int)depth_out->sh : 0;
-    fa.mode_d = (int)depth_mode; fa.mask = d_mask_u8; fa.coverage = d_coverage;
+    FwdArgs fa = fwd_args(cam, d_params_ws, rgb, depth, rgb_out, depth_out, d_mask_u8, d_coverage, (int)depth_mode);
     set_fwd_prefetch(fa, d_params_ws, rgb->n, grd);
     if (tma_enabled()) {                                           // TMA-staged variant: footprint boxes through shared memory
         TmaMaps maps;
@@ -721,17 +727,10 @@ int warp_rgbd_impl(const vidc_camera* cam, const vidc_image* rgb, const vidc_ima
         VIDC_LAUNCH_CHECK();
         return VIDC_OK;
     }
-    PrefetchMaps pm;                                               // input maps of the bulk prefetch; else the per-thread form
-    fa.pf_bulk = fa.src_boxes && pf_bulk_enabled() &&
-                 encode_store_map(&pm.img, rgb->data, cam->W, cam->H, 3, rgb->n, rgb->sh, rgb->sc, rgb->sn, false, PF_FWD_BW, PF_FWD_BH) &&
-                 (!depth || encode_store_map(&pm.dep, depth->data, cam->W, cam->H, 1, rgb->n, depth->sh, (int64_t)cam->W * cam->H, depth->sn,
-                                             true, PF_FWD_BW, PF_FWD_BH));
-    StoreMaps sm;
-    bool ts = tma_store_enabled() && encode_store_map(&sm.img, rgb_out->data, cam->W, cam->H, 3, rgb->n, rgb_out->sh, rgb_out->sc, rgb_out->sn);
-    if (ts && depth) ts = encode_store_map(&sm.dep, depth_out->data, cam->W, cam->H, 1, rgb->n, depth_out->sh, (int64_t)cam->W * cam->H, depth_out->sn, true);
-    if (ts && zero_depth_out)                                      // sparse-depth route: the zero plane leaves through the same store
-        ts = encode_store_map(&sm.dep, zero_depth_out->data, cam->W, cam->H, 1, rgb->n, zero_depth_out->sh, (int64_t)cam->W * cam->H, zero_depth_out->sn, true);
-    if (ts && d_mask_u8) ts = encode_mask_map(&sm.mask, d_mask_u8, cam->W, cam->H, rgb->n);
+    PrefetchMaps pm;
+    fa.pf_bulk = fa.src_boxes && pf_bulk_enabled() && encode_fwd_prefetch(&pm, cam, rgb, depth, false);
+    StoreMaps sm;                                                  // sparse-depth route: the zero plane leaves through the depth store
+    const bool ts = encode_fwd_store(&sm, cam, rgb->n, rgb_out, depth ? depth_out : zero_depth_out, d_mask_u8);
     with_geometry<true>(cam, true, [&](auto gw, auto gh, auto has_d, auto ts_) {
         warp_rgbd_shear_kernel<gw, gh, has_d, ts_><<<grd, blk, 0, st>>>(fa, sm, pm);
     }, depth != nullptr, ts);
