@@ -84,27 +84,53 @@ def test_product_never_imports_the_oracle():
 
 
 def test_torch_extension_builds_and_registers_its_operators():
-    """The thin torch C++ extension in front of the C ABI (csrc/torch_ops.cpp): loads on a CPU-only box, registers the four
-    operators with CUDA and Meta kernels; shapes come out of the Meta kernels without a GPU."""
+    """The thin torch C++ extension in front of the C ABI (csrc/torch_ops.cpp): loads on a CPU-only box, registers the
+    operators with CUDA and Meta kernels; shapes come out of the Meta kernels without a GPU, with the canvas of vidc_camera_init
+    and the workspace of vidc_workspace_bytes (at least one frame, as the CUDA kernels allocate it)."""
     import torch
-    from vi_depth_completion_b200 import build as vb
+    from vi_depth_completion_b200 import _cabi, build as vb
     torch.ops.load_library(vb.build_torch_ops())
-    x = torch.empty(2, 3, 240, 320, device="meta")
-    g = torch.empty(2, 3, device="meta")
-    H, y = torch.ops.vidc.warp_forward(x, g, g, 202., 202., 159.93827, 119.938015, 0)
-    assert H.shape == (2, 3, 3) and y.shape == (2, 3, 240, 320)
-    H, z = torch.ops.vidc.unwarp_normals(x, g, g, 404., 404., 319.87654, 239.87603, True)
-    assert z.shape == (2, 3, 480, 640)
-    outs = torch.ops.vidc.warp_rgbd(x, x[:, :1], g, g, 202., 202., 159.93827, 119.938015, 1)
-    assert [tuple(o.shape) for o in outs] == [(2, 3, 3), (2, 3, 240, 320), (2, 1, 240, 320), (2, 1, 240, 320)] and outs[3].dtype == torch.uint8
-    assert len(torch.ops.vidc.build_homography(g, g, 202., 202., 159.93827, 119.938015)) == 3
-    # parameters prepared once per batch: the Meta workspace has the size the library asks for
-    import ctypes
-    from vi_depth_completion_b200 import _cabi
-    cam = _cabi.VidcCamera()
-    _cabi.lib().vidc_camera_init(202., 202., 159.93827, 119.938015, ctypes.byref(cam))
-    ws, H = torch.ops.vidc.frame_params(g, g, 202., 202., 159.93827, 119.938015)
-    assert ws.numel() * 4 == _cabi.lib().vidc_workspace_bytes(ctypes.byref(cam), 2) and H.shape == (2, 3, 3)
-    outs = torch.ops.vidc.warp_rgbd_prepared(x, x[:, :1], ws, 202., 202., 159.93827, 119.938015, 0)
-    assert [tuple(o.shape) for o in outs] == [(2, 3, 240, 320), (2, 1, 240, 320), (2, 1, 240, 320)]
-    assert torch.ops.vidc.unwarp_normals_prepared(x, ws, 202., 202., 159.93827, 119.938015, True).shape == (2, 3, 240, 320)
+    lib = _cabi.lib()
+    # 320x240, 640x480 and 300x201 (a width that is not a multiple of the 32-pixel tile, an odd height)
+    for intr in ((202., 202., 159.93827, 119.938015), (404., 404., 319.87654, 239.87603), (190., 190., 150., 100.5)):
+        cam = _cabi.VidcCamera()
+        assert lib.vidc_camera_init(*intr, ctypes.byref(cam)) == _cabi.VIDC_OK
+        Hc, Wc = cam.H, cam.W
+        for B in (0, 1, 5):
+            x = torch.empty(B, 3, 200, 300, device="meta")
+            g = torch.empty(B, 3, device="meta")
+            H, y = torch.ops.vidc.warp_forward(x, g, g, *intr, 0)
+            assert H.shape == (B, 3, 3) and y.shape == (B, 3, Hc, Wc)
+            H, z = torch.ops.vidc.unwarp_normals(x, g, g, *intr, True)
+            assert H.shape == (B, 3, 3) and z.shape == (B, 3, Hc, Wc)
+            outs = torch.ops.vidc.warp_rgbd(x, x[:, :1], g, g, *intr, 1)
+            assert [tuple(o.shape) for o in outs] == [(B, 3, 3), (B, 3, Hc, Wc), (B, 1, Hc, Wc), (B, 1, Hc, Wc)]
+            assert outs[3].dtype == torch.uint8
+            assert [tuple(m.shape) for m in torch.ops.vidc.build_homography(g, g, *intr)] == [(B, 3, 3)] * 3
+            # parameters prepared once per batch: the Meta workspace has the size the library asks for
+            ws, H = torch.ops.vidc.frame_params(g, g, *intr)
+            assert ws.numel() * 4 == lib.vidc_workspace_bytes(ctypes.byref(cam), max(B, 1)) and H.shape == (B, 3, 3)
+            outs = torch.ops.vidc.warp_rgbd_prepared(x, x[:, :1], ws, *intr, 0)
+            assert [tuple(o.shape) for o in outs] == [(B, 3, Hc, Wc), (B, 1, Hc, Wc), (B, 1, Hc, Wc)]
+            assert torch.ops.vidc.unwarp_normals_prepared(x, ws, *intr, True).shape == (B, 3, Hc, Wc)
+    # intrinsics vidc_camera_init rejects are rejected by the Meta kernels too, as by the CUDA kernels
+    x, g = torch.empty(2, 3, 240, 320, device="meta"), torch.empty(2, 3, device="meta")
+    bad = (202., 202., 0., 119.938015)
+    calls = (lambda: torch.ops.vidc.warp_forward(x, g, g, *bad, 0), lambda: torch.ops.vidc.unwarp_normals(x, g, g, *bad, True),
+             lambda: torch.ops.vidc.warp_rgbd(x, x[:, :1], g, g, *bad, 0), lambda: torch.ops.vidc.build_homography(g, g, *bad),
+             lambda: torch.ops.vidc.frame_params(g, g, *bad))
+    for call in calls:
+        with pytest.raises(RuntimeError, match="intrinsics"):
+            call()
+
+
+def test_torch_extension_is_required(monkeypatch, tmp_path):
+    """The hot entry points have no second route: a missing or unloadable _vidc_torch_ops.so raises and names the fix."""
+    from vi_depth_completion_b200 import _torchops
+    monkeypatch.setattr(_torchops, "_ops", None)
+    monkeypatch.setattr(_torchops, "LIB_PATH", str(tmp_path / "_vidc_torch_ops.so"))
+    with pytest.raises(RuntimeError, match=r"python -m vi_depth_completion_b200\.build`"):
+        _torchops.ops()
+    (tmp_path / "_vidc_torch_ops.so").write_bytes(b"")
+    with pytest.raises(RuntimeError, match="--force"):
+        _torchops.ops()

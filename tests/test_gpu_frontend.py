@@ -1,7 +1,5 @@
-"""The thin torch C++ extension (csrc/torch_ops.cpp, `torch.ops.vidc.*`) in front of the C ABI: same bits as the ctypes
-route, reference error behaviour, traceable by torch.compile(fullgraph=True), and cheaper on the host."""
-import time
-
+"""The thin torch C++ extension (csrc/torch_ops.cpp, `torch.ops.vidc.*`) in front of the C ABI: the only route of the hot
+entry points, reference error behaviour, traceable by torch.compile(fullgraph=True)."""
 import numpy as np
 import pytest
 
@@ -21,30 +19,22 @@ def _setup(dev, cam="S1", B=4):
     return w, t(rgb), t(depth), t(normals), t(I_g), t(I_a)
 
 
-def test_extension_is_loaded_and_matches_the_ctypes_route(cuda_device):
+def test_extension_is_loaded_and_keeps_the_memory_format(cuda_device):
+    """The hot entry points run through the loaded extension; channels-last input gives channels-last output.  Their bits
+    against the oracle and the goldens are pinned by test_gpu_parity.py and test_gpu_golden.py."""
     import torch
     from vi_depth_completion_b200 import _torchops
-    assert _torchops.ops() is not None, "_vidc_torch_ops.so missing: __graft_entry__.build() builds it"
+    assert _torchops.ops() is torch.ops.vidc
     w, rgb, depth, normals, g, a = _setup(cuda_device)
-    outs = {}
-    for tag in ("torch", "ctypes"):
-        saved = dict(_torchops._state)
-        if tag == "ctypes":
-            _torchops._state.update(tried=True, ops=None)
-        try:
-            H1, y = w.warp_with_gravity_center_aligned(rgb, g, a)
-            _, yd = w.warp_with_gravity_center_aligned(depth, g, a, interp_mode="nearest")
-            _, z = w.inverse_warp_normal_image_with_gravity_center_aligned(normals, g, a)
-            _, zn = w.unwarp_normals(normals, g, a)
-            _, r2, d2, m2 = w.warp_rgbd(rgb, depth, g, a)
-            Hh, R, Hi = w._build_homography(g, a)
-            _, ycl = w.warp_with_gravity_center_aligned(rgb.contiguous(memory_format=torch.channels_last), g, a)
-            outs[tag] = (H1, y, yd, z, zn, r2, d2, m2, Hh, R, Hi, ycl)
-        finally:
-            _torchops._state.update(saved)
-    for p, q in zip(outs["torch"], outs["ctypes"]):
-        assert p.shape == q.shape and p.stride() == q.stride() and torch.equal(p, q)
-    assert outs["torch"][-1].is_contiguous(memory_format=torch.channels_last)
+    _, y = w.warp_with_gravity_center_aligned(rgb, g, a)
+    w.warp_with_gravity_center_aligned(depth, g, a, interp_mode="nearest")
+    w.inverse_warp_normal_image_with_gravity_center_aligned(normals, g, a)
+    w.unwarp_normals(normals, g, a)
+    w.warp_rgbd(rgb, depth, g, a)
+    w._build_homography(g, a)
+    _, ycl = w.warp_with_gravity_center_aligned(rgb.contiguous(memory_format=torch.channels_last), g, a)
+    assert ycl.is_contiguous(memory_format=torch.channels_last) and not ycl.is_contiguous()
+    assert y.is_contiguous() and torch.equal(ycl, y)
 
 
 def test_extension_error_behaviour(cuda_device):
@@ -77,73 +67,35 @@ def test_torch_compile_fullgraph(cuda_device):
     assert torch.equal(want[0], got[0]) and torch.equal(want[1], got[1])
 
 
-def test_host_time_per_call(cuda_device):
-    """B = 1 at 320x240 (the reference's only documented entry point, demo.sh:7-11): host time of one eager step through the
-    extension against the ctypes route (round 1: 88.7 us per step of two calls)."""
-    import torch
-    from vi_depth_completion_b200 import _torchops
-    w, rgb, depth, normals, g, a = _setup(cuda_device, B=1)
-
-    def step():
-        w.warp_rgbd(rgb, depth, g, a)
-        w.unwarp_normals(normals, g, a)
-
-    res = {}
-    for tag in ("torch", "ctypes"):
-        saved = dict(_torchops._state)
-        if tag == "ctypes":
-            _torchops._state.update(tried=True, ops=None)
-        try:
-            for _ in range(200):
-                step()
-            torch.cuda.synchronize()
-            t0 = time.perf_counter()
-            for _ in range(2000):
-                step()
-            res[tag] = (time.perf_counter() - t0) / 2000 * 1e6
-            torch.cuda.synchronize()
-        finally:
-            _torchops._state.update(saved)
-    print(f"host us per step (warp_rgbd + unwarp_normals, B=1): extension {res['torch']:.1f}, ctypes {res['ctypes']:.1f}")
-    assert res["torch"] < res["ctypes"]
-
-
-@pytest.mark.parametrize("frontend", ["torch", "ctypes"])
-def test_parameters_prepared_once_per_batch(cuda_device, frontend):
+def test_parameters_prepared_once_per_batch(cuda_device):
     """prepare() + warp_rgbd(params=) + unwarp_normals(params=): one per-frame kernel for the batch instead of one per call
-    (the reference rebuilds the homographies in every call, :124 and :225).  Same bits as the calls that take I_g / I_a, through
-    the extension and through ctypes; two launches saved per step; the handle is checked (camera, batch, device)."""
+    (the reference rebuilds the homographies in every call, :124 and :225).  Same bits as the calls that take I_g / I_a; two
+    launches saved per step; the handle is checked (camera, batch, device)."""
     import torch
-    from vi_depth_completion_b200 import _cabi, _torchops
+    from vi_depth_completion_b200 import _cabi
     from vi_depth_completion_b200.warping_2dof_alignment import Warping2DOFAlignment
     w, rgb, depth, normals, g, a = _setup(cuda_device, B=5)
-    saved = dict(_torchops._state)
-    if frontend == "ctypes":
-        _torchops._state.update(tried=True, ops=None)
-    try:
-        H0, r0, d0, m0 = w.warp_rgbd(rgb, depth, g, a)
-        _, z0 = w.unwarp_normals(normals, g, a)
-        _, zr0 = w.unwarp_normals(normals, g, a, normalize=False)
-        n0 = _cabi.lib().vidc_launch_count()
-        p = w.prepare(g, a)
-        H1, r1, d1, m1 = w.warp_rgbd(rgb, depth, params=p)
-        H2, z1 = w.unwarp_normals(normals, params=p)
-        _, zr1 = w.unwarp_normals(normals, params=p, normalize=False)
-        assert _cabi.lib().vidc_launch_count() - n0 == 4                    # 1 per-frame kernel + 3 warps
-        for x, y in ((H0, H1), (H0, H2), (r0, r1), (d0, d1), (m0, m1), (z0, z1), (zr0, zr1)):
-            assert torch.equal(x, y)
-        assert depth.dim() == 3 and d1.dim() == 3                            # 3-D depth in, 3-D depth out (:110-112, :153-154)
-        d4 = w.warp_rgbd(rgb, depth[:, None], params=p)[2]
-        assert d4.dim() == 4 and torch.equal(d4[:, 0], d0)
-        with pytest.raises(AssertionError):
-            w.warp_rgbd(rgb[:3], depth[:3], params=p)                        # batch of the handle
-        with pytest.raises(RuntimeError):
-            Warping2DOFAlignment(404., 404., 319.87654, 239.87603).unwarp_normals(normals, params=p)   # another camera
-        with pytest.raises(RuntimeError):
-            w.unwarp_normals(normals)                                        # neither gravity nor params
-        x = rgb.clone().requires_grad_(True)
-        out = w.warp_rgbd(x, depth, params=p)
-        with pytest.raises(NotImplementedError):
-            out[1].sum().backward()
-    finally:
-        _torchops._state.update(saved)
+    H0, r0, d0, m0 = w.warp_rgbd(rgb, depth, g, a)
+    _, z0 = w.unwarp_normals(normals, g, a)
+    _, zr0 = w.unwarp_normals(normals, g, a, normalize=False)
+    n0 = _cabi.lib().vidc_launch_count()
+    p = w.prepare(g, a)
+    H1, r1, d1, m1 = w.warp_rgbd(rgb, depth, params=p)
+    H2, z1 = w.unwarp_normals(normals, params=p)
+    _, zr1 = w.unwarp_normals(normals, params=p, normalize=False)
+    assert _cabi.lib().vidc_launch_count() - n0 == 4                    # 1 per-frame kernel + 3 warps
+    for x, y in ((H0, H1), (H0, H2), (r0, r1), (d0, d1), (m0, m1), (z0, z1), (zr0, zr1)):
+        assert torch.equal(x, y)
+    assert depth.dim() == 3 and d1.dim() == 3                            # 3-D depth in, 3-D depth out (:110-112, :153-154)
+    d4 = w.warp_rgbd(rgb, depth[:, None], params=p)[2]
+    assert d4.dim() == 4 and torch.equal(d4[:, 0], d0)
+    with pytest.raises(AssertionError):
+        w.warp_rgbd(rgb[:3], depth[:3], params=p)                        # batch of the handle
+    with pytest.raises(RuntimeError):
+        Warping2DOFAlignment(404., 404., 319.87654, 239.87603).unwarp_normals(normals, params=p)   # another camera
+    with pytest.raises(RuntimeError):
+        w.unwarp_normals(normals)                                        # neither gravity nor params
+    x = rgb.clone().requires_grad_(True)
+    out = w.warp_rgbd(x, depth, params=p)
+    with pytest.raises(NotImplementedError):
+        out[1].sum().backward()

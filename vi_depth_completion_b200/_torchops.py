@@ -1,29 +1,28 @@
 """Loader of the thin torch C++ extension (csrc/torch_ops.cpp -> _vidc_torch_ops.so): TORCH_LIBRARY operators `torch.ops.vidc.*`
-in front of the C ABI.  The operators and the ctypes binding (_cabi.py) enqueue the SAME kernels of libvidc_b200.so; the
-extension only removes Python marshalling from the hot entry points (B = 1 eager step: 88.7 us -> see profiles/r2_history.md)
-and makes them traceable by torch.compile.  VIDC_FRONTEND=ctypes selects the ctypes route for A/B runs; when the extension
-has not been built the class uses ctypes as well (both need libvidc_b200.so -- there is no CPU / PyTorch fallback either way).
+in front of the C ABI.  The hot entry points of Warping2DOFAlignment reach libvidc_b200.so through these operators only (no
+Python marshalling, traceable by torch.compile(fullgraph=True)); the ctypes binding (_cabi.py) carries the calls no operator
+takes.  Like libvidc_b200.so, the extension is part of the product: ops() raises when it is missing or does not load.
 """
 import os
 
-_HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.path.join(_HERE, "_vidc_torch_ops.so")
-_state = {"tried": False, "ops": None}
+LIB_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "_vidc_torch_ops.so")
+_ops = None
 
 
 def ops():
-    """torch.ops.vidc, or None when the extension is not available / not wanted."""
-    if not _state["tried"]:
-        _state["tried"] = True
-        if os.environ.get("VIDC_FRONTEND", "torch") != "ctypes" and os.path.exists(LIB_PATH):
-            import torch
-            from . import _cabi
-            _cabi.lib()                               # libvidc_b200.so first: a missing product library must raise, not hide
-            try:
-                torch.ops.load_library(LIB_PATH)
-                _state["ops"] = torch.ops.vidc
-            except OSError as e:                      # built against another torch: say so once, use the ctypes route
-                import warnings
-                warnings.warn(f"vi_depth_completion_b200: {LIB_PATH} could not be loaded ({e}); using the ctypes front end. "
-                              "Rebuild it with `python -m vi_depth_completion_b200.build --force`.")
-    return _state["ops"]
+    """torch.ops.vidc.  Raises RuntimeError (never falls back) when the extension has not been built or does not load."""
+    global _ops
+    if _ops is None:
+        import torch
+        from . import _cabi
+        _cabi.lib()                                   # libvidc_b200.so first: a missing product library is the error shown
+        if not os.path.exists(LIB_PATH):
+            raise RuntimeError(f"{LIB_PATH} is missing: the torch extension is part of the product and there is no fallback. "
+                               "Build it with `python -m vi_depth_completion_b200.build`.")
+        try:
+            torch.ops.load_library(LIB_PATH)
+        except OSError as e:                          # e.g. built against another torch
+            raise RuntimeError(f"{LIB_PATH} could not be loaded ({e}); rebuild it with "
+                               "`python -m vi_depth_completion_b200.build --force`.") from None
+        _ops = torch.ops.vidc
+    return _ops

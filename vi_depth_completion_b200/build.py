@@ -85,5 +85,4 @@ def build_torch_ops(force: bool = False) -> str:
 
 if __name__ == "__main__":
     print(build(force="--force" in sys.argv, verbose="-v" in sys.argv))
-    if "--no-torch-ops" not in sys.argv:
-        print(build_torch_ops(force="--force" in sys.argv))
+    print(build_torch_ops(force="--force" in sys.argv))

@@ -12,7 +12,6 @@
 #include <c10/cuda/CUDAGuard.h>
 #include <torch/library.h>
 
-#include <cmath>
 #include <tuple>
 
 #include "../../include/vidc_b200.h"
@@ -64,11 +63,14 @@ at::Tensor workspace(const vidc_camera& cam, int64_t B, const at::TensorOptions&
 }
 
 // outputs adopt the input's memory format (NCHW or channels-last), on the canvas size
-at::Tensor canvas_like_hw(const at::Tensor& x, int64_t H, int64_t W) {
+at::Tensor canvas_like(const at::Tensor& x, const vidc_camera& cam) {
     const bool cl = x.size(1) > 1 && x.is_contiguous(at::MemoryFormat::ChannelsLast) && !x.is_contiguous();
-    return at::empty({x.size(0), x.size(1), H, W}, x.options(), cl ? at::MemoryFormat::ChannelsLast : at::MemoryFormat::Contiguous);
+    return at::empty({x.size(0), x.size(1), cam.H, cam.W}, x.options(), cl ? at::MemoryFormat::ChannelsLast : at::MemoryFormat::Contiguous);
 }
-at::Tensor canvas_like(const at::Tensor& x, const vidc_camera& cam) { return canvas_like_hw(x, cam.H, cam.W); }
+// the uint8 validity mask of the fused forward warps: one plane per frame of x
+at::Tensor mask_canvas(const at::Tensor& x, const vidc_camera& cam) {
+    return at::empty({x.size(0), 1, cam.H, cam.W}, x.options().dtype(at::kByte));
+}
 
 // ---- warp_with_gravity_center_aligned (:108-156), 4-D input ------------------------------------------------------------------
 std::tuple<at::Tensor, at::Tensor> warp_forward(const at::Tensor& x, const at::Tensor& I_g, const at::Tensor& I_a, double fx, double fy,
@@ -118,7 +120,7 @@ std::tuple<at::Tensor, at::Tensor, at::Tensor, at::Tensor> warp_rgbd(const at::T
     const c10::cuda::CUDAGuard guard(rgb.device());
     auto [g, a] = gravity(I_g, I_a, rgb.device());
     at::Tensor rgb_w = canvas_like(rgb, cam), depth_w = canvas_like(depth, cam);
-    at::Tensor mask = at::empty({rgb.size(0), 1, cam.H, cam.W}, rgb.options().dtype(at::kByte));
+    at::Tensor mask = mask_canvas(rgb, cam);
     at::Tensor Hm = at::empty({g.size(0), 3, 3}, rgb.options());
     at::Tensor ws = workspace(cam, g.size(0), rgb.options());
     const vidc_image ri = image_of(rgb), di = image_of(depth), rwi = image_of(rgb_w), dwi = image_of(depth_w);
@@ -135,8 +137,8 @@ void check_u8_frames(const at::Tensor& rgb) {
     TORCH_CHECK(rgb.dim() == 4 && rgb.size(3) == 3, "x_rgb: expected (B,h,w,3) uint8 frames, got ", rgb.sizes());
     TORCH_CHECK(rgb.is_contiguous(), "x_rgb: expected contiguous (B,h,w,3) frames");
 }
-at::Tensor rgb_canvas_u8(const at::Tensor& rgb, int64_t H, int64_t W) {
-    return at::empty({rgb.size(0), 3, H, W}, rgb.options().dtype(at::kFloat));
+at::Tensor rgb_canvas_u8(const at::Tensor& rgb, const vidc_camera& cam) {
+    return at::empty({rgb.size(0), 3, cam.H, cam.W}, rgb.options().dtype(at::kFloat));
 }
 int warp_rgbd_u8_call(const vidc_camera& cam, const at::Tensor& rgb, const at::Tensor& depth, const float* g, const float* a, int64_t B_gravity,
                       int64_t depth_mode, const at::Tensor& ws, float* Hm, const at::Tensor& rgb_w, const at::Tensor& depth_w, const at::Tensor& mask) {
@@ -155,8 +157,8 @@ std::tuple<at::Tensor, at::Tensor, at::Tensor, at::Tensor> warp_rgbd_u8(const at
     const vidc_camera cam = make_camera(fx, fy, cx, cy);
     const c10::cuda::CUDAGuard guard(rgb.device());
     auto [g, a] = gravity(I_g, I_a, rgb.device());
-    at::Tensor rgb_w = rgb_canvas_u8(rgb, cam.H, cam.W), depth_w = canvas_like(depth, cam);
-    at::Tensor mask = at::empty({rgb.size(0), 1, cam.H, cam.W}, rgb.options());
+    at::Tensor rgb_w = rgb_canvas_u8(rgb, cam), depth_w = canvas_like(depth, cam);
+    at::Tensor mask = mask_canvas(rgb, cam);
     at::Tensor Hm = at::empty({g.size(0), 3, 3}, depth.options());
     at::Tensor ws = workspace(cam, g.size(0), depth.options());
     check_status(warp_rgbd_u8_call(cam, rgb, depth, g.data_ptr<float>(), a.data_ptr<float>(), g.size(0), depth_mode, ws, Hm.data_ptr<float>(),
@@ -193,7 +195,7 @@ std::tuple<at::Tensor, at::Tensor, at::Tensor> warp_rgbd_prepared(const at::Tens
     const c10::cuda::CUDAGuard guard(rgb.device());
     check_prepared(ws, cam, rgb.size(0), rgb.device());
     at::Tensor rgb_w = canvas_like(rgb, cam), depth_w = canvas_like(depth, cam);
-    at::Tensor mask = at::empty({rgb.size(0), 1, cam.H, cam.W}, rgb.options().dtype(at::kByte));
+    at::Tensor mask = mask_canvas(rgb, cam);
     const vidc_image ri = image_of(rgb), di = image_of(depth), rwi = image_of(rgb_w), dwi = image_of(depth_w);
     check_status(vidc_warp_rgbd(&cam, &ri, &di, nullptr, nullptr, (int32_t)rgb.size(0), (vidc_interp)depth_mode,
                                 reinterpret_cast<vidc_frame_params*>(ws.data_ptr<float>()), nullptr, &rwi, &dwi,
@@ -209,8 +211,8 @@ std::tuple<at::Tensor, at::Tensor, at::Tensor> warp_rgbd_u8_prepared(const at::T
     const vidc_camera cam = make_camera(fx, fy, cx, cy);
     const c10::cuda::CUDAGuard guard(rgb.device());
     check_prepared(ws, cam, rgb.size(0), rgb.device());
-    at::Tensor rgb_w = rgb_canvas_u8(rgb, cam.H, cam.W), depth_w = canvas_like(depth, cam);
-    at::Tensor mask = at::empty({rgb.size(0), 1, cam.H, cam.W}, rgb.options());
+    at::Tensor rgb_w = rgb_canvas_u8(rgb, cam), depth_w = canvas_like(depth, cam);
+    at::Tensor mask = mask_canvas(rgb, cam);
     check_status(warp_rgbd_u8_call(cam, rgb, depth, nullptr, nullptr, rgb.size(0), depth_mode, ws, nullptr, rgb_w, depth_w, mask));
     return {rgb_w, depth_w, mask};
 }
@@ -243,53 +245,47 @@ std::tuple<at::Tensor, at::Tensor, at::Tensor> build_homography(const at::Tensor
     return {out[0], out[1], out[2]};
 }
 
-// ---- Meta kernels: shapes only (torch.compile / FakeTensor) -----------------------------------------------------------------------
-int64_t canvas_w(double cx) { return (int64_t)std::ceil(2.0 * cx); }
-int64_t canvas_h(double cy) { return (int64_t)std::ceil(2.0 * cy); }
-
-std::tuple<at::Tensor, at::Tensor> warp_forward_meta(const at::Tensor& x, const at::Tensor& I_g, const at::Tensor&, double, double, double cx,
-                                                     double cy, int64_t) {
+// ---- Meta kernels: shapes only (torch.compile / FakeTensor).  The canvas comes from vidc_camera_init and the workspace from
+// vidc_workspace_bytes, as in the CUDA kernels, so both allocate the same sizes and reject the same intrinsics ---------------------
+std::tuple<at::Tensor, at::Tensor> warp_forward_meta(const at::Tensor& x, const at::Tensor& I_g, const at::Tensor&, double fx, double fy,
+                                                     double cx, double cy, int64_t) {
     TORCH_CHECK(x.dim() == 4, "x: expected a 4-D tensor, got ", x.dim(), "-D");
-    return {at::empty({I_g.size(0), 3, 3}, x.options()), canvas_like_hw(x, canvas_h(cy), canvas_w(cx))};
+    return {at::empty({I_g.size(0), 3, 3}, x.options()), canvas_like(x, make_camera(fx, fy, cx, cy))};
 }
-std::tuple<at::Tensor, at::Tensor> unwarp_normals_meta(const at::Tensor& x, const at::Tensor& I_g, const at::Tensor&, double, double, double cx,
-                                                       double cy, bool) {
+std::tuple<at::Tensor, at::Tensor> unwarp_normals_meta(const at::Tensor& x, const at::Tensor& I_g, const at::Tensor&, double fx, double fy,
+                                                       double cx, double cy, bool) {
     TORCH_CHECK(x.dim() == 4, "x: expected a 4-D tensor, got ", x.dim(), "-D");
-    return {at::empty({I_g.size(0), 3, 3}, x.options()), canvas_like_hw(x, canvas_h(cy), canvas_w(cx))};
+    return {at::empty({I_g.size(0), 3, 3}, x.options()), canvas_like(x, make_camera(fx, fy, cx, cy))};
 }
 std::tuple<at::Tensor, at::Tensor, at::Tensor, at::Tensor> warp_rgbd_meta(const at::Tensor& rgb, const at::Tensor& depth, const at::Tensor& I_g,
-                                                                          const at::Tensor&, double, double, double cx, double cy, int64_t) {
-    const int64_t H = canvas_h(cy), W = canvas_w(cx);
-    return {at::empty({I_g.size(0), 3, 3}, rgb.options()), canvas_like_hw(rgb, H, W), canvas_like_hw(depth, H, W),
-            at::empty({rgb.size(0), 1, H, W}, rgb.options().dtype(at::kByte))};
+                                                                          const at::Tensor&, double fx, double fy, double cx, double cy, int64_t) {
+    const vidc_camera cam = make_camera(fx, fy, cx, cy);
+    return {at::empty({I_g.size(0), 3, 3}, rgb.options()), canvas_like(rgb, cam), canvas_like(depth, cam), mask_canvas(rgb, cam)};
 }
 std::tuple<at::Tensor, at::Tensor, at::Tensor, at::Tensor> warp_rgbd_u8_meta(const at::Tensor& rgb, const at::Tensor& depth, const at::Tensor& I_g,
-                                                                             const at::Tensor&, double, double, double cx, double cy, int64_t) {
-    const int64_t H = canvas_h(cy), W = canvas_w(cx);
-    return {at::empty({I_g.size(0), 3, 3}, depth.options()), rgb_canvas_u8(rgb, H, W), canvas_like_hw(depth, H, W),
-            at::empty({rgb.size(0), 1, H, W}, rgb.options().dtype(at::kByte))};
+                                                                             const at::Tensor&, double fx, double fy, double cx, double cy, int64_t) {
+    const vidc_camera cam = make_camera(fx, fy, cx, cy);
+    return {at::empty({I_g.size(0), 3, 3}, depth.options()), rgb_canvas_u8(rgb, cam), canvas_like(depth, cam), mask_canvas(rgb, cam)};
 }
 std::tuple<at::Tensor, at::Tensor, at::Tensor> warp_rgbd_u8_prepared_meta(const at::Tensor& rgb, const at::Tensor& depth, const at::Tensor&,
-                                                                          double, double, double cx, double cy, int64_t) {
-    const int64_t H = canvas_h(cy), W = canvas_w(cx);
-    return {rgb_canvas_u8(rgb, H, W), canvas_like_hw(depth, H, W), at::empty({rgb.size(0), 1, H, W}, rgb.options().dtype(at::kByte))};
+                                                                          double fx, double fy, double cx, double cy, int64_t) {
+    const vidc_camera cam = make_camera(fx, fy, cx, cy);
+    return {rgb_canvas_u8(rgb, cam), canvas_like(depth, cam), mask_canvas(rgb, cam)};
 }
-int64_t workspace_floats_meta(double cx, double cy, int64_t B) {            // as vidc_workspace_bytes: 192 B per frame + 16 B per tile
-    const int64_t tiles = ((canvas_w(cx) + 31) / 32) * ((canvas_h(cy) + 31) / 32), n = std::max<int64_t>(B, 1);
-    return (n * 192 + n * tiles * 16 + 3) / 4;
-}
-std::tuple<at::Tensor, at::Tensor> frame_params_meta(const at::Tensor& I_g, const at::Tensor&, double, double, double cx, double cy) {
-    return {at::empty({workspace_floats_meta(cx, cy, I_g.size(0))}, I_g.options()), at::empty({I_g.size(0), 3, 3}, I_g.options())};
+std::tuple<at::Tensor, at::Tensor> frame_params_meta(const at::Tensor& I_g, const at::Tensor&, double fx, double fy, double cx, double cy) {
+    return {workspace(make_camera(fx, fy, cx, cy), I_g.size(0), I_g.options()), at::empty({I_g.size(0), 3, 3}, I_g.options())};
 }
 std::tuple<at::Tensor, at::Tensor, at::Tensor> warp_rgbd_prepared_meta(const at::Tensor& rgb, const at::Tensor& depth, const at::Tensor&,
-                                                                       double, double, double cx, double cy, int64_t) {
-    const int64_t H = canvas_h(cy), W = canvas_w(cx);
-    return {canvas_like_hw(rgb, H, W), canvas_like_hw(depth, H, W), at::empty({rgb.size(0), 1, H, W}, rgb.options().dtype(at::kByte))};
+                                                                       double fx, double fy, double cx, double cy, int64_t) {
+    const vidc_camera cam = make_camera(fx, fy, cx, cy);
+    return {canvas_like(rgb, cam), canvas_like(depth, cam), mask_canvas(rgb, cam)};
 }
-at::Tensor unwarp_normals_prepared_meta(const at::Tensor& x, const at::Tensor&, double, double, double cx, double cy, bool) {
-    return canvas_like_hw(x, canvas_h(cy), canvas_w(cx));
+at::Tensor unwarp_normals_prepared_meta(const at::Tensor& x, const at::Tensor&, double fx, double fy, double cx, double cy, bool) {
+    return canvas_like(x, make_camera(fx, fy, cx, cy));
 }
-std::tuple<at::Tensor, at::Tensor, at::Tensor> build_homography_meta(const at::Tensor& I_g, const at::Tensor&, double, double, double, double) {
+std::tuple<at::Tensor, at::Tensor, at::Tensor> build_homography_meta(const at::Tensor& I_g, const at::Tensor&, double fx, double fy, double cx,
+                                                                     double cy) {
+    make_camera(fx, fy, cx, cy);
     auto t = [&] { return at::empty({I_g.size(0), 3, 3}, I_g.options()); };
     return {t(), t(), t()};
 }

@@ -5,7 +5,8 @@ MARSLab-UMN/vi_depth_completion `Warping2DOFAlignment` (networks/warping_2dof_al
 so networks/surface_normal.py (:70, :148, :169) runs unmodified on top of it.  Every method is a thin
 host-side wrapper: it checks shapes, allocates the outputs with torch (device memory + streams are
 the only things torch is used for) and enqueues the hand-written sm_100a kernels of
-libvidc_b200.so on the current CUDA stream through the C ABI in include/vidc_b200.h.
+libvidc_b200.so on the current CUDA stream through the C ABI in include/vidc_b200.h: the hot entry points through the
+operators of the torch C++ extension (_torchops.py) only, the calls no operator takes through ctypes (_cabi.py).
 
 Differences from the reference that are deliberate (see DESIGN.md):
   * the device follows the inputs (the reference pins 'cuda:0', :7);
@@ -315,25 +316,13 @@ class Warping2DOFAlignment:
 
     # networks/warping_2dof_alignment.py:35-58
     def _build_homography(self, I_g, I_a):
-        ops = _torchops.ops()
-        grav_grad = _wants_grad(I_g, I_a)
-        if ops is not None and isinstance(I_g, torch.Tensor) and isinstance(I_a, torch.Tensor):
-            out = _op(ops.build_homography, _nd(I_g), _nd(I_a), *self._intr)
-            if not grav_grad:
-                return out
-            g, a = _gravity(I_g, I_a, I_g.device)
-            return _HomographyFn.apply(g, a, self, *out)
         _require_cuda_f32(I_g, "I_g")
-        device = I_g.device
-        g, a = _gravity(I_g, I_a, device)
-        B = g.shape[0]
-        out = torch.empty((3, B, 3, 3), dtype=torch.float32, device=device)
-        with torch.cuda.device(device):
-            check(lib().vidc_build_homography(ctypes.byref(self._cam), g.data_ptr(), a.data_ptr(), B,
-                                              out[0].data_ptr(), out[1].data_ptr(), out[2].data_ptr(), _stream_ptr(device)))
-        if grav_grad:
-            return _HomographyFn.apply(g, a, self, out[0], out[1], out[2])
-        return out[0], out[1], out[2]
+        _require_cuda_f32(I_a, "I_a")
+        out = _op(_torchops.ops().build_homography, _nd(I_g), _nd(I_a), *self._intr)
+        if not _wants_grad(I_g, I_a):
+            return out
+        g, a = _gravity(I_g, I_a, I_g.device)
+        return _HomographyFn.apply(g, a, self, *out)
 
     def frame_params(self, I_g, I_a):
         """Additive: the (B,48) per-frame parameter block (vidc_frame_params) as a tensor."""
@@ -363,24 +352,14 @@ class Warping2DOFAlignment:
         if x.dim() != 4:
             raise RuntimeError(f"x: expected a 3-D or 4-D tensor, got {x.dim()}-D")
         mode = _check_interp_mode(interp_mode, allow_bicubic=True)
-        device = x.device
-        ops = _torchops.ops()
+        _require_cuda_f32(I_g, "I_g")
+        _require_cuda_f32(I_a, "I_a")
         needs_graph = torch.is_grad_enabled() and x.requires_grad
         grav_grad = _wants_grad(I_g, I_a)
-        if ops is not None and isinstance(I_g, torch.Tensor) and isinstance(I_a, torch.Tensor):
-            # thin torch C++ extension; the operators carry no autograd kernel -- the graph is attached below (_attach), so they
-            # only ever see detached tensors (torch's not-implemented fallback would otherwise hand out silent zero gradients)
-            Cg_H_C, y = _op(ops.warp_forward, x.detach() if needs_graph else x, _nd(I_g), _nd(I_a), *self._intr, mode)
-            g, a = _gravity(I_g, I_a, device) if (needs_graph or grav_grad) else (None, None)
-        else:
-            g, a = _gravity(I_g, I_a, device)
-            y = self._empty_like_canvas(x)
-            Cg_H_C = torch.empty((g.shape[0], 3, 3), dtype=torch.float32, device=device)
-            xi, yi = _image(x), _image(y)
-            with torch.cuda.device(device):
-                check(lib().vidc_warp_forward(ctypes.byref(self._cam), ctypes.byref(xi), g.data_ptr(), a.data_ptr(), g.shape[0],
-                                              mode, self._params_ws(g.shape[0], device).data_ptr(), Cg_H_C.data_ptr(),
-                                              ctypes.byref(yi), _stream_ptr(device)))
+        # the operators carry no autograd kernel -- the graph is attached below (_attach), so they only ever see detached
+        # tensors (torch's not-implemented fallback would otherwise hand out silent zero gradients)
+        Cg_H_C, y = _op(_torchops.ops().warp_forward, x.detach() if needs_graph else x, _nd(I_g), _nd(I_a), *self._intr, mode)
+        g, a = _gravity(I_g, I_a, x.device) if (needs_graph or grav_grad) else (None, None)
         # the scatter kernel of vidc_warp_backward covers bilinear and nearest; bicubic is forward-only
         if mode == _cabi.VIDC_BICUBIC:
             if needs_graph:
@@ -421,26 +400,27 @@ class Warping2DOFAlignment:
         if x.dim() != 4:
             raise RuntimeError(f"x: expected a 4-D tensor, got {x.dim()}-D")
         device = x.device
-        ops = _torchops.ops()
         grav_grad = _wants_grad(I_g, I_a)
-        if ops is not None and not want_valid and isinstance(I_g, torch.Tensor) and isinstance(I_a, torch.Tensor):
-            needs_graph = torch.is_grad_enabled() and x.requires_grad
-            Cg_H_C, z = _op(ops.unwarp_normals, x.detach() if needs_graph else x, _nd(I_g), _nd(I_a), *self._intr, bool(normalize))
-            if needs_graph or grav_grad:
-                g, a = _gravity(I_g, I_a, device)
-                return self._unwarp_graph(x, z, Cg_H_C, g, a, I_g, I_a, normalize, needs_graph, grav_grad and gravity_grad) + (None,)
-            return Cg_H_C, z, None
-        g, a = _gravity(I_g, I_a, device)
-        z = self._empty_like_canvas(x)
-        Cg_H_C = torch.empty((g.shape[0], 3, 3), dtype=torch.float32, device=device)
-        valid = torch.empty((x.shape[0], 1, int(self.H), int(self.W)), dtype=torch.uint8, device=device) if want_valid else None
-        xi, zi = _image(x), _image(z)
-        with torch.cuda.device(device):
-            check(lib().vidc_unwarp_normals(ctypes.byref(self._cam), ctypes.byref(xi), g.data_ptr(), a.data_ptr(), g.shape[0],
-                                            1 if normalize else 0, self._params_ws(g.shape[0], device).data_ptr(),
-                                            Cg_H_C.data_ptr(), ctypes.byref(zi), valid.data_ptr() if want_valid else None,
-                                            _stream_ptr(device)))
         needs_graph = torch.is_grad_enabled() and x.requires_grad
+        if want_valid:                                          # no operator returns the validity plane
+            g, a = _gravity(I_g, I_a, device)
+            z = self._empty_like_canvas(x)
+            Cg_H_C = torch.empty((g.shape[0], 3, 3), dtype=torch.float32, device=device)
+            valid = torch.empty((x.shape[0], 1, int(self.H), int(self.W)), dtype=torch.uint8, device=device)
+            xi, zi = _image(x), _image(z)
+            with torch.cuda.device(device):
+                check(lib().vidc_unwarp_normals(ctypes.byref(self._cam), ctypes.byref(xi), g.data_ptr(), a.data_ptr(), g.shape[0],
+                                                1 if normalize else 0, self._params_ws(g.shape[0], device).data_ptr(),
+                                                Cg_H_C.data_ptr(), ctypes.byref(zi), valid.data_ptr(), _stream_ptr(device)))
+        else:
+            _require_cuda_f32(I_g, "I_g")
+            _require_cuda_f32(I_a, "I_a")
+            Cg_H_C, z = _op(_torchops.ops().unwarp_normals, x.detach() if needs_graph else x, _nd(I_g), _nd(I_a), *self._intr,
+                            bool(normalize))
+            if not (needs_graph or grav_grad):
+                return Cg_H_C, z, None
+            g, a = _gravity(I_g, I_a, device)
+            valid = None
         return self._unwarp_graph(x, z, Cg_H_C, g, a, I_g, I_a, normalize, needs_graph, grav_grad and gravity_grad) + (valid,)
 
     def _unwarp_graph(self, x, z, Cg_H_C, g, a, I_g, I_a, normalize, needs_graph, grav_diff):
@@ -494,19 +474,10 @@ class Warping2DOFAlignment:
         """Everything the two fused entry points need per frame (homographies, canvas scale, the kernels' per-tile tables),
         computed ONCE for a batch: pass the result as `params=` to warp_rgbd and unwarp_normals, which then launch no
         per-frame kernel of their own.  Valid for this camera and these I_g / I_a values."""
-        ops = _torchops.ops()
-        grav = (I_g, I_a) if _wants_grad(I_g, I_a) else ()
-        if ops is not None and isinstance(I_g, torch.Tensor) and isinstance(I_a, torch.Tensor):
-            ws, H = _op(ops.frame_params, _nd(I_g), _nd(I_a), *self._intr)
-            return FrameParams(ws, _no_gravity_grad((H,), *grav)[0], self._intr, grav)
         _require_cuda_f32(I_g, "I_g")
-        device = I_g.device
-        g, a = _gravity(I_g, I_a, device)
-        ws = self._params_ws(g.shape[0], device)
-        H = torch.empty((g.shape[0], 3, 3), dtype=torch.float32, device=device)
-        with torch.cuda.device(device):
-            check(lib().vidc_frame_params_prepare(ctypes.byref(self._cam), g.data_ptr(), a.data_ptr(), g.shape[0], ws.data_ptr(),
-                                                  H.data_ptr(), _stream_ptr(device)))
+        _require_cuda_f32(I_a, "I_a")
+        grav = (I_g, I_a) if _wants_grad(I_g, I_a) else ()
+        ws, H = _op(_torchops.ops().frame_params, _nd(I_g), _nd(I_a), *self._intr)
         return FrameParams(ws, _no_gravity_grad((H,), *grav)[0], self._intr, grav)
 
     def _prepared(self, params, x, name):
@@ -527,42 +498,29 @@ class Warping2DOFAlignment:
         _check_interp_mode(depth_mode)
         _require_cuda_f32(x_rgb, "x_rgb")
         device = x_rgb.device
-        ops = _torchops.ops()
+        mode = _cabi.VIDC_BILINEAR if depth_mode == "bilinear" else _cabi.VIDC_NEAREST
         if params is not None:
             if x_rgb.dim() != 4 or not isinstance(x_depth, torch.Tensor) or not with_mask or with_coverage:
                 raise RuntimeError("warp_rgbd(params=...): RGB (B,3,h,w) + depth, mask on, no coverage")
             p = self._prepared(params, x_rgb, "x_rgb")
             _require_cuda_f32(x_depth, "x_depth")
             d4 = x_depth.view(x_depth.shape[0], 1, x_depth.shape[1], x_depth.shape[2]) if x_depth.dim() == 3 else x_depth
-            mode = _cabi.VIDC_BILINEAR if depth_mode == "bilinear" else _cabi.VIDC_NEAREST
-            if ops is not None:
-                rgb_w, depth_w, mask = _op(ops.warp_rgbd_prepared, x_rgb.detach() if x_rgb.requires_grad else x_rgb,
-                                           d4.detach() if d4.requires_grad else d4, p.ws, *self._intr, mode)
-            else:
-                if d4.device != device:
-                    raise RuntimeError(f"x_depth must live on {device}, got {d4.device}")
-                rgb_w, depth_w = self._empty_like_canvas(x_rgb), self._empty_like_canvas(d4)
-                mask = torch.empty((x_rgb.shape[0], 1, int(self.H), int(self.W)), dtype=torch.uint8, device=device)
-                ri, di, rwi, dwi = _image(x_rgb), _image(d4), _image(rgb_w), _image(depth_w)
-                with torch.cuda.device(device):
-                    check(lib().vidc_warp_rgbd(ctypes.byref(self._cam), ctypes.byref(ri), ctypes.byref(di), None, None, p.B, mode,
-                                               p.ws.data_ptr(), None, ctypes.byref(rwi), ctypes.byref(dwi), mask.data_ptr(), None,
-                                               _stream_ptr(device)))
+            rgb_w, depth_w, mask = _op(_torchops.ops().warp_rgbd_prepared, _nd(x_rgb), _nd(d4), p.ws, *self._intr, mode)
             if x_depth.dim() == 3:
                 depth_w = depth_w.view(depth_w.shape[0], depth_w.shape[2], depth_w.shape[3])
             return _no_gravity_grad((p.H, _attach(x_rgb, rgb_w), _attach(x_depth, depth_w), mask), *p.grav)
         if I_g is None or I_a is None:
             raise RuntimeError("warp_rgbd: pass I_g and I_a, or params=prepare(I_g, I_a)")
-        if (ops is not None and with_mask and not with_coverage and isinstance(x_depth, torch.Tensor) and x_rgb.dim() == 4
-                and isinstance(I_g, torch.Tensor) and isinstance(I_a, torch.Tensor)):
+        if with_mask and not with_coverage and x_depth is not None:
+            _require_cuda_f32(x_depth, "x_depth")
+            _require_cuda_f32(I_g, "I_g")
+            _require_cuda_f32(I_a, "I_a")
             d4 = x_depth.view(x_depth.shape[0], 1, x_depth.shape[1], x_depth.shape[2]) if x_depth.dim() == 3 else x_depth
-            Cg_H_C, rgb_w, depth_w, mask = _op(ops.warp_rgbd, x_rgb.detach() if x_rgb.requires_grad else x_rgb,
-                                               d4.detach() if d4.requires_grad else d4, _nd(I_g), _nd(I_a), *self._intr,
-                                               _cabi.VIDC_BILINEAR if depth_mode == "bilinear" else _cabi.VIDC_NEAREST)
+            Cg_H_C, rgb_w, depth_w, mask = _op(_torchops.ops().warp_rgbd, _nd(x_rgb), _nd(d4), _nd(I_g), _nd(I_a), *self._intr, mode)
             if x_depth.dim() == 3:
                 depth_w = depth_w.view(depth_w.shape[0], depth_w.shape[2], depth_w.shape[3])
             return _no_gravity_grad((Cg_H_C, _attach(x_rgb, rgb_w), _attach(x_depth, depth_w), mask), I_g, I_a)   # forward-only
-        g, a = _gravity(I_g, I_a, device)
+        g, a = _gravity(I_g, I_a, device)                       # coverage, no mask or no depth: no operator takes these
         B = x_rgb.shape[0]
         squeeze = False
         di = dwi = None
@@ -583,10 +541,8 @@ class Warping2DOFAlignment:
         ri, rwi = _image(x_rgb), _image(rgb_w)
         with torch.cuda.device(device):
             check(lib().vidc_warp_rgbd(ctypes.byref(self._cam), ctypes.byref(ri), ctypes.byref(di) if di is not None else None,
-                                       g.data_ptr(), a.data_ptr(), g.shape[0],
-                                       _cabi.VIDC_BILINEAR if depth_mode == "bilinear" else _cabi.VIDC_NEAREST,
-                                       self._params_ws(g.shape[0], device).data_ptr(), Cg_H_C.data_ptr(),
-                                       ctypes.byref(rwi), ctypes.byref(dwi) if dwi is not None else None,
+                                       g.data_ptr(), a.data_ptr(), g.shape[0], mode, self._params_ws(g.shape[0], device).data_ptr(),
+                                       Cg_H_C.data_ptr(), ctypes.byref(rwi), ctypes.byref(dwi) if dwi is not None else None,
                                        mask.data_ptr() if with_mask else None, cov.data_ptr() if with_coverage else None,
                                        _stream_ptr(device)))
         if squeeze:
@@ -607,36 +563,27 @@ class Warping2DOFAlignment:
         x = rgb_u8.contiguous()
         device = x.device
         mode = _cabi.VIDC_BILINEAR if depth_mode == "bilinear" else _cabi.VIDC_NEAREST
-        ops = _torchops.ops()
         d4 = None
         if x_depth is not None:
             _require_cuda_f32(x_depth, "x_depth")
             d4 = x_depth.view(x_depth.shape[0], 1, x_depth.shape[1], x_depth.shape[2]) if x_depth.dim() == 3 else x_depth
+        cov = None
         if params is not None:
             if d4 is None or not with_mask or with_coverage:
                 raise RuntimeError("warp_rgbd_u8(params=...): depth, mask on, no coverage")
             p = self._prepared(params, x, "rgb_u8")
-            g = a = None
-            grav = p.grav
-        else:
-            if I_g is None or I_a is None:
-                raise RuntimeError("warp_rgbd_u8: pass I_g and I_a, or params=prepare(I_g, I_a)")
+            rgb_w, depth_w, mask = _op(_torchops.ops().warp_rgbd_u8_prepared, x, _nd(d4), p.ws, *self._intr, mode)
+            Cg_H_C, grav = p.H, p.grav
+        elif I_g is None or I_a is None:
+            raise RuntimeError("warp_rgbd_u8: pass I_g and I_a, or params=prepare(I_g, I_a)")
+        elif d4 is not None and with_mask and not with_coverage:
+            _require_cuda_f32(I_g, "I_g")
+            _require_cuda_f32(I_a, "I_a")
+            Cg_H_C, rgb_w, depth_w, mask = _op(_torchops.ops().warp_rgbd_u8, x, _nd(d4), _nd(I_g), _nd(I_a), *self._intr, mode)
             grav = (I_g, I_a)
-        torch_op = ops is not None and d4 is not None and with_mask and not with_coverage and (
-            params is not None or (isinstance(I_g, torch.Tensor) and isinstance(I_a, torch.Tensor)))
-        cov = None
-        if torch_op:
-            if params is not None:
-                rgb_w, depth_w, mask = _op(ops.warp_rgbd_u8_prepared, x, _nd(d4), p.ws, *self._intr, mode)
-                Cg_H_C = p.H
-            else:
-                Cg_H_C, rgb_w, depth_w, mask = _op(ops.warp_rgbd_u8, x, _nd(d4), _nd(I_g), _nd(I_a), *self._intr, mode)
-        else:
-            if params is None:
-                g, a = _gravity(I_g, I_a, device)
-                ws, B_g, Cg_H_C = self._params_ws(g.shape[0], device), g.shape[0], torch.empty((g.shape[0], 3, 3), dtype=torch.float32, device=device)
-            else:
-                ws, B_g, Cg_H_C = p.ws, p.B, p.H
+        else:                                                   # coverage, no mask or no depth: no operator takes these
+            grav = (I_g, I_a)
+            g, a = _gravity(I_g, I_a, device)
             B = x.shape[0]
             di = dwi = depth_w = None
             if d4 is not None:
@@ -644,17 +591,18 @@ class Warping2DOFAlignment:
                     raise RuntimeError(f"x_depth must live on {device}, got {d4.device}")
                 depth_w = self._empty_like_canvas(d4)
                 di, dwi = _image(d4), _image(depth_w)
+            Cg_H_C = torch.empty((g.shape[0], 3, 3), dtype=torch.float32, device=device)
             rgb_w = torch.empty((B, 3, int(self.H), int(self.W)), dtype=torch.float32, device=device)
             mask = torch.empty((B, 1, int(self.H), int(self.W)), dtype=torch.uint8, device=device) if with_mask else None
             cov = torch.empty((B,), dtype=torch.int32, device=device) if with_coverage else None
             rwi = _image(rgb_w)
             with torch.cuda.device(device):
                 check(lib().vidc_warp_rgbd_u8(ctypes.byref(self._cam), x.data_ptr(), B, x.shape[1], x.shape[2],
-                                              ctypes.byref(di) if di is not None else None, g.data_ptr() if g is not None else None,
-                                              a.data_ptr() if a is not None else None, B_g, mode, ws.data_ptr(),
-                                              Cg_H_C.data_ptr() if params is None else None, ctypes.byref(rwi),
-                                              ctypes.byref(dwi) if dwi is not None else None, mask.data_ptr() if with_mask else None,
-                                              cov.data_ptr() if with_coverage else None, _stream_ptr(device)))
+                                              ctypes.byref(di) if di is not None else None, g.data_ptr(), a.data_ptr(), g.shape[0],
+                                              mode, self._params_ws(g.shape[0], device).data_ptr(), Cg_H_C.data_ptr(),
+                                              ctypes.byref(rwi), ctypes.byref(dwi) if dwi is not None else None,
+                                              mask.data_ptr() if with_mask else None, cov.data_ptr() if with_coverage else None,
+                                              _stream_ptr(device)))
         if depth_w is not None:
             if x_depth.dim() == 3:
                 depth_w = depth_w.view(depth_w.shape[0], depth_w.shape[2], depth_w.shape[3])
@@ -731,15 +679,7 @@ class Warping2DOFAlignment:
                 raise RuntimeError("unwarp_normals(params=...): a 4-D image, no validity output")
             p = self._prepared(params, y, "x")
             needs_graph = torch.is_grad_enabled() and y.requires_grad
-            ops = _torchops.ops()
-            if ops is not None:
-                z = _op(ops.unwarp_normals_prepared, y.detach() if needs_graph else y, p.ws, *self._intr, bool(normalize))
-            else:
-                z = self._empty_like_canvas(y)
-                yi, zi = _image(y), _image(z)
-                with torch.cuda.device(y.device):
-                    check(lib().vidc_unwarp_normals(ctypes.byref(self._cam), ctypes.byref(yi), None, None, p.B, 1 if normalize else 0,
-                                                    p.ws.data_ptr(), None, ctypes.byref(zi), None, _stream_ptr(y.device)))
+            z = _op(_torchops.ops().unwarp_normals_prepared, y.detach() if needs_graph else y, p.ws, *self._intr, bool(normalize))
             return _no_gravity_grad((p.H, (_attach(y, z) if needs_graph else z)), *p.grav)   # forward-only with a prepared workspace
         if I_g is None or I_a is None:
             raise RuntimeError("unwarp_normals: pass I_g and I_a, or params=prepare(I_g, I_a)")
