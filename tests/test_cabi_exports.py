@@ -83,14 +83,16 @@ def test_product_never_imports_the_oracle():
                 assert not re.search(r"(from|import)\s+oracle|#include\s+\".*oracle|libwarp_oracle", text), f
 
 
-def test_torch_extension_builds_and_registers_its_operators():
+def test_torch_extension_operators_take_every_argument_set():
     """The thin torch C++ extension in front of the C ABI (csrc/torch_ops.cpp): loads on a CPU-only box, registers the
     operators with CUDA and Meta kernels; shapes come out of the Meta kernels without a GPU, with the canvas of vidc_camera_init
-    and the workspace of vidc_workspace_bytes (at least one frame, as the CUDA kernels allocate it)."""
+    and the workspace of vidc_workspace_bytes (at least one frame, as the CUDA kernels allocate it).  The fused operators take
+    every argument set of their C entry point: an output not asked for is None, and so is Cg_H_C with a prepared workspace."""
     import torch
     from vi_depth_completion_b200 import _cabi, build as vb
     torch.ops.load_library(vb.build_torch_ops())
     lib = _cabi.lib()
+    shapes = lambda outs: [None if o is None else tuple(o.shape) for o in outs]
     # 320x240, 640x480 and 300x201 (a width that is not a multiple of the 32-pixel tile, an odd height)
     for intr in ((202., 202., 159.93827, 119.938015), (404., 404., 319.87654, 239.87603), (190., 190., 150., 100.5)):
         cam = _cabi.VidcCamera()
@@ -101,27 +103,44 @@ def test_torch_extension_builds_and_registers_its_operators():
             g = torch.empty(B, 3, device="meta")
             H, y = torch.ops.vidc.warp_forward(x, g, g, *intr, 0)
             assert H.shape == (B, 3, 3) and y.shape == (B, 3, Hc, Wc)
-            H, z = torch.ops.vidc.unwarp_normals(x, g, g, *intr, True)
-            assert H.shape == (B, 3, 3) and z.shape == (B, 3, Hc, Wc)
-            outs = torch.ops.vidc.warp_rgbd(x, x[:, :1], g, g, *intr, 1)
-            assert [tuple(o.shape) for o in outs] == [(B, 3, 3), (B, 3, Hc, Wc), (B, 1, Hc, Wc), (B, 1, Hc, Wc)]
+            H, z, valid = torch.ops.vidc.unwarp_normals(x, g, g, None, *intr, True, False)
+            assert H.shape == (B, 3, 3) and z.shape == (B, 3, Hc, Wc) and valid is None
+            outs = torch.ops.vidc.warp_rgbd(x, x[:, :1], g, g, None, *intr, 1, True, False)
+            assert shapes(outs) == [(B, 3, 3), (B, 3, Hc, Wc), (B, 1, Hc, Wc), (B, 1, Hc, Wc), None]
             assert outs[3].dtype == torch.uint8
             assert [tuple(m.shape) for m in torch.ops.vidc.build_homography(g, g, *intr)] == [(B, 3, 3)] * 3
             # parameters prepared once per batch: the Meta workspace has the size the library asks for
             ws, H = torch.ops.vidc.frame_params(g, g, *intr)
             assert ws.numel() * 4 == lib.vidc_workspace_bytes(ctypes.byref(cam), max(B, 1)) and H.shape == (B, 3, 3)
-            outs = torch.ops.vidc.warp_rgbd_prepared(x, x[:, :1], ws, *intr, 0)
-            assert [tuple(o.shape) for o in outs] == [(B, 3, Hc, Wc), (B, 1, Hc, Wc), (B, 1, Hc, Wc)]
-            assert torch.ops.vidc.unwarp_normals_prepared(x, ws, *intr, True).shape == (B, 3, Hc, Wc)
+            outs = torch.ops.vidc.warp_rgbd(x, x[:, :1], None, None, ws, *intr, 0, True, False)
+            assert shapes(outs) == [None, (B, 3, Hc, Wc), (B, 1, Hc, Wc), (B, 1, Hc, Wc), None]
+            assert shapes(torch.ops.vidc.unwarp_normals(x, None, None, ws, *intr, True, False)) == [None, (B, 3, Hc, Wc), None]
+            # the optional inputs and outputs: no depth, no mask, coverage counts, the validity plane, in both forms
+            for src in ((g, g, None), (None, None, ws)):
+                Hs = (B, 3, 3) if src[2] is None else None
+                outs = torch.ops.vidc.warp_rgbd(x, None, *src, *intr, 0, False, True)
+                assert shapes(outs) == [Hs, (B, 3, Hc, Wc), None, None, (B,)] and outs[4].dtype == torch.int32
+                outs = torch.ops.vidc.warp_rgbd(x, x[:, :1], *src, *intr, 1, True, True)
+                assert shapes(outs) == [Hs, (B, 3, Hc, Wc), (B, 1, Hc, Wc), (B, 1, Hc, Wc), (B,)]
+                outs = torch.ops.vidc.unwarp_normals(x, *src, *intr, False, True)
+                assert shapes(outs) == [Hs, (B, 3, Hc, Wc), (B, 1, Hc, Wc)] and outs[2].dtype == torch.uint8
     # intrinsics vidc_camera_init rejects are rejected by the Meta kernels too, as by the CUDA kernels
     x, g = torch.empty(2, 3, 240, 320, device="meta"), torch.empty(2, 3, device="meta")
     bad = (202., 202., 0., 119.938015)
-    calls = (lambda: torch.ops.vidc.warp_forward(x, g, g, *bad, 0), lambda: torch.ops.vidc.unwarp_normals(x, g, g, *bad, True),
-             lambda: torch.ops.vidc.warp_rgbd(x, x[:, :1], g, g, *bad, 0), lambda: torch.ops.vidc.build_homography(g, g, *bad),
-             lambda: torch.ops.vidc.frame_params(g, g, *bad))
+    calls = (lambda: torch.ops.vidc.warp_forward(x, g, g, *bad, 0), lambda: torch.ops.vidc.unwarp_normals(x, g, g, None, *bad, True, False),
+             lambda: torch.ops.vidc.warp_rgbd(x, x[:, :1], g, g, None, *bad, 0, True, False),
+             lambda: torch.ops.vidc.build_homography(g, g, *bad), lambda: torch.ops.vidc.frame_params(g, g, *bad))
     for call in calls:
         with pytest.raises(RuntimeError, match="intrinsics"):
             call()
+    # the frame parameters come from I_g and I_a or from a prepared workspace: exactly one of the two
+    intr = (202., 202., 159.93827, 119.938015)
+    ws, _ = torch.ops.vidc.frame_params(g, g, *intr)
+    for src in ((g, g, ws), (None, None, None), (g, None, None)):
+        for call in (lambda: torch.ops.vidc.warp_rgbd(x, None, *src, *intr, 0, True, False),
+                     lambda: torch.ops.vidc.unwarp_normals(x, *src, *intr, True, False)):
+            with pytest.raises(RuntimeError, match="pass either I_g and I_a or params"):
+                call()
 
 
 def test_torch_extension_is_required(monkeypatch, tmp_path):

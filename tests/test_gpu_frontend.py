@@ -56,21 +56,24 @@ def test_torch_compile_fullgraph(cuda_device):
     import torch
     w, rgb, depth, normals, g, a = _setup(cuda_device)
 
-    def path(x, n, gg, aa):
+    def path(x, d, n, gg, aa):
         _, x1 = w.warp_with_gravity_center_aligned(x, gg, aa)
         _, z = w.inverse_warp_normal_image_with_gravity_center_aligned(n * 2.0, gg, aa)
-        return x1 + 1.0, torch.nn.functional.normalize(z, dim=1)
+        _, rgb_w, depth_w, mask, cov = w.warp_rgbd(x, d, gg, aa, with_coverage=True)
+        _, nh, valid = w.unwarp_normals(n, gg, aa, with_valid=True)
+        return x1 + 1.0, torch.nn.functional.normalize(z, dim=1), rgb_w * 2.0, depth_w, mask, cov, nh, valid
 
     with torch.no_grad():
-        want = path(rgb, normals, g, a)
-        got = torch.compile(path, fullgraph=True, backend="aot_eager")(rgb, normals, g, a)
-    assert torch.equal(want[0], got[0]) and torch.equal(want[1], got[1])
+        want = path(rgb, depth, normals, g, a)
+        got = torch.compile(path, fullgraph=True, backend="aot_eager")(rgb, depth, normals, g, a)
+    assert len(got) == len(want) and all(torch.equal(x, y) for x, y in zip(want, got))
 
 
 def test_parameters_prepared_once_per_batch(cuda_device):
     """prepare() + warp_rgbd(params=) + unwarp_normals(params=): one per-frame kernel for the batch instead of one per call
-    (the reference rebuilds the homographies in every call, :124 and :225).  Same bits as the calls that take I_g / I_a; two
-    launches saved per step; the handle is checked (camera, batch, device)."""
+    (the reference rebuilds the homographies in every call, :124 and :225).  Same bits as the calls that take I_g / I_a, for
+    every argument set (no depth, no mask, coverage, the validity plane, uint8 frames); two launches saved per step; the
+    handle is checked (camera, batch, device)."""
     import torch
     from vi_depth_completion_b200 import _cabi
     from vi_depth_completion_b200.warping_2dof_alignment import Warping2DOFAlignment
@@ -87,6 +90,20 @@ def test_parameters_prepared_once_per_batch(cuda_device):
     for x, y in ((H0, H1), (H0, H2), (r0, r1), (d0, d1), (m0, m1), (z0, z1), (zr0, zr1)):
         assert torch.equal(x, y)
     assert depth.dim() == 3 and d1.dim() == 3                            # 3-D depth in, 3-D depth out (:110-112, :153-154)
+    # every other argument set takes params= too: the gravity form's bits, one launch per call
+    u8 = (rgb * 255).to(torch.uint8).permute(0, 2, 3, 1).contiguous()
+    calls = (lambda **k: w.warp_rgbd(rgb, depth, with_coverage=True, **k),
+             lambda **k: w.warp_rgbd(rgb, None, **k),
+             lambda **k: w.warp_rgbd(rgb, depth, depth_mode="nearest", with_mask=False, with_coverage=True, **k),
+             lambda **k: w.warp_rgbd_u8(u8, None, with_mask=False, with_coverage=True, **k),
+             lambda **k: w.unwarp_normals(normals, with_valid=True, **k),
+             lambda **k: w.unwarp_normals(normals, normalize=False, with_valid=True, **k))
+    want = [call(I_g=g, I_a=a) for call in calls]
+    n0 = _cabi.lib().vidc_launch_count()
+    got = [call(params=p) for call in calls]
+    assert _cabi.lib().vidc_launch_count() - n0 == len(calls)
+    for x, y in zip(want, got):
+        assert len(x) == len(y) and all((u is None and v is None) or torch.equal(u, v) for u, v in zip(x, y))
     d4 = w.warp_rgbd(rgb, depth[:, None], params=p)[2]
     assert d4.dim() == 4 and torch.equal(d4[:, 0], d0)
     with pytest.raises(AssertionError):

@@ -307,7 +307,7 @@ def test_errors(cuda_device):
     _, y = w.unwarp_normals(x, g, g)                        # fused renormalising entry point: forward-only
     with pytest.raises(NotImplementedError):
         y.sum().backward()
-    # the same for the fused forward entry (through the torch extension and through ctypes): never a silent zero gradient
+    # the same for the fused forward entry (with and without coverage counts): never a silent zero gradient
     import warnings
     for kw in ({}, {"with_coverage": True}):
         x = torch.rand(2, 3, 240, 320, device=cuda_device, requires_grad=True)

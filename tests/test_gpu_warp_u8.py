@@ -223,11 +223,11 @@ def test_u8_warp_errors_and_autograd(cuda_device):
     with pytest.raises(RuntimeError):
         w.warp_rgbd_u8(u8, depth.cpu(), g, a)                               # depth on another device
     with pytest.raises(RuntimeError):
-        w.warp_rgbd_u8(u8, depth.cpu(), g, a, with_coverage=True)           # the same through the C ABI
+        w.warp_rgbd_u8(u8, depth.cpu(), g, a, with_coverage=True)           # the same with coverage counts
     with pytest.raises(AssertionError):
-        w.warp_rgbd_u8(u8, depth, g[:1], a[:1])                             # batch mismatch, torch operator
+        w.warp_rgbd_u8(u8, depth, g[:1], a[:1])                             # batch mismatch
     with pytest.raises(AssertionError):
-        w.warp_rgbd_u8(u8, depth, g[:1], a[:1], with_coverage=True)         # batch mismatch, C ABI
+        w.warp_rgbd_u8(u8, depth, g[:1], a[:1], with_coverage=True)         # batch mismatch, with coverage counts
     with pytest.raises(AssertionError):
         w.warp_rgbd_u8(u8, depth, params=w.prepare(g[:1], a[:1]))
     with pytest.raises(RuntimeError):
@@ -254,7 +254,7 @@ def test_u8_warp_errors_and_autograd(cuda_device):
 
 
 @pytest.mark.gpu
-def test_u8_operators_trace_under_torch_compile(cuda_device):
+def test_u8_operator_traces_under_torch_compile_in_both_forms(cuda_device):
     import torch
 
     from vi_depth_completion_b200 import _torchops
@@ -268,7 +268,8 @@ def test_u8_operators_trace_under_torch_compile(cuda_device):
 
     def f(u8, depth, g, a):
         ws, _ = ops.frame_params(g, a, *intr)
-        return ops.warp_rgbd_u8(u8, depth, g, a, *intr, 0)[1] + ops.warp_rgbd_u8_prepared(u8, depth, ws, *intr, 0)[0]
+        return ops.warp_rgbd_u8(u8, depth, g, a, None, *intr, 0, True, False)[1] + \
+            ops.warp_rgbd_u8(u8, depth, None, None, ws, *intr, 0, True, False)[1]
 
     got = torch.compile(f, fullgraph=True, backend="eager")(u8, depth, g, a)
     assert torch.equal(got, f(u8, depth, g, a))

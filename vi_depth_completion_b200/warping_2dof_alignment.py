@@ -391,43 +391,29 @@ class Warping2DOFAlignment:
 
     # networks/warping_2dof_alignment.py:216-255
     def inverse_warp_normal_image_with_gravity_center_aligned(self, x, I_g, I_a):
-        return self._unwarp(x, I_g, I_a, normalize=False, gravity_grad=True)[:2]
+        return self._unwarp(x, I_g, I_a, None, normalize=False, with_valid=False, gravity_grad=True)[:2]
 
-    def _unwarp(self, x, I_g, I_a, normalize, want_valid=False, gravity_grad=False):
+    def _unwarp(self, x, I_g, I_a, params, normalize, with_valid, gravity_grad=False):
         """gravity_grad: the reference-shaped method, differentiable w.r.t. I_g / I_a; the fused entry point (unwarp_normals)
-        is forward-only w.r.t. them."""
+        is forward-only w.r.t. them, and w.r.t. the image too when it renormalises or reads params=."""
         _require_cuda_f32(x, "x")
         if x.dim() != 4:
             raise RuntimeError(f"x: expected a 4-D tensor, got {x.dim()}-D")
-        device = x.device
-        grav_grad = _wants_grad(I_g, I_a)
+        grav, source = self._frame_source(x, "x", I_g, I_a, params)
         needs_graph = torch.is_grad_enabled() and x.requires_grad
-        if want_valid:                                          # no operator returns the validity plane
-            g, a = _gravity(I_g, I_a, device)
-            z = self._empty_like_canvas(x)
-            Cg_H_C = torch.empty((g.shape[0], 3, 3), dtype=torch.float32, device=device)
-            valid = torch.empty((x.shape[0], 1, int(self.H), int(self.W)), dtype=torch.uint8, device=device)
-            xi, zi = _image(x), _image(z)
-            with torch.cuda.device(device):
-                check(lib().vidc_unwarp_normals(ctypes.byref(self._cam), ctypes.byref(xi), g.data_ptr(), a.data_ptr(), g.shape[0],
-                                                1 if normalize else 0, self._params_ws(g.shape[0], device).data_ptr(),
-                                                Cg_H_C.data_ptr(), ctypes.byref(zi), valid.data_ptr(), _stream_ptr(device)))
-        else:
-            _require_cuda_f32(I_g, "I_g")
-            _require_cuda_f32(I_a, "I_a")
-            Cg_H_C, z = _op(_torchops.ops().unwarp_normals, x.detach() if needs_graph else x, _nd(I_g), _nd(I_a), *self._intr,
-                            bool(normalize))
-            if not (needs_graph or grav_grad):
-                return Cg_H_C, z, None
-            g, a = _gravity(I_g, I_a, device)
-            valid = None
-        return self._unwarp_graph(x, z, Cg_H_C, g, a, I_g, I_a, normalize, needs_graph, grav_grad and gravity_grad) + (valid,)
-
-    def _unwarp_graph(self, x, z, Cg_H_C, g, a, I_g, I_a, normalize, needs_graph, grav_diff):
-        if grav_diff and not normalize:
-            return _HomographyFn.apply(g, a, self, Cg_H_C), _WarpFn.apply(x, z, self, g, a, True, _cabi.VIDC_BILINEAR)
-        z = _attach(x, z, self, g, a, True, _cabi.VIDC_BILINEAR) if not normalize else _attach(x, z)
-        return _no_gravity_grad((Cg_H_C, z), I_g, I_a)
+        Cg_H_C, z, valid = _op(_torchops.ops().unwarp_normals, x.detach() if needs_graph else x, *source, *self._intr, bool(normalize),
+                               bool(with_valid))
+        if params is not None:
+            Cg_H_C = params.H
+        grav_grad = _wants_grad(*grav)
+        if not (needs_graph or grav_grad):
+            return Cg_H_C, z, valid
+        if params is not None or normalize:                     # no backward kernel for these
+            return _no_gravity_grad((Cg_H_C, _attach(x, z)), *grav) + (valid,)
+        g, a = _gravity(I_g, I_a, x.device)
+        if grav_grad and gravity_grad:
+            return _HomographyFn.apply(g, a, self, Cg_H_C), _WarpFn.apply(x, z, self, g, a, True, _cabi.VIDC_BILINEAR), valid
+        return _no_gravity_grad((Cg_H_C, _attach(x, z, self, g, a, True, _cabi.VIDC_BILINEAR)), I_g, I_a) + (valid,)
 
     # networks/warping_2dof_alignment.py:258-290.  The reference method cannot run (:259 unpacks three
     # return values into two); this implements its evident intent: forward warp, then z = R y.
@@ -491,124 +477,54 @@ class Warping2DOFAlignment:
             raise AssertionError(f"{name}.shape[0]={x.shape[0]} != I_g.shape[0]={params.B}")
         return params
 
+    def _frame_source(self, x, name, I_g, I_a, params):
+        """The gravity whose gradient the call's outputs refuse, and the operator's (I_g, I_a, params) arguments: the per-frame
+        parameters from I_g / I_a, or from params=prepare(I_g, I_a)."""
+        if params is not None:
+            p = self._prepared(params, x, name)
+            return p.grav, (None, None, p.ws)
+        if I_g is None or I_a is None:
+            raise RuntimeError("pass I_g and I_a, or params=prepare(I_g, I_a)")
+        _require_cuda_f32(I_g, "I_g")
+        _require_cuda_f32(I_a, "I_a")
+        return (I_g, I_a), (_nd(I_g), _nd(I_a), None)
+
+    def _warp_rgbd(self, op, x, name, x_depth, I_g, I_a, mode, with_mask, with_coverage, params):
+        """warp_rgbd / warp_rgbd_u8 once their RGB input x is checked: one call of the operator `op`."""
+        d4 = None
+        if x_depth is not None:
+            _require_cuda_f32(x_depth, "x_depth")
+            d4 = x_depth.view(x_depth.shape[0], 1, x_depth.shape[1], x_depth.shape[2]) if x_depth.dim() == 3 else x_depth
+        grav, source = self._frame_source(x, name, I_g, I_a, params)
+        Cg_H_C, rgb_w, depth_w, mask, cov = _op(op, _nd(x), _nd(d4), *source, *self._intr, mode, bool(with_mask), bool(with_coverage))
+        if params is not None:
+            Cg_H_C = params.H
+        if depth_w is not None:
+            if x_depth.dim() == 3:
+                depth_w = depth_w.view(depth_w.shape[0], depth_w.shape[2], depth_w.shape[3])
+            depth_w = _attach(x_depth, depth_w)
+        out = _no_gravity_grad((Cg_H_C, _attach(x, rgb_w), depth_w, mask), *grav)                  # forward-only
+        return out + (cov,) if with_coverage else out
+
     def warp_rgbd(self, x_rgb, x_depth, I_g=None, I_a=None, depth_mode='bilinear', with_mask=True, with_coverage=False, params=None):
         """One pass: warp RGB (B,3,h,w) and sparse depth (B,h,w)/(B,1,h,w) into the gravity-aligned canvas and
         emit the validity mask of surface_normal.py:151.  Returns (Cg_H_C, rgb_w, depth_w, mask_u8[, coverage]).
         params=prepare(I_g, I_a) instead of I_g / I_a: no per-frame kernel in this call."""
-        _check_interp_mode(depth_mode)
+        mode = _check_interp_mode(depth_mode)
         _require_cuda_f32(x_rgb, "x_rgb")
-        device = x_rgb.device
-        mode = _cabi.VIDC_BILINEAR if depth_mode == "bilinear" else _cabi.VIDC_NEAREST
-        if params is not None:
-            if x_rgb.dim() != 4 or not isinstance(x_depth, torch.Tensor) or not with_mask or with_coverage:
-                raise RuntimeError("warp_rgbd(params=...): RGB (B,3,h,w) + depth, mask on, no coverage")
-            p = self._prepared(params, x_rgb, "x_rgb")
-            _require_cuda_f32(x_depth, "x_depth")
-            d4 = x_depth.view(x_depth.shape[0], 1, x_depth.shape[1], x_depth.shape[2]) if x_depth.dim() == 3 else x_depth
-            rgb_w, depth_w, mask = _op(_torchops.ops().warp_rgbd_prepared, _nd(x_rgb), _nd(d4), p.ws, *self._intr, mode)
-            if x_depth.dim() == 3:
-                depth_w = depth_w.view(depth_w.shape[0], depth_w.shape[2], depth_w.shape[3])
-            return _no_gravity_grad((p.H, _attach(x_rgb, rgb_w), _attach(x_depth, depth_w), mask), *p.grav)
-        if I_g is None or I_a is None:
-            raise RuntimeError("warp_rgbd: pass I_g and I_a, or params=prepare(I_g, I_a)")
-        if with_mask and not with_coverage and x_depth is not None:
-            _require_cuda_f32(x_depth, "x_depth")
-            _require_cuda_f32(I_g, "I_g")
-            _require_cuda_f32(I_a, "I_a")
-            d4 = x_depth.view(x_depth.shape[0], 1, x_depth.shape[1], x_depth.shape[2]) if x_depth.dim() == 3 else x_depth
-            Cg_H_C, rgb_w, depth_w, mask = _op(_torchops.ops().warp_rgbd, _nd(x_rgb), _nd(d4), _nd(I_g), _nd(I_a), *self._intr, mode)
-            if x_depth.dim() == 3:
-                depth_w = depth_w.view(depth_w.shape[0], depth_w.shape[2], depth_w.shape[3])
-            return _no_gravity_grad((Cg_H_C, _attach(x_rgb, rgb_w), _attach(x_depth, depth_w), mask), I_g, I_a)   # forward-only
-        g, a = _gravity(I_g, I_a, device)                       # coverage, no mask or no depth: no operator takes these
-        B = x_rgb.shape[0]
-        squeeze = False
-        di = dwi = None
-        depth_w = None
-        if x_depth is not None:
-            _require_cuda_f32(x_depth, "x_depth")
-            if x_depth.device != device:
-                raise RuntimeError(f"x_depth must live on {device}, got {x_depth.device}")
-            if x_depth.dim() == 3:
-                x_depth = x_depth.view(x_depth.shape[0], 1, x_depth.shape[1], x_depth.shape[2])
-                squeeze = True
-            depth_w = self._empty_like_canvas(x_depth)
-            di, dwi = _image(x_depth), _image(depth_w)
-        rgb_w = self._empty_like_canvas(x_rgb)
-        mask = torch.empty((B, 1, int(self.H), int(self.W)), dtype=torch.uint8, device=device) if with_mask else None
-        cov = torch.empty((B,), dtype=torch.int32, device=device) if with_coverage else None
-        Cg_H_C = torch.empty((g.shape[0], 3, 3), dtype=torch.float32, device=device)
-        ri, rwi = _image(x_rgb), _image(rgb_w)
-        with torch.cuda.device(device):
-            check(lib().vidc_warp_rgbd(ctypes.byref(self._cam), ctypes.byref(ri), ctypes.byref(di) if di is not None else None,
-                                       g.data_ptr(), a.data_ptr(), g.shape[0], mode, self._params_ws(g.shape[0], device).data_ptr(),
-                                       Cg_H_C.data_ptr(), ctypes.byref(rwi), ctypes.byref(dwi) if dwi is not None else None,
-                                       mask.data_ptr() if with_mask else None, cov.data_ptr() if with_coverage else None,
-                                       _stream_ptr(device)))
-        if squeeze:
-            depth_w = depth_w.view(B, depth_w.shape[2], depth_w.shape[3])
-        out = (Cg_H_C, _attach(x_rgb, rgb_w), depth_w if depth_w is None else _attach(x_depth, depth_w), mask)   # forward-only
-        out = _no_gravity_grad(out, I_g, I_a)
-        return out + (cov,) if with_coverage else out
+        return self._warp_rgbd(_torchops.ops().warp_rgbd, x_rgb, "x_rgb", x_depth, I_g, I_a, mode, with_mask, with_coverage, params)
 
     def warp_rgbd_u8(self, rgb_u8, x_depth, I_g=None, I_a=None, depth_mode='bilinear', with_mask=True, with_coverage=False, params=None):
         """warp_rgbd on the frames as the loader decodes them: rgb_u8 is (B,h,w,3) uint8 on the device (dataset.py:468-471,
         before ToTensor).  Same arguments, return tuple and bits as warp_rgbd(to_tensor_u8(rgb_u8), ...); RGB comes out as
         contiguous (B,3,H,W) float32.  The kernel converts each tap itself, so the float copy of the frames is never made."""
-        _check_interp_mode(depth_mode)
+        mode = _check_interp_mode(depth_mode)
         if not isinstance(rgb_u8, torch.Tensor) or not rgb_u8.is_cuda or rgb_u8.dtype != torch.uint8 or rgb_u8.dim() != 4:
             raise RuntimeError("rgb_u8: expected a (B,H,W,3) uint8 CUDA tensor")
         if rgb_u8.shape[3] != 3:
             raise RuntimeError(f"rgb_u8: 3 channels, got {rgb_u8.shape[3]}")
-        x = rgb_u8.contiguous()
-        device = x.device
-        mode = _cabi.VIDC_BILINEAR if depth_mode == "bilinear" else _cabi.VIDC_NEAREST
-        d4 = None
-        if x_depth is not None:
-            _require_cuda_f32(x_depth, "x_depth")
-            d4 = x_depth.view(x_depth.shape[0], 1, x_depth.shape[1], x_depth.shape[2]) if x_depth.dim() == 3 else x_depth
-        cov = None
-        if params is not None:
-            if d4 is None or not with_mask or with_coverage:
-                raise RuntimeError("warp_rgbd_u8(params=...): depth, mask on, no coverage")
-            p = self._prepared(params, x, "rgb_u8")
-            rgb_w, depth_w, mask = _op(_torchops.ops().warp_rgbd_u8_prepared, x, _nd(d4), p.ws, *self._intr, mode)
-            Cg_H_C, grav = p.H, p.grav
-        elif I_g is None or I_a is None:
-            raise RuntimeError("warp_rgbd_u8: pass I_g and I_a, or params=prepare(I_g, I_a)")
-        elif d4 is not None and with_mask and not with_coverage:
-            _require_cuda_f32(I_g, "I_g")
-            _require_cuda_f32(I_a, "I_a")
-            Cg_H_C, rgb_w, depth_w, mask = _op(_torchops.ops().warp_rgbd_u8, x, _nd(d4), _nd(I_g), _nd(I_a), *self._intr, mode)
-            grav = (I_g, I_a)
-        else:                                                   # coverage, no mask or no depth: no operator takes these
-            grav = (I_g, I_a)
-            g, a = _gravity(I_g, I_a, device)
-            B = x.shape[0]
-            di = dwi = depth_w = None
-            if d4 is not None:
-                if d4.device != device:
-                    raise RuntimeError(f"x_depth must live on {device}, got {d4.device}")
-                depth_w = self._empty_like_canvas(d4)
-                di, dwi = _image(d4), _image(depth_w)
-            Cg_H_C = torch.empty((g.shape[0], 3, 3), dtype=torch.float32, device=device)
-            rgb_w = torch.empty((B, 3, int(self.H), int(self.W)), dtype=torch.float32, device=device)
-            mask = torch.empty((B, 1, int(self.H), int(self.W)), dtype=torch.uint8, device=device) if with_mask else None
-            cov = torch.empty((B,), dtype=torch.int32, device=device) if with_coverage else None
-            rwi = _image(rgb_w)
-            with torch.cuda.device(device):
-                check(lib().vidc_warp_rgbd_u8(ctypes.byref(self._cam), x.data_ptr(), B, x.shape[1], x.shape[2],
-                                              ctypes.byref(di) if di is not None else None, g.data_ptr(), a.data_ptr(), g.shape[0],
-                                              mode, self._params_ws(g.shape[0], device).data_ptr(), Cg_H_C.data_ptr(),
-                                              ctypes.byref(rwi), ctypes.byref(dwi) if dwi is not None else None,
-                                              mask.data_ptr() if with_mask else None, cov.data_ptr() if with_coverage else None,
-                                              _stream_ptr(device)))
-        if depth_w is not None:
-            if x_depth.dim() == 3:
-                depth_w = depth_w.view(depth_w.shape[0], depth_w.shape[2], depth_w.shape[3])
-            depth_w = _attach(x_depth, depth_w)                                                  # forward-only
-        out = _no_gravity_grad((Cg_H_C, rgb_w, depth_w, mask), *grav)
-        return out + (cov,) if with_coverage else out
+        return self._warp_rgbd(_torchops.ops().warp_rgbd_u8, rgb_u8.contiguous(), "rgb_u8", x_depth, I_g, I_a, mode, with_mask,
+                               with_coverage, params)
 
     def warp_rgb_sparse_depth(self, x_rgb, tracks, counts, fc, cc, I_g, I_a, depth_mode='bilinear', with_mask=True, with_coverage=False):
         """SURVEY row f2: warp RGB (B,3,H,W) and the SPARSE depth given as KLT tracks (B,N,>=4) float64 [id, x, y, z, ...] (valid
@@ -673,15 +589,5 @@ class Warping2DOFAlignment:
     def unwarp_normals(self, y, I_g=None, I_a=None, normalize=True, with_valid=False, params=None):
         """One pass: inverse warp + R^T rotation + F.normalize(dim=1) (surface_normal.py:169-170).
         Returns (Cg_H_C, n_hat[, valid_u8]).  params=prepare(I_g, I_a) instead of I_g / I_a: no per-frame kernel here."""
-        if params is not None:
-            _require_cuda_f32(y, "x")
-            if y.dim() != 4 or with_valid:
-                raise RuntimeError("unwarp_normals(params=...): a 4-D image, no validity output")
-            p = self._prepared(params, y, "x")
-            needs_graph = torch.is_grad_enabled() and y.requires_grad
-            z = _op(_torchops.ops().unwarp_normals_prepared, y.detach() if needs_graph else y, p.ws, *self._intr, bool(normalize))
-            return _no_gravity_grad((p.H, (_attach(y, z) if needs_graph else z)), *p.grav)   # forward-only with a prepared workspace
-        if I_g is None or I_a is None:
-            raise RuntimeError("unwarp_normals: pass I_g and I_a, or params=prepare(I_g, I_a)")
-        H, z, valid = self._unwarp(y, I_g, I_a, normalize=normalize, want_valid=with_valid)
+        H, z, valid = self._unwarp(y, I_g, I_a, params, normalize, with_valid)
         return (H, z, valid) if with_valid else (H, z)
