@@ -10,6 +10,7 @@ import sys, os, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
 from tests import common as C
+from tests import exact_reference as X
 from oracle import oracle as O
 from vi_depth_completion_b200.warping_2dof_alignment import Warping2DOFAlignment
 
@@ -74,7 +75,7 @@ def main(cases=300, seed=2024):
         assert np.array_equal(mask.cpu().numpy().reshape(-1), om.reshape(-1)), ("mask", tag)
         assert np.array_equal(mask_p.cpu().numpy().reshape(-1), om.reshape(-1)), ("mask prepared", tag)
         assert np.array_equal(cov.cpu().numpy().astype(np.int64), om.reshape(B, -1).sum(1).astype(np.int64)), ("coverage", tag)
-        assert int(valid.max()) <= 1
+        assert np.array_equal(valid.cpu().numpy().reshape(-1), X.touch_plane(o, I_g, I_a).reshape(-1)), ("valid", tag)
         px += B * o.H * o.W
     print(f"fuzz ok: {cases} cameras, {px / 1e6:.1f} Mpx per output, paths {paths}, {time.time() - t0:.0f} s", flush=True)
 

@@ -336,6 +336,7 @@ _VARIANT_CODE = r'''
 import sys, numpy as np, torch
 sys.path.insert(0, %r)
 from tests import common as C
+from tests import exact_reference as X
 from oracle import oracle as O
 from vi_depth_completion_b200.warping_2dof_alignment import Warping2DOFAlignment
 dev = torch.device("cuda", 0)
@@ -368,7 +369,7 @@ for cam, (I_g, I_a) in (("S1", C.random_gravity(6, 1234)), ("S2", C.random_gravi
     _, oz = o.inverse_warp_normal_image_with_gravity_center_aligned(nrm, I_g, I_a)
     assert C.count_bit_mismatches(z.cpu().numpy(), oz) == 0, (cam, "unwarp")
     assert C.count_bit_mismatches(nh.cpu().numpy(), O.normalize(oz)) == 0, (cam, "unwarp+normalize")
-    assert valid.cpu().numpy().min() >= 0 and valid.cpu().numpy().max() <= 1, (cam, "valid flags")
+    assert np.array_equal(valid.cpu().numpy().reshape(-1), X.touch_plane(o, I_g, I_a).reshape(-1)), (cam, "valid flags")
 # signed zeros / denormals / inf / NaN through the same variant
 w, o = Warping2DOFAlignment(*C.CAMERAS["S1"]), O.Oracle(*C.CAMERAS["S1"])
 rgb, depth, nrm = C.special_value_images(4, o.H, o.W, 21)

@@ -8,9 +8,13 @@ namespace vidc_k {
 // ------------------------------------------------------------------------------------------
 // Backward kernels (SURVEY.md section 8 row f4): gradient w.r.t. the sampled image.  Same coordinates as the
 // forward kernels; each output-gradient pixel scatters w_tap * g into its (in-bounds) taps with atomicAdd, as
-// ATen's grid_sampler_2d_backward does on CUDA.  The sum order is therefore not deterministic: parity is to
-// tolerance, not bit-exact.  ROT: the incoming gradient is first rotated, g <- R g (the forward pass of the
-// inverse warp applied R^T after sampling, :253).
+// ATen's grid_sampler_2d_backward does on CUDA.  The sum order is therefore not deterministic: each element S is an
+// fp32 sum, from the memset's +0 in some order, of its k terms t, and tests/test_gpu_atomic_backward.py holds it to
+// that: k = 0 gives +0, k <= 2 the order-free bits of (+0 + t1) + t2, NaN / infinite terms the IEEE result, and finite
+// terms |S - E| <= gamma_{k-1} sum|t| + k 2^-52 sum|t| + k 2^-126 (E the exact sum, gamma_n = n u / (1 - n u),
+// u = 2^-24); the last term because the fp32 atomicAdd flushes subnormal terms and sums to zero (measured on a B200).
+// ROT: the incoming gradient is first rotated, g <- R g (the forward pass of the inverse warp applied R^T after
+// sampling, :253).
 template <bool INVERSE>
 __global__ void __launch_bounds__(256)
 warp_backward_kernel(const vidc_frame_params* __restrict__ prm, CamConst cam, ImgView gy /* (B,C,H,W) grad of the output */,
